@@ -339,6 +339,25 @@ int rbv_last_kernel(const RbvContext* ctx);
 int rbv_voigt_h(RbvContext* ctx, const double* x, const double* a, double* out, int n, int method,
                 void* stream);
 
+/* Analytic gradient (DESIGN.md section 14): value and d/dtheta of vfit.lnprob (apply_prior != 0) or vfit.lnlike
+ * (apply_prior == 0) for a batch of walkers, from one forward pass and one adjoint pass per walker (no extra rows).
+ *   theta  DEVICE [n_walkers, ndim];  value DEVICE [n_walkers];  grad DEVICE [n_walkers, ndim] (columns beyond
+ *          3 * n_components are 0)
+ *   apply_prior != 0: rows outside the bounds get value -inf and a zero gradient row (the flat prior has zero
+ *          gradient; such rows are not evaluated).  apply_prior == 0: every row is evaluated.
+ *   NaN where the forward model gives NaN (b <= 0, NaN theta).  FP64 always (ignores rbv_set_precision); every
+ *   (line, pixel) pair is evaluated directly (ignores rbv_set_farfield).  Every LSF width the lnprob path accepts.
+ *   RBV_EINVAL for an instrument with voigt_method = RBV_VOIGT_FAST; at most 16 instruments.  Each row's result is
+ *   bit-identical whatever the batch size or the row's position in it.  Asynchronous.
+ * Workspace: rbv_grad_workspace_bytes() (no initialisation needed). */
+int rbv_grad_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* bytes);
+int rbv_lnprob_grad_batch(RbvContext* ctx, const double* theta, int n_walkers, int apply_prior, double* value,
+                          double* grad, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Test hook, like rbv_voigt_h: H = Re w(x + i a), dH/dx and dH/da on a lattice; all DEVICE arrays. */
+int rbv_voigt_h_grad(RbvContext* ctx, const double* x, const double* a, double* H, double* Hx, double* Ha, int n,
+                     void* stream);
+
 /* FP64 FMA throughput of the device (roofline denominator measured on the box): runs a dependent-chain
  * DFMA kernel for about `millis` ms and returns TFLOP/s (2 flops per FMA). */
 int rbv_measure_fp64_peak(RbvContext* ctx, double millis, double* tflops);

@@ -1061,6 +1061,7 @@ __global__ void __launch_bounds__(128) finalize_stream_kernel(const LaunchParams
 
 }  // namespace rbv
 #include "rbv_stream.cuh"   // warp-autonomous streaming form of the lnprob kernel (big batches)
+#include "rbv_grad.cuh"     // analytic gradient of lnprob / lnlike (forward + adjoint pass)
 namespace rbv {
 
 // ------------------------------------------------------------------------------------------ small kernels
@@ -1315,6 +1316,7 @@ struct HostInst {
   InstDev dev;
   std::vector<double> taps;  // LSF taps as applied by the reference (normalised if requested), length K
   double* d_taps = nullptr;  // flipped + zero-padded copy on the device (rebuilt when R changes)
+  double* d_grad_cum = nullptr;   // [2K] prefix / suffix sums of the flipped taps (gradient path, built on first use)
   std::vector<void*> owned;  // device allocations owned by the library for this instrument
 };
 
@@ -1454,6 +1456,7 @@ void rbv_destroy(RbvContext* ctx) {
   for (auto& hi : ctx->inst) {
     for (void* p : hi.owned) cudaFree(p);
     cudaFree(hi.d_taps);
+    cudaFree(hi.d_grad_cum);
   }
   if (ctx->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(ctx->comm);
   for (int r = 0; r < 16; ++r)
@@ -3073,6 +3076,144 @@ int rbv_voigt_h(RbvContext* ctx, const double* x, const double* a, double* out, 
   voigt_h_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(x, a, out, n, method, ctx->d_core_tab);
   RBV_CUDA(cudaGetLastError());
   ctx->launches++;
+  return RBV_OK;
+}
+
+int rbv_voigt_h_grad(RbvContext* ctx, const double* x, const double* a, double* H, double* Hx, double* Ha, int n,
+                     void* stream) {
+  if (!ctx || !x || !a || !H || !Hx || !Ha || n < 0) return fail(RBV_EINVAL, "rbv_voigt_h_grad: bad argument");
+  if (n == 0) return RBV_OK;
+  RBV_ON_DEVICE(ctx);
+  voigt_h_grad_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(x, a, H, Hx, Ha, n, ctx->d_core_tab);
+  RBV_CUDA(cudaGetLastError());
+  ctx->launches++;
+  return RBV_OK;
+}
+
+// ------------------------------------------------------------------------------------------ analytic gradient
+// Workspace of rbv_lnprob_grad_batch (byte offsets, 256-byte aligned); geometry per instrument is fixed by its pixel
+// count alone, so every row is reduced in the same order whatever the batch.
+struct GradLayout {
+  size_t oob, lc, F, r, g, pval, pline, linegrad, total;
+  int n_blk_total, n_tiles_total;
+  long long part_stride;
+};
+static GradLayout grad_layout(const RbvContext* ctx, int W, GradInst* gi) {
+  GradLayout L;
+  memset(&L, 0, sizeof(L));
+  int blk = 0, tiles = 0;
+  long long part = 0;
+  for (size_t k = 0; k < ctx->inst.size(); ++k) {
+    const InstDev& I = ctx->inst[k].dev;
+    GradInst g;
+    memset(&g, 0, sizeof(g));
+    g.blk_off = blk;
+    g.n_blk = (I.P + kGradBlock - 1) / kGradBlock;
+    g.tile_off = tiles;
+    g.n_tiles = (I.P + kGradTile - 1) / kGradTile;
+    g.part_off = part;
+    blk += g.n_blk;
+    tiles += g.n_tiles;
+    part += (long long)g.n_tiles * I.L * 3;
+    if (gi && k < (size_t)kMaxInst) gi[k] = g;
+  }
+  L.n_blk_total = blk;
+  L.n_tiles_total = tiles;
+  L.part_stride = part;
+  auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
+  const size_t Wz = (size_t)std::max(W, 1);
+  size_t off = 0;
+  L.oob = off;      off = al(off + Wz * sizeof(int));
+  L.lc = off;       off = al(off + Wz * ctx->n_lines_total * LC_STRIDE * sizeof(double));
+  L.F = off;        off = al(off + Wz * blk * kGradBlock * sizeof(double));
+  L.r = off;        off = al(off + Wz * blk * kGradBlock * sizeof(double));
+  L.g = off;        off = al(off + Wz * blk * kGradBlock * sizeof(double));
+  L.pval = off;     off = al(off + Wz * blk * sizeof(double));
+  L.pline = off;    off = al(off + Wz * (size_t)part * sizeof(double));
+  L.linegrad = off; off = al(off + Wz * ctx->n_lines_total * 3 * sizeof(double));
+  L.total = off;
+  return L;
+}
+
+int rbv_grad_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* bytes) {
+  if (!ctx || !bytes || n_walkers < 0) return fail(RBV_EINVAL, "rbv_grad_workspace_bytes: bad argument");
+  *bytes = grad_layout(ctx, n_walkers, nullptr).total;
+  return RBV_OK;
+}
+
+int rbv_lnprob_grad_batch(RbvContext* ctx, const double* theta, int W, int apply_prior, double* value, double* grad,
+                          void* workspace, size_t workspace_bytes, void* stream) {
+  const char* who = "rbv_lnprob_grad_batch";
+  if (!ctx || !theta || !value || !grad) return fail(RBV_EINVAL, std::string(who) + ": null argument");
+  if (W < 0) return fail(RBV_EINVAL, std::string(who) + ": negative n_walkers");
+  if (W == 0) return RBV_OK;
+  if (ctx->inst.empty()) return fail(RBV_ESTATE, std::string(who) + ": no instrument added");
+  if (ctx->ndim == 0) return fail(RBV_ESTATE, std::string(who) + ": bounds not set (rbv_set_bounds)");
+  if (ctx->inst.size() > (size_t)kMaxInst)
+    return fail(RBV_EINVAL, std::string(who) + ": at most 16 instruments in a joint fit");
+  for (auto& hi : ctx->inst) {
+    if (!hi.dev.flux || !hi.dev.inv_sigma2 || !hi.dev.log_inv_sigma2)
+      return fail(RBV_ESTATE, std::string(who) + ": an instrument has no observed spectrum (flux-only instrument)");
+    if (3 * hi.dev.C > ctx->ndim) return fail(RBV_EINVAL, std::string(who) + ": ndim smaller than 3 * n_components");
+    if (hi.dev.method != RBV_VOIGT_WOFZ)
+      return fail(RBV_EINVAL, std::string(who) + ": no gradient for voigt_method='fast' (Tepper-Garcia)");
+  }
+  GradParams prm;
+  memset(&prm, 0, sizeof(prm));
+  const GradLayout lay = grad_layout(ctx, W, prm.gi);
+  if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, std::string(who) + ": workspace too small");
+  RBV_ON_DEVICE(ctx);
+  for (size_t k = 0; k < ctx->inst.size(); ++k) {
+    HostInst& hi = ctx->inst[k];
+    if (!hi.d_grad_cum) {   // prefix / suffix sums of the flipped taps: what the edge replication piles on 0 and P-1
+      const int K = hi.dev.K;
+      std::vector<double> cum(2 * (size_t)K);
+      double s = 0.0;
+      for (int m = 0; m < K; ++m) cum[m] = (s += hi.taps[K - 1 - m]);
+      s = 0.0;
+      for (int m = K - 1; m >= 0; --m) cum[K + m] = (s += hi.taps[K - 1 - m]);
+      RBV_CUDA(upload(&hi.d_grad_cum, cum.data(), cum.size()));
+    }
+    prm.gi[k].cum_lo = hi.d_grad_cum;
+    prm.gi[k].cum_hi = hi.d_grad_cum + hi.dev.K;
+  }
+  char* ws = (char*)workspace;
+  prm.inst = ctx->d_inst;
+  prm.theta = theta;
+  prm.lb = apply_prior ? ctx->d_lb : nullptr;
+  prm.ub = apply_prior ? ctx->d_ub : nullptr;
+  prm.core_tab = ctx->d_core_tab;
+  prm.value = value;
+  prm.grad = grad;
+  prm.oob = (int*)(ws + lay.oob);
+  prm.lc = (double*)(ws + lay.lc);
+  prm.F = (double*)(ws + lay.F);
+  prm.r = (double*)(ws + lay.r);
+  prm.g = (double*)(ws + lay.g);
+  prm.pval = (double*)(ws + lay.pval);
+  prm.pline = (double*)(ws + lay.pline);
+  prm.linegrad = (double*)(ws + lay.linegrad);
+  prm.part_stride = lay.part_stride;
+  prm.W = W;
+  prm.ndim = ctx->ndim;
+  prm.n_inst = (int)ctx->inst.size();
+  prm.n_lines_total = ctx->n_lines_total;
+  prm.n_blk_total = lay.n_blk_total;
+  prm.n_tiles_total = lay.n_tiles_total;
+  cudaStream_t st = (cudaStream_t)stream;
+  grad_prep_kernel<<<dim3(W, (ctx->n_lines_total + 127) / 128), 128, 0, st>>>(prm);
+  RBV_CUDA(cudaGetLastError());
+  grad_flux_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+  RBV_CUDA(cudaGetLastError());
+  grad_resid_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+  RBV_CUDA(cudaGetLastError());
+  grad_adjoint_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+  RBV_CUDA(cudaGetLastError());
+  grad_line_kernel<<<dim3(lay.n_tiles_total, W), kGradBlock, 0, st>>>(prm);
+  RBV_CUDA(cudaGetLastError());
+  grad_finalize_kernel<<<(W + 3) / 4, 128, 0, st>>>(prm);
+  RBV_CUDA(cudaGetLastError());
+  ctx->launches += 6;
   return RBV_OK;
 }
 

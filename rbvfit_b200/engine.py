@@ -202,6 +202,49 @@ class Engine:
                                         self._ws_bytes, self._stream()), "rbv_lnprob_batch")
         return out_t
 
+    def lnprob_grad_device(self, theta_t, apply_prior: bool, value_t=None, grad_t=None):
+        """DEVICE theta [W, ndim] -> (value [W], gradient [W, ndim]) DEVICE tensors (``rbv_lnprob_grad_batch``):
+        lnprob and its gradient with ``apply_prior``, lnlike and its gradient without; asynchronous."""
+        torch = _torch()
+        self._dev_tensor(theta_t, torch.float64, "theta")
+        if theta_t.dim() != 2 or theta_t.shape[1] != self.ndim:
+            raise ValueError(f"theta must be [W, {self.ndim}]")
+        W = int(theta_t.shape[0])
+        if value_t is None:
+            value_t = torch.empty(W, dtype=torch.float64, device=self.tdev)
+        if grad_t is None:
+            grad_t = torch.empty((W, self.ndim), dtype=torch.float64, device=self.tdev)
+        self._dev_tensor(value_t, torch.float64, "value", (W,))
+        self._dev_tensor(grad_t, torch.float64, "grad", (W, self.ndim))
+        nbytes = C.c_size_t(0)
+        check(self.lib.rbv_grad_workspace_bytes(self._h, max(W, 1), C.byref(nbytes)), "rbv_grad_workspace_bytes")
+        if getattr(self, "_grad_ws", None) is None or self._grad_ws.numel() < nbytes.value:
+            self._grad_ws = torch.empty(max(int(nbytes.value), 8), dtype=torch.uint8, device=self.tdev)
+        check(self.lib.rbv_lnprob_grad_batch(self._h, theta_t.data_ptr(), W, int(bool(apply_prior)),
+                                             value_t.data_ptr(), grad_t.data_ptr(), self._grad_ws.data_ptr(),
+                                             self._grad_ws.numel(), self._stream()), "rbv_lnprob_grad_batch")
+        return value_t, grad_t
+
+    def lnprob_grad_host(self, theta: np.ndarray, apply_prior: bool):
+        """HOST theta [W, ndim] -> HOST (value [W], gradient [W, ndim])."""
+        torch = _torch()
+        theta = np.ascontiguousarray(theta, dtype=np.float64)
+        if theta.ndim != 2:
+            raise ValueError("theta must be [W, ndim]")
+        th = torch.as_tensor(theta, device=self.tdev)
+        v, g = self.lnprob_grad_device(th, apply_prior)
+        return v.cpu().numpy(), g.cpu().numpy()
+
+    def voigt_h_grad(self, x: np.ndarray, a: np.ndarray):
+        """H, dH/dx, dH/da on a lattice (``rbv_voigt_h_grad``, test hook)."""
+        torch = _torch()
+        xs = torch.as_tensor(np.ascontiguousarray(x, dtype=np.float64).ravel(), device=self.tdev)
+        as_ = torch.as_tensor(np.ascontiguousarray(a, dtype=np.float64).ravel(), device=self.tdev)
+        H, Hx, Ha = (torch.empty_like(xs) for _ in range(3))
+        check(self.lib.rbv_voigt_h_grad(self._h, xs.data_ptr(), as_.data_ptr(), H.data_ptr(), Hx.data_ptr(),
+                                        Ha.data_ptr(), xs.numel(), self._stream()), "rbv_voigt_h_grad")
+        return tuple(t.cpu().numpy().reshape(np.shape(x)) for t in (H, Hx, Ha))
+
     def lnlike_host(self, theta: np.ndarray) -> np.ndarray:
         """HOST theta [W, ndim] -> HOST lnlike [W] (``rbv_lnlike_batch``: the same launch without the prior)."""
         torch = _torch()

@@ -26,6 +26,37 @@ def _weights(error):
     return inv_sigma2, log_inv_sigma2
 
 
+class _LnprobFunction:
+    """``torch.autograd.Function`` for ``GpuLikelihood.lnprob_torch``, built on first use (torch is imported lazily
+    throughout the package)."""
+    _cls = None
+
+    @classmethod
+    def apply(cls, theta_t, engine):
+        if cls._cls is None:
+            import torch
+
+            class LnprobFunction(torch.autograd.Function):
+                @staticmethod
+                def forward(ctx, theta, eng):
+                    rows = theta.detach()
+                    rows = (rows[None, :] if rows.dim() == 1 else rows).contiguous()
+                    value, grad = eng.lnprob_grad_device(rows, True)
+                    ctx.save_for_backward(grad)
+                    ctx.squeeze = theta.dim() == 1
+                    return value[0] if ctx.squeeze else value
+
+                @staticmethod
+                def backward(ctx, grad_output):
+                    (grad,) = ctx.saved_tensors
+                    if ctx.squeeze:
+                        return grad_output * grad[0], None
+                    return grad_output[:, None] * grad, None
+
+            cls._cls = LnprobFunction
+        return cls._cls.apply(theta_t, engine)
+
+
 class GpuLikelihood:
     """All instruments of one fit on one GPU."""
 
@@ -114,6 +145,33 @@ class GpuLikelihood:
     def lnprob_device(self, theta_t, out_t=None):
         """Device-resident variant (torch tensors in / out, asynchronous)."""
         return self.engine.lnprob_device(theta_t, out_t)
+
+    # ------------------------------------------------------------------ analytic gradient (DESIGN.md section 14)
+    def _value_and_grad(self, theta, apply_prior: bool):
+        theta = np.asarray(theta, dtype=np.float64)
+        if theta.ndim not in (1, 2) or theta.shape[-1] != self.ndim:
+            raise ValueError(f"theta must be ({self.ndim},) or (n, {self.ndim})")
+        if theta.ndim == 2 and theta.shape[0] == 0:
+            return np.zeros(0), np.zeros((0, self.ndim))
+        v, g = self.engine.lnprob_grad_host(np.atleast_2d(theta), apply_prior)
+        if theta.ndim == 1:
+            return float(v[0]), g[0]
+        return v, g
+
+    def lnprob_and_grad(self, theta):
+        """lnprob and its exact gradient from one device row per theta row: ``(ndim,) -> (float, (ndim,))``,
+        ``(n, ndim) -> ((n,), (n, ndim))``.  Rows outside the bounds give -inf and a zero gradient."""
+        return self._value_and_grad(theta, True)
+
+    def lnlike_and_grad(self, theta):
+        """lnlike (no prior: every row evaluated) and its exact gradient; shapes as ``lnprob_and_grad``."""
+        return self._value_and_grad(theta, False)
+
+    def lnprob_torch(self, theta_t):
+        """lnprob as a differentiable torch function of a DEVICE float64 tensor (``(n, ndim) -> (n,)``,
+        ``(ndim,) -> 0-d``): the forward pass is one ``rbv_lnprob_grad_batch`` launch, the backward pass scales the
+        saved gradient by ``grad_output``."""
+        return _LnprobFunction.apply(theta_t, self.engine)
 
     def set_far_field(self, mode: str = "chebyshev"):
         """``"chebyshev"`` (default): the summed far wings (lines >= 24 Doppler widths away) of each 1024-pixel

@@ -120,14 +120,26 @@ class vfit:
         return self._like.lnlike(theta)
 
     # ------------------------------------------------------------------ optimiser (vfit_mcmc.py:355-360)
-    def optimize_guess(self, theta):
+    def optimize_guess(self, theta, gradient="fd"):
         """L-BFGS-B on -lnprob with scipy's 2-point finite differences (absolute step 1e-8, flipped at the
         upper bound), exactly what ``op.minimize(nll, theta, method='L-BFGS-B', bounds=bounds)`` does -- but
         f(x) and its ndim forward-difference probes are ONE device batch per iteration instead of ndim+1
-        serial calls."""
+        serial calls.  ``gradient="device"``: f and its exact gradient from one device row per call
+        (``rbv_lnprob_grad_batch``)."""
         import scipy.optimize as op
+        if gradient not in ("fd", "device"):
+            raise ValueError("gradient must be 'fd' or 'device'")
         lb, ub = self.lb.astype(float), self.ub.astype(float)
         h = 1e-8
+
+        if gradient == "device":
+            def fun_and_grad(x):
+                v, g = self._like.lnprob_and_grad(np.asarray(x, dtype=np.float64))
+                return -v, -g
+
+            result = op.minimize(fun_and_grad, np.asarray(theta, dtype=np.float64), jac=True, method="L-BFGS-B",
+                                 bounds=list(zip(lb, ub)))
+            return result.x
 
         def fun_and_grad(x):
             x = np.asarray(x, dtype=np.float64)
@@ -152,11 +164,14 @@ class vfit:
         chi2 = -2.0 * ll + const
         return np.where(np.isfinite(chi2), chi2, 1e10)            # the reference returns 1e10 when evaluation fails
 
-    def fit_quick(self, verbose=True):
+    def fit_quick(self, verbose=True, gradient="fd"):
         """Deterministic chi^2 fit (L-BFGS-B, maxfun 5000) with finite-difference 1-sigma errors -- same
         objective, optimiser, step rule and fallbacks as core/quick_fit_interface.py:10-128; the objective, its
-        gradient probes and the 2 ndim + 1 curvature probes are device batches."""
+        gradient probes and the 2 ndim + 1 curvature probes are device batches.  ``gradient="device"``: chi^2 and
+        its exact gradient (-2 d lnlike) from one device row per call; the error bars keep the rule above."""
         import scipy.optimize as op
+        if gradient not in ("fd", "device"):
+            raise ValueError("gradient must be 'fd' or 'device'")
         self.mcmc_flag = False
         lb, ub = self.lb.astype(float), self.ub.astype(float)
         h = 1e-8
@@ -168,6 +183,17 @@ class vfit:
             steps[x + h > ub] = -h
             vals = self._chi2_batch(np.vstack([x, x[None, :] + np.diag(steps)]))
             return vals[0], (vals[1:] - vals[0]) / steps
+
+        if gradient == "device":
+            const = sum(float(np.sum(np.asarray(d["log_inv_sigma2"], dtype=np.float64)))
+                        for d in self.instrument_data.values())
+
+            def fun_and_grad(x):      # noqa: F811 -- the exact-gradient objective replaces the FD one
+                ll, g = self._like.lnlike_and_grad(np.asarray(x, dtype=np.float64))
+                chi2 = -2.0 * ll + const
+                if not np.isfinite(chi2):
+                    return 1e10, np.zeros_like(g)          # the reference returns 1e10 when evaluation fails
+                return chi2, -2.0 * g
 
         try:
             result = op.minimize(fun_and_grad, theta0, jac=True, bounds=list(zip(lb, ub)), method="L-BFGS-B",
