@@ -354,6 +354,24 @@ int rbv_grad_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* bytes
 int rbv_lnprob_grad_batch(RbvContext* ctx, const double* theta, int n_walkers, int apply_prior, double* value,
                           double* grad, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Model Jacobian and Gauss-Newton (Fisher) matrix of vfit.lnlike (DESIGN.md section 15), forward mode: one column
+ * per parameter, the LSF applied to each column, the weighted Gram reduction J^T W J.  Same forward pass as
+ * rbv_lnprob_grad_batch; FP64 always (ignores rbv_set_precision / rbv_set_farfield).  NaN where the forward model
+ * gives NaN (b <= 0, NaN theta).  RBV_EINVAL for voigt_method = RBV_VOIGT_FAST, more than 16 instruments or
+ * ndim < 3 * n_components; RBV_ESTATE before rbv_add_instrument / rbv_set_bounds; RBV_ENOMEM when the workspace is
+ * short.  Each row's results are bit-identical whatever the batch size or the row's position in it.  Asynchronous.
+ * Workspace: rbv_fisher_workspace_bytes() (about 2 * 3C * P doubles per walker; no initialisation needed). */
+int rbv_fisher_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* bytes);
+/* vfit.lnlike (no prior: every row evaluated, as rbv_lnlike_batch), its gradient and its Gauss-Newton matrix.
+ *   value  [W]; grad [W, ndim] = sum_p r_p dM_p/dtheta; fisher [W, ndim, ndim] = sum_inst sum_p w_p dM_p/dtheta_i dM_p/dtheta_j
+ *   (exactly symmetric; rows / columns beyond 3C are 0).  All DEVICE arrays.  RBV_ESTATE for a flux-only instrument. */
+int rbv_lnlike_fisher_batch(RbvContext* ctx, const double* theta, int n_walkers, double* value, double* grad,
+                            double* fisher, void* workspace, size_t workspace_bytes, void* stream);
+/* d(rbv_model_flux_batch with convolve = 1)/dtheta on instrument inst: out_jac DEVICE [W, ndim, n_pixels], rows beyond
+ * 3C = 0.  Same workspace as rbv_lnlike_fisher_batch; allowed on flux-only instruments. */
+int rbv_model_jacobian_batch(RbvContext* ctx, int inst, const double* theta, int n_walkers, double* out_jac,
+                             void* workspace, size_t workspace_bytes, void* stream);
+
 /* Test hook, like rbv_voigt_h: H = Re w(x + i a), dH/dx and dH/da on a lattice; all DEVICE arrays. */
 int rbv_voigt_h_grad(RbvContext* ctx, const double* x, const double* a, double* H, double* Hx, double* Ha, int n,
                      void* stream);

@@ -103,6 +103,11 @@ EXPORTS = {
     "rbv_grad_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_size_t)]),
     "rbv_lnprob_grad_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_size_t, C.c_void_p]),
+    "rbv_fisher_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_size_t)]),
+    "rbv_lnlike_fisher_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_void_p, C.c_size_t, C.c_void_p]),
+    "rbv_model_jacobian_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                           C.c_size_t, C.c_void_p]),
     "rbv_measure_fp64_peak": (C.c_int, [C.c_void_p, C.c_double, C.POINTER(C.c_double)]),
     "rbv_selftest_rcp": (C.c_int, [C.c_void_p, C.POINTER(C.c_double)]),
     "rbv_last_error": (C.c_char_p, []),

@@ -1062,6 +1062,7 @@ __global__ void __launch_bounds__(128) finalize_stream_kernel(const LaunchParams
 }  // namespace rbv
 #include "rbv_stream.cuh"   // warp-autonomous streaming form of the lnprob kernel (big batches)
 #include "rbv_grad.cuh"     // analytic gradient of lnprob / lnlike (forward + adjoint pass)
+#include "rbv_fisher.cuh"   // model Jacobian and Gauss-Newton matrix of lnlike (forward mode per column)
 namespace rbv {
 
 // ------------------------------------------------------------------------------------------ small kernels
@@ -1317,6 +1318,7 @@ struct HostInst {
   std::vector<double> taps;  // LSF taps as applied by the reference (normalised if requested), length K
   double* d_taps = nullptr;  // flipped + zero-padded copy on the device (rebuilt when R changes)
   double* d_grad_cum = nullptr;   // [2K] prefix / suffix sums of the flipped taps (gradient path, built on first use)
+  int* d_fisher_order = nullptr;  // [L] line indices sorted by component, stable (Jacobian path; in owned)
   std::vector<void*> owned;  // device allocations owned by the library for this instrument
 };
 
@@ -1791,6 +1793,12 @@ int rbv_add_instrument(RbvContext* ctx, const RbvLineTable* lt, const RbvSpectru
   RBV_CUDA(upload(&d_z, lt->zfac, (size_t)I.L));     hi.owned.push_back(d_z);
   RBV_CUDA(upload(&d_c, lt->comp, (size_t)I.L));     hi.owned.push_back(d_c);
   I.lambda0 = d_l0; I.gamma = d_g; I.f = d_f; I.zfac = d_z; I.comp = d_c;
+  {
+    std::vector<int> order(I.L);
+    for (int l = 0; l < I.L; ++l) order[l] = l;
+    std::stable_sort(order.begin(), order.end(), [lt](int x, int y) { return lt->comp[x] < lt->comp[y]; });
+    RBV_CUDA(upload(&hi.d_fisher_order, order.data(), order.size())); hi.owned.push_back(hi.d_fisher_order);
+  }
 
   reciprocal_kernel<<<(I.P + 255) / 256, 256>>>(sp->wave, sp->inv_wave, I.P);
   RBV_CUDA(cudaGetLastError());
@@ -3214,6 +3222,160 @@ int rbv_lnprob_grad_batch(RbvContext* ctx, const double* theta, int W, int apply
   grad_finalize_kernel<<<(W + 3) / 4, 128, 0, st>>>(prm);
   RBV_CUDA(cudaGetLastError());
   ctx->launches += 6;
+  return RBV_OK;
+}
+
+// ------------------------------------------------------------------------------------------ Jacobian / Fisher
+// Workspace of rbv_lnlike_fisher_batch and rbv_model_jacobian_batch (byte offsets, 256-byte aligned): the forward
+// buffers of the gradient path plus the columns JF, JM and the Gram partials.
+struct FisherLayout {
+  size_t oob, lc, F, r, pval, JF, JM, pgram, total;
+  int n_blk_total, n_tiles_total, ncol, npart;
+};
+static FisherLayout fisher_layout(const RbvContext* ctx, int W, GradInst* gi) {
+  const GradLayout g = grad_layout(ctx, 0, gi);
+  FisherLayout L;
+  memset(&L, 0, sizeof(L));
+  L.n_blk_total = g.n_blk_total;
+  L.n_tiles_total = g.n_tiles_total;
+  for (auto& hi : ctx->inst) L.ncol = std::max(L.ncol, 3 * hi.dev.C);
+  L.npart = L.ncol * (L.ncol + 1) / 2 + L.ncol;
+  auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
+  const size_t Wz = (size_t)std::max(W, 1), px = (size_t)g.n_blk_total * kGradBlock;
+  size_t off = 0;
+  L.oob = off;   off = al(off + Wz * sizeof(int));
+  L.lc = off;    off = al(off + Wz * ctx->n_lines_total * LC_STRIDE * sizeof(double));
+  L.F = off;     off = al(off + Wz * px * sizeof(double));
+  L.r = off;     off = al(off + Wz * px * sizeof(double));
+  L.pval = off;  off = al(off + Wz * g.n_blk_total * sizeof(double));
+  L.JF = off;    off = al(off + Wz * L.ncol * px * sizeof(double));
+  L.JM = off;    off = al(off + Wz * L.ncol * px * sizeof(double));
+  L.pgram = off; off = al(off + Wz * g.n_tiles_total * L.npart * sizeof(double));
+  L.total = off;
+  return L;
+}
+
+int rbv_fisher_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* bytes) {
+  if (!ctx || !bytes || n_walkers < 0) return fail(RBV_EINVAL, "rbv_fisher_workspace_bytes: bad argument");
+  *bytes = fisher_layout(ctx, n_walkers, nullptr).total;
+  return RBV_OK;
+}
+
+// Checks shared by both entry points, the parameter block, and the launches up to JF / JM:
+// prep -> flux [-> resid] -> columns [-> LSF]
+static int fisher_forward(RbvContext* ctx, const char* who, const double* theta, int W, bool with_resid,
+                          void* workspace, size_t workspace_bytes, cudaStream_t st, FisherParams& fp,
+                          FisherLayout& lay) {
+  if (ctx->inst.empty()) return fail(RBV_ESTATE, std::string(who) + ": no instrument added");
+  if (ctx->ndim == 0) return fail(RBV_ESTATE, std::string(who) + ": bounds not set (rbv_set_bounds)");
+  if (ctx->inst.size() > (size_t)kMaxInst)
+    return fail(RBV_EINVAL, std::string(who) + ": at most 16 instruments in a joint fit");
+  for (auto& hi : ctx->inst) {
+    if (3 * hi.dev.C > ctx->ndim) return fail(RBV_EINVAL, std::string(who) + ": ndim smaller than 3 * n_components");
+    if (hi.dev.method != RBV_VOIGT_WOFZ)
+      return fail(RBV_EINVAL, std::string(who) + ": no Jacobian for voigt_method='fast' (Tepper-Garcia)");
+    if (with_resid && (!hi.dev.flux || !hi.dev.inv_sigma2 || !hi.dev.log_inv_sigma2))
+      return fail(RBV_ESTATE, std::string(who) + ": an instrument has no observed spectrum (flux-only instrument)");
+  }
+  memset(&fp, 0, sizeof(fp));
+  GradParams& prm = fp.gp;
+  lay = fisher_layout(ctx, W, prm.gi);
+  if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, std::string(who) + ": workspace too small");
+  const size_t smem = (size_t)(lay.ncol + 2) * kFisherChunk * sizeof(double);
+  if (smem > (size_t)ctx->max_dyn_smem) return fail(RBV_EINVAL, std::string(who) + ": too many components");
+  RBV_ON_DEVICE(ctx);
+  if (smem > 48 * 1024)
+    RBV_CUDA(cudaFuncSetAttribute(fisher_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  bool any_lsf = false;
+  for (size_t k = 0; k < ctx->inst.size(); ++k) {
+    const HostInst& hi = ctx->inst[k];
+    fp.order[k] = hi.d_fisher_order;
+    fp.has_lsf[k] = !(hi.taps.size() == 1 && hi.taps[0] == 1.0);
+    any_lsf = any_lsf || fp.has_lsf[k];
+  }
+  char* ws = (char*)workspace;
+  prm.inst = ctx->d_inst;
+  prm.theta = theta;
+  prm.core_tab = ctx->d_core_tab;
+  prm.oob = (int*)(ws + lay.oob);
+  prm.lc = (double*)(ws + lay.lc);
+  prm.F = (double*)(ws + lay.F);
+  prm.r = (double*)(ws + lay.r);
+  prm.pval = (double*)(ws + lay.pval);
+  prm.W = W;
+  prm.ndim = ctx->ndim;
+  prm.n_inst = (int)ctx->inst.size();
+  prm.n_lines_total = ctx->n_lines_total;
+  prm.n_blk_total = lay.n_blk_total;
+  prm.n_tiles_total = lay.n_tiles_total;
+  fp.ncol = lay.ncol;
+  fp.npart = lay.npart;
+  fp.col_stride = (long long)lay.n_blk_total * kGradBlock;
+  fp.JF = (double*)(ws + lay.JF);
+  fp.JM = (double*)(ws + lay.JM);
+  fp.pgram = (double*)(ws + lay.pgram);
+  grad_prep_kernel<<<dim3(W, (ctx->n_lines_total + 127) / 128), 128, 0, st>>>(prm);
+  RBV_CUDA(cudaGetLastError());
+  grad_flux_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+  RBV_CUDA(cudaGetLastError());
+  ctx->launches += 2;
+  if (with_resid) {
+    grad_resid_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+    RBV_CUDA(cudaGetLastError());
+    ctx->launches++;
+  }
+  fisher_col_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(fp);
+  RBV_CUDA(cudaGetLastError());
+  ctx->launches++;
+  if (any_lsf) {
+    fisher_lsf_kernel<<<dim3(lay.n_blk_total, lay.ncol, W), kGradBlock, 0, st>>>(fp);
+    RBV_CUDA(cudaGetLastError());
+    ctx->launches++;
+  }
+  return RBV_OK;
+}
+
+int rbv_lnlike_fisher_batch(RbvContext* ctx, const double* theta, int W, double* value, double* grad, double* fisher,
+                            void* workspace, size_t workspace_bytes, void* stream) {
+  const char* who = "rbv_lnlike_fisher_batch";
+  if (!ctx || !theta || !value || !grad || !fisher) return fail(RBV_EINVAL, std::string(who) + ": null argument");
+  if (W < 0) return fail(RBV_EINVAL, std::string(who) + ": negative n_walkers");
+  if (W == 0) return RBV_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  FisherParams fp;
+  FisherLayout lay;
+  const int rc = fisher_forward(ctx, who, theta, W, true, workspace, workspace_bytes, st, fp, lay);
+  if (rc != RBV_OK) return rc;
+  fp.gp.value = value;
+  fp.gp.grad = grad;
+  fp.fisher = fisher;
+  fisher_gram_kernel<<<dim3(lay.n_tiles_total, W), kGradBlock, (lay.ncol + 2) * kFisherChunk * sizeof(double), st>>>(
+      fp);
+  RBV_CUDA(cudaGetLastError());
+  fisher_finalize_kernel<<<(W + 3) / 4, 128, 0, st>>>(fp);
+  RBV_CUDA(cudaGetLastError());
+  ctx->launches += 2;
+  return RBV_OK;
+}
+
+int rbv_model_jacobian_batch(RbvContext* ctx, int inst, const double* theta, int W, double* out_jac, void* workspace,
+                             size_t workspace_bytes, void* stream) {
+  const char* who = "rbv_model_jacobian_batch";
+  if (!ctx || !theta || !out_jac) return fail(RBV_EINVAL, std::string(who) + ": null argument");
+  if (inst < 0 || inst >= (int)ctx->inst.size()) return fail(RBV_EINVAL, std::string(who) + ": bad instrument index");
+  if (W < 0) return fail(RBV_EINVAL, std::string(who) + ": negative n_walkers");
+  if (W == 0) return RBV_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  FisherParams fp;
+  FisherLayout lay;
+  const int rc = fisher_forward(ctx, who, theta, W, false, workspace, workspace_bytes, st, fp, lay);
+  if (rc != RBV_OK) return rc;
+  fp.jac = out_jac;
+  fp.jac_inst = inst;
+  const int P = ctx->inst[inst].dev.P;
+  fisher_jac_out_kernel<<<dim3((P + kGradBlock - 1) / kGradBlock, ctx->ndim, W), kGradBlock, 0, st>>>(fp);
+  RBV_CUDA(cudaGetLastError());
+  ctx->launches++;
   return RBV_OK;
 }
 

@@ -235,6 +235,86 @@ class Engine:
         v, g = self.lnprob_grad_device(th, apply_prior)
         return v.cpu().numpy(), g.cpu().numpy()
 
+    # host calls split a batch so that the Jacobian workspace (about 2 * 3C * P doubles per row) stays below this
+    fisher_chunk_bytes = 1 << 30
+
+    def _fisher_ws(self, W: int):
+        torch = _torch()
+        nbytes = C.c_size_t(0)
+        check(self.lib.rbv_fisher_workspace_bytes(self._h, max(W, 1), C.byref(nbytes)), "rbv_fisher_workspace_bytes")
+        if getattr(self, "_fisher_ws_t", None) is None or self._fisher_ws_t.numel() < nbytes.value:
+            self._fisher_ws_t = None
+            self._fisher_ws_t = torch.empty(max(int(nbytes.value), 8), dtype=torch.uint8, device=self.tdev)
+        return self._fisher_ws_t
+
+    def _fisher_rows_per_chunk(self) -> int:
+        one = C.c_size_t(0)
+        check(self.lib.rbv_fisher_workspace_bytes(self._h, 1, C.byref(one)), "rbv_fisher_workspace_bytes")
+        return max(1, int(self.fisher_chunk_bytes // max(int(one.value), 1)))
+
+    def lnlike_fisher_device(self, theta_t, value_t=None, grad_t=None, fisher_t=None):
+        """DEVICE theta [W, ndim] -> (lnlike [W], gradient [W, ndim], Gauss-Newton matrix [W, ndim, ndim]) DEVICE
+        tensors (``rbv_lnlike_fisher_batch``); asynchronous."""
+        torch = _torch()
+        self._dev_tensor(theta_t, torch.float64, "theta")
+        if theta_t.dim() != 2 or theta_t.shape[1] != self.ndim:
+            raise ValueError(f"theta must be [W, {self.ndim}]")
+        W, n = int(theta_t.shape[0]), self.ndim
+        if value_t is None:
+            value_t = torch.empty(W, dtype=torch.float64, device=self.tdev)
+        if grad_t is None:
+            grad_t = torch.empty((W, n), dtype=torch.float64, device=self.tdev)
+        if fisher_t is None:
+            fisher_t = torch.empty((W, n, n), dtype=torch.float64, device=self.tdev)
+        self._dev_tensor(value_t, torch.float64, "value", (W,))
+        self._dev_tensor(grad_t, torch.float64, "grad", (W, n))
+        self._dev_tensor(fisher_t, torch.float64, "fisher", (W, n, n))
+        ws = self._fisher_ws(W)
+        check(self.lib.rbv_lnlike_fisher_batch(self._h, theta_t.data_ptr(), W, value_t.data_ptr(), grad_t.data_ptr(),
+                                               fisher_t.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()),
+              "rbv_lnlike_fisher_batch")
+        return value_t, grad_t, fisher_t
+
+    def lnlike_fisher_host(self, theta: np.ndarray):
+        """HOST theta [W, ndim] -> HOST (lnlike [W], gradient [W, ndim], Gauss-Newton matrix [W, ndim, ndim]), in
+        chunks of rows whose workspace stays below ``fisher_chunk_bytes`` (every row is reduced in an order of its
+        own, so the chunking does not change any result)."""
+        torch = _torch()
+        theta = np.ascontiguousarray(theta, dtype=np.float64)
+        if theta.ndim != 2:
+            raise ValueError("theta must be [W, ndim]")
+        W, n = theta.shape[0], self.ndim
+        value, grad, fisher = np.empty(W), np.empty((W, n)), np.empty((W, n, n))
+        step = self._fisher_rows_per_chunk()
+        for i in range(0, W, step):
+            th = torch.as_tensor(theta[i:i + step], device=self.tdev)
+            v, g, f = self.lnlike_fisher_device(th)
+            value[i:i + step], grad[i:i + step], fisher[i:i + step] = v.cpu().numpy(), g.cpu().numpy(), f.cpu().numpy()
+        return value, grad, fisher
+
+    def model_jacobian(self, inst: int, theta: np.ndarray) -> np.ndarray:
+        """HOST theta [W, ndim] -> HOST d(model flux)/d theta [W, ndim, P] of instrument ``inst``
+        (``rbv_model_jacobian_batch``: the LSF-convolved model of ``model_flux``), in chunks as
+        ``lnlike_fisher_host``."""
+        torch = _torch()
+        theta = np.ascontiguousarray(theta, dtype=np.float64)
+        if theta.ndim != 2 or theta.shape[1] != self.ndim:
+            raise ValueError(f"theta must be [W, {self.ndim}]")
+        if not 0 <= inst < len(self.pixels):
+            raise ValueError("bad instrument index")
+        W, n, P = theta.shape[0], self.ndim, self.pixels[inst]
+        out = np.empty((W, n, P))
+        step = self._fisher_rows_per_chunk()
+        for i in range(0, W, step):
+            th = torch.as_tensor(theta[i:i + step], device=self.tdev)
+            w = th.shape[0]
+            jac = torch.empty((w, n, P), dtype=torch.float64, device=self.tdev)
+            ws = self._fisher_ws(w)
+            check(self.lib.rbv_model_jacobian_batch(self._h, inst, th.data_ptr(), w, jac.data_ptr(), ws.data_ptr(),
+                                                    ws.numel(), self._stream()), "rbv_model_jacobian_batch")
+            out[i:i + step] = jac.cpu().numpy()
+        return out
+
     def voigt_h_grad(self, x: np.ndarray, a: np.ndarray):
         """H, dH/dx, dH/da on a lattice (``rbv_voigt_h_grad``, test hook)."""
         torch = _torch()

@@ -173,6 +173,36 @@ class GpuLikelihood:
         saved gradient by ``grad_output``."""
         return _LnprobFunction.apply(theta_t, self.engine)
 
+    # ------------------------------------------------------------------ Jacobian / Fisher (DESIGN.md section 15)
+    def _rows(self, theta):
+        theta = np.asarray(theta, dtype=np.float64)
+        if theta.ndim not in (1, 2) or theta.shape[-1] != self.ndim:
+            raise ValueError(f"theta must be ({self.ndim},) or (n, {self.ndim})")
+        return theta
+
+    def lnlike_and_fisher(self, theta):
+        """lnlike (no prior), its gradient and its Gauss-Newton matrix sum_p w_p dM_p/dtheta_i dM_p/dtheta_j from one
+        device row per theta row: ``(ndim,) -> (float, (ndim,), (ndim, ndim))``,
+        ``(n, ndim) -> ((n,), (n, ndim), (n, ndim, ndim))``.  -2 lnlike is chi^2 up to a constant, so the inverse
+        of the matrix is the Delta chi^2 = 1 covariance of the parameters."""
+        theta = self._rows(theta)
+        if theta.ndim == 2 and theta.shape[0] == 0:
+            return np.zeros(0), np.zeros((0, self.ndim)), np.zeros((0, self.ndim, self.ndim))
+        v, g, f = self.engine.lnlike_fisher_host(np.atleast_2d(theta))
+        if theta.ndim == 1:
+            return float(v[0]), g[0], f[0]
+        return v, g, f
+
+    def model_jacobian(self, theta, instrument):
+        """d(model flux)/dtheta of one instrument (name or index), LSF applied: ``(ndim,) -> [P, ndim]``,
+        ``(n, ndim) -> [n, P, ndim]`` (the layout of scipy's ``least_squares``)."""
+        theta = self._rows(theta)
+        inst = self.names.index(instrument) if isinstance(instrument, str) else int(instrument)
+        if theta.ndim == 2 and theta.shape[0] == 0:
+            return np.zeros((0, self.pixels[inst], self.ndim))
+        jac = np.swapaxes(self.engine.model_jacobian(inst, np.atleast_2d(theta)), 1, 2)
+        return jac[0] if theta.ndim == 1 else jac
+
     def set_far_field(self, mode: str = "chebyshev"):
         """``"chebyshev"`` (default): the summed far wings (lines >= 24 Doppler widths away) of each 1024-pixel
         super-chunk are evaluated at 8 Chebyshev nodes and interpolated; a line takes part only where an

@@ -164,14 +164,25 @@ class vfit:
         chi2 = -2.0 * ll + const
         return np.where(np.isfinite(chi2), chi2, 1e10)            # the reference returns 1e10 when evaluation fails
 
-    def fit_quick(self, verbose=True, gradient="fd"):
+    def fit_quick(self, verbose=True, gradient="fd", method="lbfgsb"):
         """Deterministic chi^2 fit (L-BFGS-B, maxfun 5000) with finite-difference 1-sigma errors -- same
         objective, optimiser, step rule and fallbacks as core/quick_fit_interface.py:10-128; the objective, its
         gradient probes and the 2 ndim + 1 curvature probes are device batches.  ``gradient="device"``: chi^2 and
-        its exact gradient (-2 d lnlike) from one device row per call; the error bars keep the rule above."""
+        its exact gradient (-2 d lnlike) from one device row per call; the error bars keep the rule above.
+
+        ``method="lm"``: bounded Levenberg-Marquardt (``rbvfit_b200.lm``) on the device's Gauss-Newton matrix, one
+        ``lnlike_and_fisher`` row per point evaluated; the errors are sqrt(diag) of the full covariance
+        (J^T W J)^-1 over the free parameters, also stored as ``theta_best_covariance`` (NaN for parameters pinned
+        on a bound or not constrained by the data).  ``gradient`` applies to L-BFGS-B only."""
         import scipy.optimize as op
         if gradient not in ("fd", "device"):
             raise ValueError("gradient must be 'fd' or 'device'")
+        if method not in ("lbfgsb", "lm"):
+            raise ValueError("method must be 'lbfgsb' or 'lm'")
+        if method == "lm":
+            if gradient != "fd":
+                raise ValueError("gradient applies to method='lbfgsb' only")
+            return self._fit_quick_lm(verbose)
         self.mcmc_flag = False
         lb, ub = self.lb.astype(float), self.ub.astype(float)
         h = 1e-8
@@ -217,6 +228,34 @@ class vfit:
                 print("WARNING: Some uncertainties are NaN")
         self.theta_best, self.theta_best_error = best, err
         return best, err
+
+    def _fit_quick_lm(self, verbose):
+        from .lm import levenberg_marquardt
+        self.mcmc_flag = False
+        res = levenberg_marquardt(self._like.lnlike_and_fisher, np.asarray(self.theta, dtype=np.float64),
+                                  self.lb.astype(float), self.ub.astype(float))
+        if res.status <= 0:
+            warnings.warn(f"Optimization may not have converged: {res.message}")
+        err = np.sqrt(np.diag(res.cov))
+        if verbose:
+            print("Quick fit completed")
+            if np.any(np.isnan(err)):
+                print("WARNING: Some uncertainties are NaN")
+        self.theta_best, self.theta_best_error, self.theta_best_covariance = res.x, err, res.cov
+        return res.x, err
+
+    def covariance(self, theta=None):
+        """Inverse Gauss-Newton matrix (J^T W J)^-1 at ``theta`` (default ``theta_best``, else ``theta``) from one
+        device row: the Delta chi^2 = 1 covariance over the free parameters, NaN rows / columns for parameters
+        pinned on a bound (gradient pointing out of the box) or not constrained by the data."""
+        from . import lm
+        if theta is None:
+            theta = getattr(self, "theta_best", None)
+            if theta is None:
+                theta = self.theta
+        theta = np.asarray(theta, dtype=np.float64)
+        _ll, g, F = self._like.lnlike_and_fisher(theta)
+        return lm.covariance(F, lm.free_set(theta, g, F, self.lb.astype(float), self.ub.astype(float)))
 
     # ------------------------------------------------------------------ walkers (vfit_mcmc.py:442-466)
     def _initialize_walkers(self, popt):
