@@ -372,6 +372,40 @@ int rbv_lnlike_fisher_batch(RbvContext* ctx, const double* theta, int n_walkers,
 int rbv_model_jacobian_batch(RbvContext* ctx, int inst, const double* theta, int n_walkers, double* out_jac,
                              void* workspace, size_t workspace_bytes, void* stream);
 
+/* Survey mode of rbv_lnlike_fisher_batch (DESIGN.md section 16): the context holds S sightlines with identical
+ * n_pixels, n_taps, n_lines and n_components (see rbv_lnprob_batch_sightlines); row w is evaluated against sightline
+ * w / walkers_per_sightline alone, and its results equal bit for bit those of rbv_lnlike_fisher_batch on a context
+ * holding that sightline only.  Any number of sightlines; the workspace grows with n_walkers only.  Errors as
+ * rbv_lnlike_fisher_batch, and RBV_EINVAL for mismatched sightline geometry or n_walkers != S * walkers_per_sightline.
+ * Asynchronous. */
+int rbv_fisher_workspace_bytes_sightlines(const RbvContext* ctx, int n_walkers, size_t* bytes);
+int rbv_lnlike_fisher_batch_sightlines(RbvContext* ctx, const double* theta, int n_walkers, int walkers_per_sightline,
+                                       double* value, double* grad, double* fisher, void* workspace,
+                                       size_t workspace_bytes, void* stream);
+
+/* Stopping rules of rbvfit_b200.lm.levenberg_marquardt: at most max_evals evaluations (>= 1); stop when an accepted
+ * step lowers chi^2 by at most ftol |chi^2| or when a step is at most xtol (|theta| + xtol) long. */
+typedef struct RbvLMControl {
+  int max_evals;
+  double ftol, xtol;
+} RbvLMControl;
+
+/* Bounded Levenberg-Marquardt fit of every sightline in [first, first + n) of a survey-mode context, with the rules of
+ * rbvfit_b200.lm.levenberg_marquardt, the context's bounds shared by all sightlines.  Each iteration is one
+ * survey-mode Fisher evaluation of the sightlines still iterating, one update kernel (a warp per sightline: step,
+ * accept / reject, damping) and a 4-byte read-back of the number still iterating.
+ *   theta   [n, ndim]        in: start (clipped into the bounds), out: best point
+ *   chi2    [n]              -2 lnlike at theta;  n_evals [n]: evaluations;  status [n]: lm.STATUS_*
+ *   cov     [n, ndim, ndim]  inv(F_ff) over the free set at theta, NaN rows / columns elsewhere
+ *   flags   [n]              bit 0: F_ff not positive definite at the end (cov left NaN)
+ * All DEVICE arrays.  A sightline's results depend on its own data only, not on n, first or the other sightlines.
+ * Errors as rbv_lnlike_fisher_batch_sightlines, and RBV_EINVAL for a bad [first, first + n) or control.  Returns
+ * after the run has finished (synchronises the stream). */
+int rbv_lm_workspace_bytes_sightlines(const RbvContext* ctx, int n_sightlines, size_t* bytes);
+int rbv_lm_run_sightlines(RbvContext* ctx, int first, int n, double* theta, const RbvLMControl* ctl, double* chi2,
+                          double* cov, int* n_evals, int* status, int* flags, void* workspace,
+                          size_t workspace_bytes, void* stream);
+
 /* Test hook, like rbv_voigt_h: H = Re w(x + i a), dH/dx and dH/da on a lattice; all DEVICE arrays. */
 int rbv_voigt_h_grad(RbvContext* ctx, const double* x, const double* a, double* H, double* Hx, double* Ha, int n,
                      void* stream);

@@ -33,6 +33,10 @@ class RbvSliceTuning(C.Structure):
                 ("n_batches", C.c_ulonglong)]
 
 
+class RbvLMControl(C.Structure):
+    _fields_ = [("max_evals", C.c_int), ("ftol", C.c_double), ("xtol", C.c_double)]
+
+
 class RbvChainSink(C.Structure):
     _fields_ = [("chain_host", C.c_void_p), ("lnprob_chain_host", C.c_void_p), ("ring_dev", C.c_void_p),
                 ("ring_pinned", C.c_void_p), ("block_steps", C.c_int)]
@@ -108,6 +112,13 @@ EXPORTS = {
                                           C.c_void_p, C.c_size_t, C.c_void_p]),
     "rbv_model_jacobian_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                            C.c_size_t, C.c_void_p]),
+    "rbv_fisher_workspace_bytes_sightlines": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_size_t)]),
+    "rbv_lnlike_fisher_batch_sightlines": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "rbv_lm_workspace_bytes_sightlines": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_size_t)]),
+    "rbv_lm_run_sightlines": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(RbvLMControl),
+                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_size_t, C.c_void_p]),
     "rbv_measure_fp64_peak": (C.c_int, [C.c_void_p, C.c_double, C.POINTER(C.c_double)]),
     "rbv_selftest_rcp": (C.c_int, [C.c_void_p, C.POINTER(C.c_double)]),
     "rbv_last_error": (C.c_char_p, []),

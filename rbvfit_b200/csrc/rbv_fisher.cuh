@@ -18,6 +18,8 @@
 //   fisher_jac_out_kernel  (256 px, row, walker)   rbv_model_jacobian_batch only: [W, ndim, P] out of JM / JF
 // Every reduction runs in an order fixed by the instrument geometry alone (no atomics): a row's results do not
 // depend on the batch size or on the position of the row in the batch.
+// Survey mode (SL = true, SlRows of rbv_grad.cuh): the same kernels with the geometry of one sightline and the
+// row's own instrument, so a row gives bit for bit what a one-instrument context of that sightline gives.
 #pragma once
 
 namespace rbv {
@@ -69,12 +71,15 @@ __device__ __forceinline__ void fisher_store(double* jf, long long stride, int C
   jf[(size_t)(2 * C + c) * stride] = mF * (u * sX / (kCkms + th[2 * C + c]));
 }
 
-__global__ void __launch_bounds__(kGradBlock) fisher_col_kernel(const FisherParams fp) {
+template <bool SL>
+__global__ void __launch_bounds__(kGradBlock) fisher_col_kernel(const FisherParams fp, const SlRows sl) {
   __shared__ double s_q[kGradLineChunk][2][kNQNear];
   const GradParams& prm = fp.gp;
   const int w = blockIdx.y, tid = threadIdx.x;
-  const int k = grad_inst_of_blk(prm, blockIdx.x);
-  const InstDev& I = prm.inst[k];
+  if (sl_skip<SL>(sl, w)) return;
+  const int k = SL ? 0 : grad_inst_of_blk(prm, blockIdx.x);
+  const int ki = sl_inst<SL>(sl, w, k);
+  const InstDev& I = prm.inst[ki];
   const int p = (blockIdx.x - prm.gi[k].blk_off) * kGradBlock + tid;
   const bool valid = p < I.P;
   const size_t pix = (size_t)blockIdx.x * kGradBlock + tid;
@@ -82,8 +87,8 @@ __global__ void __launch_bounds__(kGradBlock) fisher_col_kernel(const FisherPara
   const double mF = valid ? -prm.F[(size_t)w * fp.col_stride + pix] : 0.0;
   double* jf = fp.JF + (size_t)w * fp.ncol * fp.col_stride + pix;
   const double* th = prm.theta + (size_t)w * prm.ndim;
-  const double* lcw = prm.lc + ((size_t)w * prm.n_lines_total + I.line_base) * LC_STRIDE;
-  const int* ord = fp.order[k];
+  const double* lcw = prm.lc + ((size_t)w * prm.n_lines_total + (SL ? 0 : I.line_base)) * LC_STRIDE;
+  const int* ord = SL ? sl.order[ki] : fp.order[k];
   int c = 0;
   double sN = 0.0, sE = 0.0, sX = 0.0;
   for (int l0 = 0; l0 < I.L; l0 += kGradLineChunk) {
@@ -117,12 +122,15 @@ __global__ void __launch_bounds__(kGradBlock) fisher_col_kernel(const FisherPara
 }
 
 // JM = taps * JF per column, the expression grad_resid_kernel forms M with
-__global__ void __launch_bounds__(kGradBlock) fisher_lsf_kernel(const FisherParams fp) {
+template <bool SL>
+__global__ void __launch_bounds__(kGradBlock) fisher_lsf_kernel(const FisherParams fp, const SlRows sl) {
   const GradParams& prm = fp.gp;
   const int w = blockIdx.z, col = blockIdx.y;
-  const int k = grad_inst_of_blk(prm, blockIdx.x);
-  if (!fp.has_lsf[k]) return;
-  const InstDev& I = prm.inst[k];
+  if (sl_skip<SL>(sl, w)) return;
+  const int k = SL ? 0 : grad_inst_of_blk(prm, blockIdx.x);
+  const int ki = sl_inst<SL>(sl, w, k);
+  if (!(SL ? sl.has_lsf[ki] : fp.has_lsf[k])) return;
+  const InstDev& I = prm.inst[ki];
   const int p = (blockIdx.x - prm.gi[k].blk_off) * kGradBlock + threadIdx.x;
   if (p >= I.P) return;
   const size_t base = fisher_col_base(fp, w, col, k);
@@ -134,16 +142,19 @@ __global__ void __launch_bounds__(kGradBlock) fisher_lsf_kernel(const FisherPara
 }
 
 // per 1024-pixel tile: sum_p w_p J_i J_j (i <= j) and sum_p r_p J_i, pixels in ascending order
-__global__ void __launch_bounds__(kGradBlock) fisher_gram_kernel(const FisherParams fp) {
+template <bool SL>
+__global__ void __launch_bounds__(kGradBlock) fisher_gram_kernel(const FisherParams fp, const SlRows sl) {
   extern __shared__ double s_j[];   // [ncol][kFisherChunk] columns, then weights, then residuals
   const GradParams& prm = fp.gp;
   const int w = blockIdx.y, tid = threadIdx.x;
-  const int k = grad_inst_of_tile(prm, blockIdx.x);
-  const InstDev& I = prm.inst[k];
+  if (sl_skip<SL>(sl, w)) return;
+  const int k = SL ? 0 : grad_inst_of_tile(prm, blockIdx.x);
+  const int ki = sl_inst<SL>(sl, w, k);
+  const InstDev& I = prm.inst[ki];
   const int p0 = (blockIdx.x - prm.gi[k].tile_off) * kGradTile;
   const int np = min(kGradTile, I.P - p0);
   const int ncol = fp.ncol, ntri = ncol * (ncol + 1) / 2;
-  const double* J = (fp.has_lsf[k] ? fp.JM : fp.JF) + fisher_col_base(fp, w, 0, k) + p0;
+  const double* J = ((SL ? sl.has_lsf[ki] : fp.has_lsf[k]) ? fp.JM : fp.JF) + fisher_col_base(fp, w, 0, k) + p0;
   const double* r = prm.r + (size_t)w * fp.col_stride + (size_t)prm.gi[k].blk_off * kGradBlock + p0;
   double* s_w = s_j + ncol * kFisherChunk;
   double* s_r = s_w + kFisherChunk;
@@ -180,10 +191,11 @@ __global__ void __launch_bounds__(kGradBlock) fisher_gram_kernel(const FisherPar
 }
 
 // one warp per walker: value as grad_finalize_kernel; gradient and the mirrored matrix from the tile partials
-__global__ void __launch_bounds__(128) fisher_finalize_kernel(const FisherParams fp) {
+template <bool SL>
+__global__ void __launch_bounds__(128) fisher_finalize_kernel(const FisherParams fp, const SlRows sl) {
   const GradParams& prm = fp.gp;
   const int w = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (w >= prm.W) return;
+  if (w >= prm.W || sl_skip<SL>(sl, w)) return;
   const int ndim = prm.ndim, ncol = fp.ncol, ntri = ncol * (ncol + 1) / 2;
   double* row = prm.grad + (size_t)w * ndim;
   double* F = fp.fisher + (size_t)w * ndim * ndim;
@@ -192,7 +204,7 @@ __global__ void __launch_bounds__(128) fisher_finalize_kernel(const FisherParams
     if (x / ndim >= ncol || x % ndim >= ncol) F[x] = 0.0;
   double total = 0.0;
   for (int k = 0; k < prm.n_inst; ++k) {
-    const InstDev& I = prm.inst[k];
+    const InstDev& I = prm.inst[sl_inst<SL>(sl, w, k)];
     const GradInst& gi = prm.gi[k];
     double s = 0.0;
     const double* pv = prm.pval + (size_t)w * prm.n_blk_total + gi.blk_off;

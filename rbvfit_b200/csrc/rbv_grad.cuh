@@ -60,6 +60,28 @@ struct GradParams {
   int W, ndim, n_inst, n_lines_total, n_blk_total, n_tiles_total;
 };
 
+// Survey mode of the forward and Fisher kernels (template parameter SL): row w is evaluated against instrument
+// inst0 + w / wps alone, with the geometry of one instrument (gi[0], n_inst = 1, its lines at lc offset 0), so every
+// buffer and grid is sized for one sightline whatever the number of sightlines.  The per-instrument tables that the
+// joint fit passes as kernel parameters (at most kMaxInst) come from device arrays indexed by instrument.
+struct SlRows {
+  int wps;                  // rows per sightline
+  int inst0;                // instrument of row 0
+  const int* active;        // [W] or NULL: a row with active[w] == 0 returns at kernel entry
+  const int* const* order;  // [n_inst] FisherParams::order of each instrument
+  const int* has_lsf;       // [n_inst] FisherParams::has_lsf of each instrument
+};
+
+template <bool SL>
+__device__ __forceinline__ bool sl_skip(const SlRows& sl, int w) {
+  return SL && sl.active != nullptr && !sl.active[w];
+}
+// instrument of row w; k is the joint fit's instrument (from the block / tile / line index)
+template <bool SL>
+__device__ __forceinline__ int sl_inst(const SlRows& sl, int w, int k) {
+  return SL ? sl.inst0 + w / sl.wps : k;
+}
+
 // ------------------------------------------------------------------------------------------ H and its derivatives
 // q_p(a^2) and dq_p/d(a^2), p = 1..kNQNear, unscaled (kappa = 1)
 __device__ __forceinline__ void asym_coef_grad(double a2, double* q, double* qd) {
@@ -232,8 +254,10 @@ __device__ __forceinline__ int grad_inst_of_blk(const GradParams& prm, int blk) 
 }
 
 // prior flag + per-line constants (the record prep_kernel writes: A, B, a^2, a, S, kappa-scaled series)
-__global__ void __launch_bounds__(128) grad_prep_kernel(const GradParams prm) {
+template <bool SL>
+__global__ void __launch_bounds__(128) grad_prep_kernel(const GradParams prm, const SlRows sl) {
   const int w = blockIdx.x;
+  if (sl_skip<SL>(sl, w)) return;
   const double* th = prm.theta + (size_t)w * prm.ndim;
   if (blockIdx.y == 0) {
     int bad = 0;
@@ -245,10 +269,11 @@ __global__ void __launch_bounds__(128) grad_prep_kernel(const GradParams prm) {
   const int gl = blockIdx.y * blockDim.x + threadIdx.x;
   if (gl >= prm.n_lines_total) return;
   int k = 0;
-  while (k + 1 < prm.n_inst && gl >= prm.inst[k + 1].line_base) ++k;
+  if (SL) k = sl_inst<SL>(sl, w, 0);
+  else while (k + 1 < prm.n_inst && gl >= prm.inst[k + 1].line_base) ++k;
   const InstDev& I = prm.inst[k];
   double lc[LC_STRIDE];
-  prep_line_wofz(I, gl - I.line_base, th, lc);
+  prep_line_wofz(I, SL ? gl : gl - I.line_base, th, lc);
 #pragma unroll
   for (int p = 0; p < kNQNear; ++p) lc[LC_Q + p] = asym_coef(p + 1, lc[LC_A2], lc[LC_AUX]);
   double* dst = prm.lc + ((size_t)w * prm.n_lines_total + gl) * LC_STRIDE;
@@ -257,15 +282,17 @@ __global__ void __launch_bounds__(128) grad_prep_kernel(const GradParams prm) {
 }
 
 // tau over every line, directly, then F = exp(-tau)
-__global__ void __launch_bounds__(kGradBlock) grad_flux_kernel(const GradParams prm) {
+template <bool SL>
+__global__ void __launch_bounds__(kGradBlock) grad_flux_kernel(const GradParams prm, const SlRows sl) {
   const int w = blockIdx.y;
+  if (sl_skip<SL>(sl, w)) return;
   if (prm.oob[w]) return;
-  const int k = grad_inst_of_blk(prm, blockIdx.x);
-  const InstDev& I = prm.inst[k];
+  const int k = SL ? 0 : grad_inst_of_blk(prm, blockIdx.x);
+  const InstDev& I = prm.inst[sl_inst<SL>(sl, w, k)];
   const int p = (blockIdx.x - prm.gi[k].blk_off) * kGradBlock + threadIdx.x;
   if (p >= I.P) return;
   const double u = __ldg(I.inv_wave + p);
-  const double* lcw = prm.lc + ((size_t)w * prm.n_lines_total + I.line_base) * LC_STRIDE;
+  const double* lcw = prm.lc + ((size_t)w * prm.n_lines_total + (SL ? 0 : I.line_base)) * LC_STRIDE;
   double tau = 0.0;
   for (int l = 0; l < I.L; ++l) {
     const double* lc = lcw + l * LC_STRIDE;
@@ -282,12 +309,14 @@ __global__ void __launch_bounds__(kGradBlock) grad_flux_kernel(const GradParams 
 }
 
 // M_p = sum_m taps_rev[m] F[clamp(p - h + m)], r_p = (D_p - M_p) w_p, chi^2 partial of the block
-__global__ void __launch_bounds__(kGradBlock) grad_resid_kernel(const GradParams prm) {
+template <bool SL>
+__global__ void __launch_bounds__(kGradBlock) grad_resid_kernel(const GradParams prm, const SlRows sl) {
   __shared__ double s_red[kGradBlock / 32];
   const int w = blockIdx.y;
+  if (sl_skip<SL>(sl, w)) return;
   if (prm.oob[w]) return;
-  const int k = grad_inst_of_blk(prm, blockIdx.x);
-  const InstDev& I = prm.inst[k];
+  const int k = SL ? 0 : grad_inst_of_blk(prm, blockIdx.x);
+  const InstDev& I = prm.inst[sl_inst<SL>(sl, w, k)];
   const int p = (blockIdx.x - prm.gi[k].blk_off) * kGradBlock + threadIdx.x;
   const size_t base = (size_t)w * prm.n_blk_total * kGradBlock + (size_t)prm.gi[k].blk_off * kGradBlock;
   double part = 0.0;

@@ -1063,6 +1063,7 @@ __global__ void __launch_bounds__(128) finalize_stream_kernel(const LaunchParams
 #include "rbv_stream.cuh"   // warp-autonomous streaming form of the lnprob kernel (big batches)
 #include "rbv_grad.cuh"     // analytic gradient of lnprob / lnlike (forward + adjoint pass)
 #include "rbv_fisher.cuh"   // model Jacobian and Gauss-Newton matrix of lnlike (forward mode per column)
+#include "rbv_lm.cuh"       // survey-mode Levenberg-Marquardt update (one warp per sightline)
 namespace rbv {
 
 // ------------------------------------------------------------------------------------------ small kernels
@@ -1254,6 +1255,12 @@ struct DeviceGuard {
   DeviceGuard _guard((ctx)->device);          \
   RBV_CUDA(_guard.err)
 
+#define RBV_CHECK(expr)                   \
+  do {                                    \
+    const int _rc = (expr);               \
+    if (_rc != RBV_OK) return _rc;        \
+  } while (0)
+
 static int fail(int code, const std::string& msg) {
   g_last_error = msg;
   return code;
@@ -1355,6 +1362,12 @@ struct RbvContext {
   // rbv_slice_run: pinned landing slots + events for the per-iteration read-back of the counters
   SliceCounters* h_poll = nullptr;     // [2], page-locked
   cudaEvent_t poll_ev[2] = {nullptr, nullptr};
+  // survey-mode Fisher: per-instrument order / has_lsf as device tables (host copies to detect a change)
+  std::vector<const int*> sl_order;
+  std::vector<int> sl_has_lsf;
+  const int** d_sl_order = nullptr;
+  int* d_sl_has_lsf = nullptr;
+  int* h_lm_count = nullptr;           // rbv_lm_run_sightlines: page-locked landing slot of the active count
 };
 
 template <typename T>
@@ -1476,6 +1489,9 @@ void rbv_destroy(RbvContext* ctx) {
   cudaFree(ctx->d_unit_taps);
   cudaFree(ctx->d_grid_bar);
   if (ctx->h_poll) cudaFreeHost(ctx->h_poll);
+  if (ctx->h_lm_count) cudaFreeHost(ctx->h_lm_count);
+  cudaFree(ctx->d_sl_order);
+  cudaFree(ctx->d_sl_has_lsf);
   for (int k = 0; k < 2; ++k)
     if (ctx->poll_ev[k]) cudaEventDestroy(ctx->poll_ev[k]);
   delete ctx;
@@ -3106,12 +3122,13 @@ struct GradLayout {
   int n_blk_total, n_tiles_total;
   long long part_stride;
 };
-static GradLayout grad_layout(const RbvContext* ctx, int W, GradInst* gi) {
+// one_inst: the geometry of instrument 0 alone (survey mode, where every sightline shares it)
+static GradLayout grad_layout(const RbvContext* ctx, int W, GradInst* gi, bool one_inst = false) {
   GradLayout L;
   memset(&L, 0, sizeof(L));
   int blk = 0, tiles = 0;
   long long part = 0;
-  for (size_t k = 0; k < ctx->inst.size(); ++k) {
+  for (size_t k = 0; k < (one_inst ? std::min<size_t>(1, ctx->inst.size()) : ctx->inst.size()); ++k) {
     const InstDev& I = ctx->inst[k].dev;
     GradInst g;
     memset(&g, 0, sizeof(g));
@@ -3209,11 +3226,11 @@ int rbv_lnprob_grad_batch(RbvContext* ctx, const double* theta, int W, int apply
   prm.n_blk_total = lay.n_blk_total;
   prm.n_tiles_total = lay.n_tiles_total;
   cudaStream_t st = (cudaStream_t)stream;
-  grad_prep_kernel<<<dim3(W, (ctx->n_lines_total + 127) / 128), 128, 0, st>>>(prm);
+  grad_prep_kernel<false><<<dim3(W, (ctx->n_lines_total + 127) / 128), 128, 0, st>>>(prm, SlRows{});
   RBV_CUDA(cudaGetLastError());
-  grad_flux_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+  grad_flux_kernel<false><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm, SlRows{});
   RBV_CUDA(cudaGetLastError());
-  grad_resid_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+  grad_resid_kernel<false><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm, SlRows{});
   RBV_CUDA(cudaGetLastError());
   grad_adjoint_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
   RBV_CUDA(cudaGetLastError());
@@ -3227,13 +3244,14 @@ int rbv_lnprob_grad_batch(RbvContext* ctx, const double* theta, int W, int apply
 
 // ------------------------------------------------------------------------------------------ Jacobian / Fisher
 // Workspace of rbv_lnlike_fisher_batch and rbv_model_jacobian_batch (byte offsets, 256-byte aligned): the forward
-// buffers of the gradient path plus the columns JF, JM and the Gram partials.
+// buffers of the gradient path plus the columns JF, JM and the Gram partials.  sl: survey mode, every buffer sized for
+// the geometry of one sightline (instrument 0), so the workspace grows as O(W) whatever the number of sightlines.
 struct FisherLayout {
   size_t oob, lc, F, r, pval, JF, JM, pgram, total;
   int n_blk_total, n_tiles_total, ncol, npart;
 };
-static FisherLayout fisher_layout(const RbvContext* ctx, int W, GradInst* gi) {
-  const GradLayout g = grad_layout(ctx, 0, gi);
+static FisherLayout fisher_layout(const RbvContext* ctx, int W, GradInst* gi, bool sl = false) {
+  const GradLayout g = grad_layout(ctx, 0, gi, sl);
   FisherLayout L;
   memset(&L, 0, sizeof(L));
   L.n_blk_total = g.n_blk_total;
@@ -3242,9 +3260,10 @@ static FisherLayout fisher_layout(const RbvContext* ctx, int W, GradInst* gi) {
   L.npart = L.ncol * (L.ncol + 1) / 2 + L.ncol;
   auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
   const size_t Wz = (size_t)std::max(W, 1), px = (size_t)g.n_blk_total * kGradBlock;
+  const size_t n_lines = sl && !ctx->inst.empty() ? (size_t)ctx->inst[0].dev.L : (size_t)ctx->n_lines_total;
   size_t off = 0;
   L.oob = off;   off = al(off + Wz * sizeof(int));
-  L.lc = off;    off = al(off + Wz * ctx->n_lines_total * LC_STRIDE * sizeof(double));
+  L.lc = off;    off = al(off + Wz * n_lines * LC_STRIDE * sizeof(double));
   L.F = off;     off = al(off + Wz * px * sizeof(double));
   L.r = off;     off = al(off + Wz * px * sizeof(double));
   L.pval = off;  off = al(off + Wz * g.n_blk_total * sizeof(double));
@@ -3261,16 +3280,26 @@ int rbv_fisher_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* byt
   return RBV_OK;
 }
 
-// Checks shared by both entry points, the parameter block, and the launches up to JF / JM:
-// prep -> flux [-> resid] -> columns [-> LSF]
-static int fisher_forward(RbvContext* ctx, const char* who, const double* theta, int W, bool with_resid,
-                          void* workspace, size_t workspace_bytes, cudaStream_t st, FisherParams& fp,
-                          FisherLayout& lay) {
+int rbv_fisher_workspace_bytes_sightlines(const RbvContext* ctx, int n_walkers, size_t* bytes) {
+  if (!ctx || !bytes || n_walkers < 0) return fail(RBV_EINVAL, "rbv_fisher_workspace_bytes_sightlines: bad argument");
+  *bytes = fisher_layout(ctx, n_walkers, nullptr, true).total;
+  return RBV_OK;
+}
+
+static bool has_lsf(const HostInst& hi) { return !(hi.taps.size() == 1 && hi.taps[0] == 1.0); }
+
+// Checks shared by every entry point and the parameter block of the launches.  sl: survey mode (any number of
+// instruments, identical geometry, one instrument's geometry in fp.gp).
+static int fisher_setup(RbvContext* ctx, const char* who, const double* theta, int W, bool with_resid, bool sl,
+                        void* workspace, size_t workspace_bytes, FisherParams& fp, FisherLayout& lay, bool& any_lsf) {
   if (ctx->inst.empty()) return fail(RBV_ESTATE, std::string(who) + ": no instrument added");
   if (ctx->ndim == 0) return fail(RBV_ESTATE, std::string(who) + ": bounds not set (rbv_set_bounds)");
-  if (ctx->inst.size() > (size_t)kMaxInst)
+  if (!sl && ctx->inst.size() > (size_t)kMaxInst)
     return fail(RBV_EINVAL, std::string(who) + ": at most 16 instruments in a joint fit");
+  const InstDev& A = ctx->inst[0].dev;
   for (auto& hi : ctx->inst) {
+    if (sl && (hi.dev.P != A.P || hi.dev.K != A.K || hi.dev.L != A.L || hi.dev.C != A.C))
+      return fail(RBV_EINVAL, std::string(who) + ": sightlines must share n_pixels, n_taps, n_lines, n_components");
     if (3 * hi.dev.C > ctx->ndim) return fail(RBV_EINVAL, std::string(who) + ": ndim smaller than 3 * n_components");
     if (hi.dev.method != RBV_VOIGT_WOFZ)
       return fail(RBV_EINVAL, std::string(who) + ": no Jacobian for voigt_method='fast' (Tepper-Garcia)");
@@ -3279,19 +3308,18 @@ static int fisher_forward(RbvContext* ctx, const char* who, const double* theta,
   }
   memset(&fp, 0, sizeof(fp));
   GradParams& prm = fp.gp;
-  lay = fisher_layout(ctx, W, prm.gi);
+  lay = fisher_layout(ctx, W, prm.gi, sl);
   if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, std::string(who) + ": workspace too small");
   const size_t smem = (size_t)(lay.ncol + 2) * kFisherChunk * sizeof(double);
   if (smem > (size_t)ctx->max_dyn_smem) return fail(RBV_EINVAL, std::string(who) + ": too many components");
-  RBV_ON_DEVICE(ctx);
-  if (smem > 48 * 1024)
-    RBV_CUDA(cudaFuncSetAttribute(fisher_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  bool any_lsf = false;
+  any_lsf = false;
   for (size_t k = 0; k < ctx->inst.size(); ++k) {
     const HostInst& hi = ctx->inst[k];
-    fp.order[k] = hi.d_fisher_order;
-    fp.has_lsf[k] = !(hi.taps.size() == 1 && hi.taps[0] == 1.0);
-    any_lsf = any_lsf || fp.has_lsf[k];
+    if (!sl) {
+      fp.order[k] = hi.d_fisher_order;
+      fp.has_lsf[k] = has_lsf(hi);
+    }
+    any_lsf = any_lsf || has_lsf(hi);
   }
   char* ws = (char*)workspace;
   prm.inst = ctx->d_inst;
@@ -3304,8 +3332,8 @@ static int fisher_forward(RbvContext* ctx, const char* who, const double* theta,
   prm.pval = (double*)(ws + lay.pval);
   prm.W = W;
   prm.ndim = ctx->ndim;
-  prm.n_inst = (int)ctx->inst.size();
-  prm.n_lines_total = ctx->n_lines_total;
+  prm.n_inst = sl ? 1 : (int)ctx->inst.size();
+  prm.n_lines_total = sl ? A.L : ctx->n_lines_total;
   prm.n_blk_total = lay.n_blk_total;
   prm.n_tiles_total = lay.n_tiles_total;
   fp.ncol = lay.ncol;
@@ -3314,24 +3342,68 @@ static int fisher_forward(RbvContext* ctx, const char* who, const double* theta,
   fp.JF = (double*)(ws + lay.JF);
   fp.JM = (double*)(ws + lay.JM);
   fp.pgram = (double*)(ws + lay.pgram);
-  grad_prep_kernel<<<dim3(W, (ctx->n_lines_total + 127) / 128), 128, 0, st>>>(prm);
+  return RBV_OK;
+}
+
+// prep -> flux [-> resid] -> columns [-> LSF] [-> Gram -> finalize]
+extern "C++" {
+template <bool SL>
+static int fisher_launch(RbvContext* ctx, const FisherParams& fp, const FisherLayout& lay, bool with_resid,
+                         bool any_lsf, bool gram, const SlRows& sl, cudaStream_t st) {
+  const GradParams& prm = fp.gp;
+  const int W = prm.W;
+  grad_prep_kernel<SL><<<dim3(W, (prm.n_lines_total + 127) / 128), 128, 0, st>>>(prm, sl);
   RBV_CUDA(cudaGetLastError());
-  grad_flux_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+  grad_flux_kernel<SL><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm, sl);
   RBV_CUDA(cudaGetLastError());
   ctx->launches += 2;
   if (with_resid) {
-    grad_resid_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
+    grad_resid_kernel<SL><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm, sl);
     RBV_CUDA(cudaGetLastError());
     ctx->launches++;
   }
-  fisher_col_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(fp);
+  fisher_col_kernel<SL><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(fp, sl);
   RBV_CUDA(cudaGetLastError());
   ctx->launches++;
   if (any_lsf) {
-    fisher_lsf_kernel<<<dim3(lay.n_blk_total, lay.ncol, W), kGradBlock, 0, st>>>(fp);
+    fisher_lsf_kernel<SL><<<dim3(lay.n_blk_total, lay.ncol, W), kGradBlock, 0, st>>>(fp, sl);
     RBV_CUDA(cudaGetLastError());
     ctx->launches++;
   }
+  if (!gram) return RBV_OK;
+  const size_t smem = (size_t)(lay.ncol + 2) * kFisherChunk * sizeof(double);
+  if (smem > 48 * 1024)
+    RBV_CUDA(cudaFuncSetAttribute(fisher_gram_kernel<SL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  fisher_gram_kernel<SL><<<dim3(lay.n_tiles_total, W), kGradBlock, smem, st>>>(fp, sl);
+  RBV_CUDA(cudaGetLastError());
+  fisher_finalize_kernel<SL><<<(W + 3) / 4, 128, 0, st>>>(fp, sl);
+  RBV_CUDA(cudaGetLastError());
+  ctx->launches += 2;
+  return RBV_OK;
+}
+}  // extern "C++"
+
+// survey mode: order / has_lsf of every instrument as device tables; uploaded again only when they changed
+static int sightline_tables(RbvContext* ctx, SlRows& sl) {
+  std::vector<const int*> order;
+  std::vector<int> lsf;
+  for (auto& hi : ctx->inst) {
+    order.push_back(hi.d_fisher_order);
+    lsf.push_back(has_lsf(hi) ? 1 : 0);
+  }
+  if (order != ctx->sl_order || lsf != ctx->sl_has_lsf || !ctx->d_sl_order) {
+    cudaFree(ctx->d_sl_order);
+    cudaFree(ctx->d_sl_has_lsf);
+    ctx->d_sl_order = nullptr;
+    ctx->d_sl_has_lsf = nullptr;
+    ctx->sl_order.clear();
+    RBV_CUDA(upload(&ctx->d_sl_order, order.data(), order.size()));
+    RBV_CUDA(upload(&ctx->d_sl_has_lsf, lsf.data(), lsf.size()));
+    ctx->sl_order = order;
+    ctx->sl_has_lsf = lsf;
+  }
+  sl.order = ctx->d_sl_order;
+  sl.has_lsf = ctx->d_sl_has_lsf;
   return RBV_OK;
 }
 
@@ -3341,21 +3413,42 @@ int rbv_lnlike_fisher_batch(RbvContext* ctx, const double* theta, int W, double*
   if (!ctx || !theta || !value || !grad || !fisher) return fail(RBV_EINVAL, std::string(who) + ": null argument");
   if (W < 0) return fail(RBV_EINVAL, std::string(who) + ": negative n_walkers");
   if (W == 0) return RBV_OK;
-  cudaStream_t st = (cudaStream_t)stream;
   FisherParams fp;
   FisherLayout lay;
-  const int rc = fisher_forward(ctx, who, theta, W, true, workspace, workspace_bytes, st, fp, lay);
+  bool any_lsf;
+  const int rc = fisher_setup(ctx, who, theta, W, true, false, workspace, workspace_bytes, fp, lay, any_lsf);
   if (rc != RBV_OK) return rc;
+  RBV_ON_DEVICE(ctx);
   fp.gp.value = value;
   fp.gp.grad = grad;
   fp.fisher = fisher;
-  fisher_gram_kernel<<<dim3(lay.n_tiles_total, W), kGradBlock, (lay.ncol + 2) * kFisherChunk * sizeof(double), st>>>(
-      fp);
-  RBV_CUDA(cudaGetLastError());
-  fisher_finalize_kernel<<<(W + 3) / 4, 128, 0, st>>>(fp);
-  RBV_CUDA(cudaGetLastError());
-  ctx->launches += 2;
-  return RBV_OK;
+  return fisher_launch<false>(ctx, fp, lay, true, any_lsf, true, SlRows{}, (cudaStream_t)stream);
+}
+
+int rbv_lnlike_fisher_batch_sightlines(RbvContext* ctx, const double* theta, int W, int walkers_per_sightline,
+                                       double* value, double* grad, double* fisher, void* workspace,
+                                       size_t workspace_bytes, void* stream) {
+  const char* who = "rbv_lnlike_fisher_batch_sightlines";
+  if (!ctx || !theta || !value || !grad || !fisher) return fail(RBV_EINVAL, std::string(who) + ": null argument");
+  if (W < 0 || walkers_per_sightline <= 0)
+    return fail(RBV_EINVAL, std::string(who) + ": negative n_walkers or walkers_per_sightline <= 0");
+  if ((long long)walkers_per_sightline * (long long)ctx->inst.size() != (long long)W)
+    return fail(RBV_EINVAL, std::string(who) + ": n_walkers must equal n_sightlines * walkers_per_sightline");
+  if (W == 0) return RBV_OK;
+  FisherParams fp;
+  FisherLayout lay;
+  bool any_lsf;
+  const int rc = fisher_setup(ctx, who, theta, W, true, true, workspace, workspace_bytes, fp, lay, any_lsf);
+  if (rc != RBV_OK) return rc;
+  RBV_ON_DEVICE(ctx);
+  SlRows sl;
+  memset(&sl, 0, sizeof(sl));
+  RBV_CHECK(sightline_tables(ctx, sl));
+  sl.wps = walkers_per_sightline;
+  fp.gp.value = value;
+  fp.gp.grad = grad;
+  fp.fisher = fisher;
+  return fisher_launch<true>(ctx, fp, lay, true, any_lsf, true, sl, (cudaStream_t)stream);
 }
 
 int rbv_model_jacobian_batch(RbvContext* ctx, int inst, const double* theta, int W, double* out_jac, void* workspace,
@@ -3368,8 +3461,11 @@ int rbv_model_jacobian_batch(RbvContext* ctx, int inst, const double* theta, int
   cudaStream_t st = (cudaStream_t)stream;
   FisherParams fp;
   FisherLayout lay;
-  const int rc = fisher_forward(ctx, who, theta, W, false, workspace, workspace_bytes, st, fp, lay);
+  bool any_lsf;
+  const int rc = fisher_setup(ctx, who, theta, W, false, false, workspace, workspace_bytes, fp, lay, any_lsf);
   if (rc != RBV_OK) return rc;
+  RBV_ON_DEVICE(ctx);
+  RBV_CHECK(fisher_launch<false>(ctx, fp, lay, false, any_lsf, false, SlRows{}, st));
   fp.jac = out_jac;
   fp.jac_inst = inst;
   const int P = ctx->inst[inst].dev.P;
@@ -3377,6 +3473,125 @@ int rbv_model_jacobian_batch(RbvContext* ctx, int inst, const double* theta, int
   RBV_CUDA(cudaGetLastError());
   ctx->launches++;
   return RBV_OK;
+}
+
+// ------------------------------------------------------------------------------------------ survey-mode LM
+// Workspace of rbv_lm_run_sightlines: the survey-mode Fisher workspace of n rows, then the per-sightline state of
+// LMParams (rbv_lm.cuh).
+struct LMLayout {
+  FisherLayout fl;
+  size_t g, F, xc, vc, gc, Fc, L, Li, y, idx, lam, nu, started, active, count, total;
+};
+static LMLayout lm_layout(const RbvContext* ctx, int n) {
+  LMLayout L;
+  memset(&L, 0, sizeof(L));
+  L.fl = fisher_layout(ctx, n, nullptr, true);
+  auto al = [](size_t v) { return (v + 255) & ~(size_t)255; };
+  const size_t nz = (size_t)std::max(n, 1), d = (size_t)ctx->ndim, dd = d * d * sizeof(double);
+  size_t off = L.fl.total;
+  L.g = off;       off = al(off + nz * d * sizeof(double));
+  L.F = off;       off = al(off + nz * dd);
+  L.xc = off;      off = al(off + nz * d * sizeof(double));
+  L.vc = off;      off = al(off + nz * sizeof(double));
+  L.gc = off;      off = al(off + nz * d * sizeof(double));
+  L.Fc = off;      off = al(off + nz * dd);
+  L.L = off;       off = al(off + nz * dd);
+  L.Li = off;      off = al(off + nz * dd);
+  L.y = off;       off = al(off + nz * d * sizeof(double));
+  L.idx = off;     off = al(off + nz * d * sizeof(int));
+  L.lam = off;     off = al(off + nz * sizeof(double));
+  L.nu = off;      off = al(off + nz * sizeof(double));
+  L.started = off; off = al(off + nz * sizeof(int));
+  L.active = off;  off = al(off + nz * sizeof(int));
+  L.count = off;   off = al(off + sizeof(int));
+  L.total = off;
+  return L;
+}
+
+int rbv_lm_workspace_bytes_sightlines(const RbvContext* ctx, int n_sightlines, size_t* bytes) {
+  if (!ctx || !bytes || n_sightlines < 0) return fail(RBV_EINVAL, "rbv_lm_workspace_bytes_sightlines: bad argument");
+  *bytes = lm_layout(ctx, n_sightlines).total;
+  return RBV_OK;
+}
+
+int rbv_lm_run_sightlines(RbvContext* ctx, int first, int n, double* theta, const RbvLMControl* ctl, double* chi2,
+                          double* cov, int* n_evals, int* status, int* flags, void* workspace, size_t workspace_bytes,
+                          void* stream) {
+  const char* who = "rbv_lm_run_sightlines";
+  if (!ctx || !theta || !ctl || !chi2 || !cov || !n_evals || !status || !flags)
+    return fail(RBV_EINVAL, std::string(who) + ": null argument");
+  if (first < 0 || n < 0 || (long long)first + n > (long long)ctx->inst.size())
+    return fail(RBV_EINVAL, std::string(who) + ": [first, first + n) is not a range of the context's sightlines");
+  if (ctl->max_evals < 1 || !(ctl->ftol >= 0.0) || !(ctl->xtol >= 0.0))
+    return fail(RBV_EINVAL, std::string(who) + ": max_evals < 1 or a negative tolerance");
+  if (n == 0) return RBV_OK;
+  const LMLayout L = lm_layout(ctx, n);
+  FisherParams fp;
+  FisherLayout lay;
+  bool any_lsf;
+  char* ws = (char*)workspace;
+  double* xc = (double*)(ws + L.xc);
+  int rc = fisher_setup(ctx, who, xc, n, true, true, workspace, workspace_bytes, fp, lay, any_lsf);
+  if (rc != RBV_OK) return rc;
+  if (workspace_bytes < L.total) return fail(RBV_ENOMEM, std::string(who) + ": workspace too small");
+  RBV_ON_DEVICE(ctx);
+  if (!ctx->h_lm_count) RBV_CUDA(cudaMallocHost((void**)&ctx->h_lm_count, sizeof(int)));
+  SlRows sl;
+  memset(&sl, 0, sizeof(sl));
+  RBV_CHECK(sightline_tables(ctx, sl));
+  sl.wps = 1;
+  sl.inst0 = first;
+  sl.active = (const int*)(ws + L.active);
+  fp.gp.value = (double*)(ws + L.vc);
+  fp.gp.grad = (double*)(ws + L.gc);
+  fp.fisher = (double*)(ws + L.Fc);
+  LMParams p;
+  memset(&p, 0, sizeof(p));
+  p.n = n;
+  p.ndim = ctx->ndim;
+  p.max_evals = ctl->max_evals;
+  p.ftol = ctl->ftol;
+  p.xtol = ctl->xtol;
+  p.lb = ctx->d_lb;
+  p.ub = ctx->d_ub;
+  p.x = theta;
+  p.g = (double*)(ws + L.g);
+  p.F = (double*)(ws + L.F);
+  p.xc = xc;
+  p.vc = (const double*)(ws + L.vc);
+  p.gc = (const double*)(ws + L.gc);
+  p.Fc = (const double*)(ws + L.Fc);
+  p.L = (double*)(ws + L.L);
+  p.Li = (double*)(ws + L.Li);
+  p.y = (double*)(ws + L.y);
+  p.idx = (int*)(ws + L.idx);
+  p.lam = (double*)(ws + L.lam);
+  p.nu = (double*)(ws + L.nu);
+  p.started = (int*)(ws + L.started);
+  p.active = (int*)(ws + L.active);
+  p.count = (int*)(ws + L.count);
+  p.chi2 = chi2;
+  p.cov = cov;
+  p.n_evals = n_evals;
+  p.status = status;
+  p.flags = flags;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int blocks = (n + kLMWarps - 1) / kLMWarps;
+  lm_init_kernel<<<blocks, 32 * kLMWarps, 0, st>>>(p);
+  RBV_CUDA(cudaGetLastError());
+  ctx->launches++;
+  // every iteration evaluates one row per active sightline and n_evals never exceeds max_evals
+  for (int it = 0; it < ctl->max_evals; ++it) {
+    RBV_CHECK(fisher_launch<true>(ctx, fp, lay, true, any_lsf, true, sl, st));
+    RBV_CUDA(cudaMemsetAsync(p.count, 0, sizeof(int), st));
+    lm_update_kernel<<<blocks, 32 * kLMWarps, 0, st>>>(p);
+    RBV_CUDA(cudaGetLastError());
+    ctx->launches++;
+    RBV_CUDA(cudaMemcpyAsync(ctx->h_lm_count, p.count, sizeof(int), cudaMemcpyDeviceToHost, st));
+    RBV_CUDA(cudaStreamSynchronize(st));
+    if (*ctx->h_lm_count == 0) return RBV_OK;
+  }
+  return fail(RBV_ESTATE, std::string(who) + ": sightlines still active after max_evals iterations");
 }
 
 int rbv_measure_fp64_peak(RbvContext* ctx, double millis, double* tflops) {

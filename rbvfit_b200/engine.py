@@ -315,6 +315,93 @@ class Engine:
             out[i:i + step] = jac.cpu().numpy()
         return out
 
+    def _sl_bytes(self, fn, n: int, what: str) -> int:
+        nbytes = C.c_size_t(0)
+        check(fn(self._h, max(int(n), 1), C.byref(nbytes)), what)
+        return int(nbytes.value)
+
+    def _sl_ws(self, nbytes: int):
+        torch = _torch()
+        if getattr(self, "_sl_ws_t", None) is None or self._sl_ws_t.numel() < nbytes:
+            self._sl_ws_t = None
+            self._sl_ws_t = torch.empty(max(nbytes, 8), dtype=torch.uint8, device=self.tdev)
+        return self._sl_ws_t
+
+    def lnlike_fisher_sightlines_device(self, theta_t, wps: int):
+        """Survey mode (``rbv_lnlike_fisher_batch_sightlines``): DEVICE theta [S * wps, ndim], ``wps`` consecutive rows
+        per sightline -> DEVICE (lnlike [S * wps], gradient [S * wps, ndim], Gauss-Newton matrix [S * wps, ndim,
+        ndim]); each row bit for bit what a one-sightline context gives.  Asynchronous."""
+        torch = _torch()
+        self._dev_tensor(theta_t, torch.float64, "theta")
+        if theta_t.dim() != 2 or theta_t.shape[1] != self.ndim:
+            raise ValueError(f"theta must be [W, {self.ndim}]")
+        W, n = int(theta_t.shape[0]), self.ndim
+        value_t = torch.empty(W, dtype=torch.float64, device=self.tdev)
+        grad_t = torch.empty((W, n), dtype=torch.float64, device=self.tdev)
+        fisher_t = torch.empty((W, n, n), dtype=torch.float64, device=self.tdev)
+        ws = self._sl_ws(self._sl_bytes(self.lib.rbv_fisher_workspace_bytes_sightlines, W,
+                                        "rbv_fisher_workspace_bytes_sightlines"))
+        check(self.lib.rbv_lnlike_fisher_batch_sightlines(self._h, theta_t.data_ptr(), W, int(wps), value_t.data_ptr(),
+                                                          grad_t.data_ptr(), fisher_t.data_ptr(), ws.data_ptr(),
+                                                          ws.numel(), self._stream()),
+              "rbv_lnlike_fisher_batch_sightlines")
+        return value_t, grad_t, fisher_t
+
+    def lnlike_fisher_sightlines_host(self, theta: np.ndarray, wps: int):
+        """HOST theta [S * wps, ndim] (``wps`` consecutive rows per sightline) -> HOST (lnlike, gradient, Gauss-Newton
+        matrix).  The launch always covers every sightline, so a batch whose workspace would pass
+        ``fisher_chunk_bytes`` is split into blocks of walkers of every sightline (down to one row per sightline);
+        each row's results do not depend on the batch."""
+        torch = _torch()
+        theta = np.ascontiguousarray(theta, dtype=np.float64)
+        S, wps = len(self.pixels), int(wps)
+        if theta.ndim != 2 or theta.shape != (S * wps, self.ndim) or wps <= 0:
+            raise ValueError(f"theta must be [{S} * walkers_per_sightline, {self.ndim}]")
+        n = self.ndim
+        one = self._sl_bytes(self.lib.rbv_fisher_workspace_bytes_sightlines, S, "rbv_fisher_workspace_bytes_sightlines")
+        step = max(1, int(self.fisher_chunk_bytes // max(one, 1)))
+        th3 = theta.reshape(S, wps, n)
+        value, grad, fisher = np.empty((S, wps)), np.empty((S, wps, n)), np.empty((S, wps, n, n))
+        for j in range(0, wps, step):
+            c = min(step, wps - j)
+            th = torch.as_tensor(np.ascontiguousarray(th3[:, j:j + c]).reshape(S * c, n), device=self.tdev)
+            v, g, f = self.lnlike_fisher_sightlines_device(th, c)
+            value[:, j:j + c] = v.cpu().numpy().reshape(S, c)
+            grad[:, j:j + c] = g.cpu().numpy().reshape(S, c, n)
+            fisher[:, j:j + c] = f.cpu().numpy().reshape(S, c, n, n)
+        return value.reshape(S * wps), grad.reshape(S * wps, n), fisher.reshape(S * wps, n, n)
+
+    def lm_sightlines(self, theta0: np.ndarray, first: int, n: int, max_evals: int = 200, ftol: float = 1e-10,
+                      xtol: float = 1e-10):
+        """Levenberg-Marquardt fits of sightlines [first, first + n) on the device (``rbv_lm_run_sightlines``):
+        HOST theta0 [n, ndim] -> HOST (x [n, ndim], chi2 [n], cov [n, ndim, ndim], n_evals [n], status [n],
+        flags [n]).  Runs in blocks of whole sightlines whose workspace stays below ``fisher_chunk_bytes``: the
+        sightlines are independent, so the blocks do not change any result."""
+        torch = _torch()
+        theta0 = np.ascontiguousarray(theta0, dtype=np.float64)
+        nd, first, n = self.ndim, int(first), int(n)
+        if theta0.shape != (n, nd):
+            raise ValueError(f"theta0 must be [{n}, {nd}]")
+        ctl = _lib.RbvLMControl(int(max_evals), float(ftol), float(xtol))
+        one = self._sl_bytes(self.lib.rbv_lm_workspace_bytes_sightlines, 1, "rbv_lm_workspace_bytes_sightlines")
+        step = max(1, int(self.fisher_chunk_bytes // max(one, 1)))
+        x, chi2, cov = theta0.copy(), np.empty(n), np.empty((n, nd, nd))
+        n_evals, status, flags = (np.empty(n, dtype=np.int32) for _ in range(3))
+        for b in range(0, n, step):
+            c = min(step, n - b)
+            th = torch.as_tensor(theta0[b:b + c], device=self.tdev)
+            ch = torch.empty(c, dtype=torch.float64, device=self.tdev)
+            cv = torch.empty((c, nd, nd), dtype=torch.float64, device=self.tdev)
+            ne, st, fl = (torch.empty(c, dtype=torch.int32, device=self.tdev) for _ in range(3))
+            ws = self._sl_ws(self._sl_bytes(self.lib.rbv_lm_workspace_bytes_sightlines, c,
+                                            "rbv_lm_workspace_bytes_sightlines"))
+            check(self.lib.rbv_lm_run_sightlines(self._h, first + b, c, th.data_ptr(), C.byref(ctl), ch.data_ptr(),
+                                                 cv.data_ptr(), ne.data_ptr(), st.data_ptr(), fl.data_ptr(),
+                                                 ws.data_ptr(), ws.numel(), self._stream()), "rbv_lm_run_sightlines")
+            x[b:b + c], chi2[b:b + c], cov[b:b + c] = th.cpu().numpy(), ch.cpu().numpy(), cv.cpu().numpy()
+            n_evals[b:b + c], status[b:b + c], flags[b:b + c] = ne.cpu().numpy(), st.cpu().numpy(), fl.cpu().numpy()
+        return x, chi2, cov, n_evals, status, flags
+
     def voigt_h_grad(self, x: np.ndarray, a: np.ndarray):
         """H, dH/dx, dH/da on a lattice (``rbv_voigt_h_grad``, test hook)."""
         torch = _torch()

@@ -7,7 +7,8 @@ called by an optimiser exactly like the reference's bound method.
 """
 from __future__ import annotations
 
-from typing import Dict, Optional
+import warnings
+from typing import Dict, NamedTuple, Optional
 
 import numpy as np
 
@@ -244,6 +245,16 @@ class GpuLikelihood:
         self.engine.close()
 
 
+class SightlineFit(NamedTuple):
+    """Per-sightline results of ``SightlineBatch.fit_quick``, each field with the meaning of ``lm.LMResult``."""
+    x: np.ndarray          # [S, ndim] best points
+    chi2: np.ndarray       # [S] -2 lnlike at x
+    cov: np.ndarray        # [S, ndim, ndim] inv(F_ff) over the free set; NaN rows / columns elsewhere
+    n_evals: np.ndarray    # [S] Fisher evaluations
+    status: np.ndarray     # [S] lm.STATUS_*: > 0 converged
+    errors: np.ndarray     # [S, ndim] sqrt(diag(cov))
+
+
 class SightlineBatch:
     """Survey mode (BASELINE.json config 5, "1024 independent sightlines batched"): S independent fits that share
     the model *structure* (same number of lines / components / pixels / LSF taps) but have their own redshift,
@@ -297,6 +308,41 @@ class SightlineBatch:
 
     def lnprob_device(self, theta_t, wps: int, out_t=None):
         return self.engine.lnprob_sightlines_device(theta_t, wps, out_t)
+
+    def lnlike_and_fisher(self, theta):
+        """theta [S, Ws, ndim] -> (lnlike [S, Ws], gradient [S, Ws, ndim], Gauss-Newton matrix [S, Ws, ndim, ndim]),
+        every row against its own sightline (``GpuLikelihood.lnlike_and_fisher`` of that sightline, bit for bit)."""
+        theta = np.asarray(theta, dtype=np.float64)
+        if theta.ndim != 3 or theta.shape[0] != self.n_sightlines or theta.shape[2] != self.ndim:
+            raise ValueError(f"theta must be [{self.n_sightlines}, walkers_per_sightline, {self.ndim}]")
+        S, Ws, nd = theta.shape
+        v, g, f = self.engine.lnlike_fisher_sightlines_host(theta.reshape(S * Ws, nd), Ws)
+        return v.reshape(S, Ws), g.reshape(S, Ws, nd), f.reshape(S, Ws, nd, nd)
+
+    def fit_quick(self, theta0, max_evals: int = 200, ftol: float = 1e-10, xtol: float = 1e-10) -> SightlineFit:
+        """Bounded Levenberg-Marquardt fit of every sightline (the rules of ``lm.levenberg_marquardt``) in one device
+        loop: each iteration is one Fisher evaluation of the sightlines still iterating and one update kernel
+        (DESIGN.md section 16).  ``theta0``: [S, ndim] starts, or one [ndim] start for every sightline.  Sightlines
+        whose F_ff is not positive definite at the end get ``lm.covariance``'s pinv (with its warning)."""
+        from . import lm
+        S, nd = self.n_sightlines, self.ndim
+        theta0 = np.asarray(theta0, dtype=np.float64)
+        if theta0.shape == (nd,):
+            theta0 = np.broadcast_to(theta0, (S, nd))
+        if theta0.shape != (S, nd):
+            raise ValueError(f"theta0 must be [{S}, {nd}] or [{nd}]")
+        x, chi2, cov, n_evals, status, flags = self.engine.lm_sightlines(theta0, 0, S, max_evals, ftol, xtol)
+        bad = np.flatnonzero(flags & 1)
+        if bad.size:
+            _v, g, F = self.engine.lnlike_fisher_sightlines_host(x, 1)
+            for s in bad:
+                cov[s] = lm.covariance(F[s], lm.free_set(x[s], g[s], F[s], self.lb, self.ub))
+        n_bad = int(np.count_nonzero(status <= 0))
+        if n_bad:
+            warnings.warn(f"Optimization may not have converged on {n_bad} of {S} sightlines (status <= 0)")
+        with np.errstate(invalid="ignore"):
+            errors = np.sqrt(np.diagonal(cov, axis1=1, axis2=2))
+        return SightlineFit(x, chi2, cov, n_evals, status, errors)
 
     def close(self):
         self.engine.close()
