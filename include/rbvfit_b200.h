@@ -310,6 +310,33 @@ int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers
                   double* mu_history, int* flag, void* workspace, size_t workspace_bytes, int use_graph,
                   void* stream);
 
+/* Survey mode of the slice sampler: the context holds S sightlines (see rbv_lnprob_batch_sightlines) and every
+ * sightline has its OWN ensemble of walkers_per_sightline walkers -- what the reference does as S separate
+ * vfit(..., sampler='zeus') runs.  The S ensembles advance in lockstep: an iteration is ONE sightline-mode lnprob
+ * launch over the candidate rows of every ensemble (masked rows skipped), and a half-step iterates until no walker of
+ * any sightline is unfinished; a sightline whose walkers have finished masks its rows, so its chain does not depend
+ * on the others.  Ensembles never mix.  Random streams: those of rbv_slice_run with the walker counter offset by
+ * sightline * walkers_per_sightline (the step's split is shared), so sightline 0 of a survey run reproduces the
+ * single-ensemble run with the same seed.  Loop drivers (use_graph) and depth as in rbv_slice_run; chains, mu and
+ * the counters do not depend on either.  Rows are never split across ranks: an attached communicator is not used.
+ *   coords, lnprob   DEVICE [S, walkers_per_sightline, ndim] / [S, walkers_per_sightline], in place (wps >= 4)
+ *   tuning           HOST: tolerance, patience, maxsteps, maxiter and depth, shared by every sightline; n_batches
+ *                    (lnprob launches of this run) is written; mu, tune, good and the other n_* fields are not used
+ *   mu               DEVICE double[S], in/out: each sightline's scale, adapted after every step (must be > 0)
+ *   tune_good        DEVICE int[S, 2], in/out: each sightline's tune flag and count of good steps
+ *   totals           DEVICE uint64[S, 3], accumulated: expansions, contractions, likelihood rows of each sightline
+ *   chain            DEVICE [n_steps, S, wps, ndim] or NULL; lnprob_chain DEVICE [n_steps, S, wps] or NULL
+ *   mu_history       DEVICE [n_steps, S] or NULL: every sightline's mu after each step
+ *   flag             DEVICE int, bit 0 set if a candidate's lnprob was NaN
+ *   workspace        DEVICE, rbv_slice_workspace_bytes_sightlines().  Returns RBV_ESTATE when a half-step of any
+ *                    sightline needed more than maxiter iterations.  The call returns after the run has finished. */
+int rbv_slice_workspace_bytes_sightlines(const RbvContext* ctx, int walkers_per_sightline, size_t* bytes);
+int rbv_slice_run_sightlines(RbvContext* ctx, double* coords, double* lnprob, int walkers_per_sightline, int n_steps,
+                             RbvSliceTuning* tuning, double* mu, int* tune_good, unsigned long long* totals,
+                             unsigned long long seed, unsigned long long first_step, double* chain,
+                             double* lnprob_chain, double* mu_history, int* flag, void* workspace,
+                             size_t workspace_bytes, int use_graph, void* stream);
+
 /* Model flux for a batch of walkers on instrument `inst`; CompiledVoigtModel.model_flux,
  * voigt_model.py:295-311 (convolve != 0: the instrument's LSF is applied, :221-230) or
  * VoigtModel.evaluate(return_unconvolved=True), :509-558 (convolve == 0: exp(-tau) as it is, :217).

@@ -93,6 +93,11 @@ EXPORTS = {
     "rbv_slice_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(RbvSliceTuning),
                                 C.c_ulonglong, C.c_ulonglong, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
+    "rbv_slice_workspace_bytes_sightlines": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_size_t)]),
+    "rbv_slice_run_sightlines": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                           C.POINTER(RbvSliceTuning), C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_ulonglong, C.c_ulonglong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "rbv_flux_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
     "rbv_model_flux_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p,
                                        C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -1360,7 +1360,7 @@ struct RbvContext {
   unsigned int* d_grid_bar = nullptr;   // grid-barrier counter of voigt_mcmc_kernel
   size_t max_smem_lnprob[2] = {0, 0};  // per LOGR in {2,3}
   // rbv_slice_run: pinned landing slots + events for the per-iteration read-back of the counters
-  SliceCounters* h_poll = nullptr;     // [2], page-locked
+  SliceState* h_poll = nullptr;        // [2], page-locked
   cudaEvent_t poll_ev[2] = {nullptr, nullptr};
   // survey-mode Fisher: per-instrument order / has_lsf as device tables (host copies to detect a change)
   std::vector<const int*> sl_order;
@@ -1458,7 +1458,7 @@ int rbv_create(int device, RbvContext** out) {
   RBV_CUDA(cudaFuncSetAttribute(voigt_mcmc_kernel<3, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_dyn));
   RBV_CUDA(cudaFuncSetAttribute(voigt_mcmc_kernel<3, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_dyn));
   RBV_CUDA(cudaMalloc((void**)&ctx->d_grid_bar, 256));
-  RBV_CUDA(cudaMallocHost((void**)&ctx->h_poll, 2 * sizeof(SliceCounters)));
+  RBV_CUDA(cudaMallocHost((void**)&ctx->h_poll, 2 * sizeof(SliceState)));
   for (int k = 0; k < 2; ++k) RBV_CUDA(cudaEventCreateWithFlags(&ctx->poll_ev[k], cudaEventDisableTiming));
   guard.c = nullptr;
   *out = ctx;
@@ -2770,11 +2770,15 @@ int rbv_stretch_run_sightlines(RbvContext* ctx, double* coords, double* lnprob, 
 
 // ---- device-resident ensemble slice sampler (zeus's differential move), rbv_slice.cuh ------------------------
 struct SliceLayout {
-  size_t cand, lnp_cand, dir, z0, lo, hi, tcur, jbudget, kbudget, phase, lit, skip, walker_of, ctr, lnprob_ws, total;
+  size_t cand, lnp_cand, dir, z0, lo, hi, tcur, jbudget, kbudget, phase, lit, skip, walker_of, ctr, nstep, lnprob_ws,
+      total;
 };
-static SliceLayout slice_layout(const RbvContext* ctx, int W) {
+// sl = false: rbv_slice_run (one ensemble, joint-fit lnprob workspace, its SliceEnsemble inside the SliceState
+// block); sl = true: survey mode, one ensemble per sightline of the context
+static SliceLayout slice_layout(const RbvContext* ctx, int W, bool sl) {
   auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-  const size_t h = (size_t)(W + 1) / 2, row = h * std::max(ctx->ndim, 1) * sizeof(double);
+  const size_t S = sl ? std::max<size_t>(ctx->inst.size(), 1) : 1;
+  const size_t h = (size_t)(W + 1) / 2 * S, row = h * std::max(ctx->ndim, 1) * sizeof(double);   // h: all ensembles
   SliceLayout lay;
   size_t o = 0;
   auto take = [&](size_t bytes) { size_t at = o; o += up(bytes); return at; };
@@ -2791,34 +2795,32 @@ static SliceLayout slice_layout(const RbvContext* ctx, int W) {
   lay.lit = take(h * sizeof(int));
   lay.skip = take(4 * h * sizeof(int));
   lay.walker_of = take(h * sizeof(int));
-  lay.ctr = take(sizeof(SliceCounters));
+  lay.ctr = take(sizeof(SliceState));
+  lay.nstep = sl ? take(2 * S * sizeof(unsigned int)) : lay.ctr + offsetof(SliceState, solo.nstep);
   lay.lnprob_ws = o;
-  lay.total = o + workspace_layout(ctx, (int)(4 * h), false).total;
+  lay.total = o + workspace_layout(ctx, (int)(4 * h), sl).total;
   return lay;
 }
 
 int rbv_slice_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* bytes) {
   if (!ctx || !bytes || n_walkers < 4) return fail(RBV_EINVAL, "rbv_slice_workspace_bytes: bad argument");
-  *bytes = slice_layout(ctx, n_walkers).total;
+  *bytes = slice_layout(ctx, n_walkers, false).total;
   return RBV_OK;
 }
 
-int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers, int n_steps, RbvSliceTuning* tuning,
-                  unsigned long long seed, unsigned long long first_step, double* chain, double* lnprob_chain,
-                  double* mu_history, int* flag, void* workspace, size_t workspace_bytes, int use_graph,
-                  void* stream) {
-  if (!ctx || !coords || !lnprob || !tuning || !flag) return fail(RBV_EINVAL, "rbv_slice_run: null argument");
-  if (n_walkers < 4) return fail(RBV_EINVAL, "rbv_slice_run: need at least four walkers (two per complement)");
-  if (n_steps < 0 || !(tuning->mu > 0.0) || tuning->maxsteps < 1 || tuning->maxiter < 1)
-    return fail(RBV_EINVAL, "rbv_slice_run: n_steps < 0, mu <= 0, maxsteps < 1 or maxiter < 1");
-  if (ctx->inst.empty() || ctx->ndim == 0) return fail(RBV_ESTATE, "rbv_slice_run: context not set up");
-  if (n_steps == 0) return RBV_OK;
-  const SliceLayout lay = slice_layout(ctx, n_walkers);
-  if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, "rbv_slice_run: workspace too small");
-  RBV_ON_DEVICE(ctx);
-  cudaStream_t st = (cudaStream_t)stream;
-  char* ws = (char*)workspace;
-  SliceParams P;
+int rbv_slice_workspace_bytes_sightlines(const RbvContext* ctx, int walkers_per_sightline, size_t* bytes) {
+  if (!ctx || !bytes || walkers_per_sightline < 4 || ctx->inst.empty())
+    return fail(RBV_EINVAL, "rbv_slice_workspace_bytes_sightlines: bad argument");
+  if (4LL * ((walkers_per_sightline + 1) / 2) * (long long)ctx->inst.size() > 0x7fffffffLL)
+    return fail(RBV_EINVAL, "rbv_slice_workspace_bytes_sightlines: too many rows");
+  *bytes = slice_layout(ctx, walkers_per_sightline, true).total;
+  return RBV_OK;
+}
+
+// Half-step buffers, loop state and settings of a run (P.mu / adapt / totals / nstep are the caller's).
+static void slice_params(RbvContext* ctx, SliceParams& P, const SliceLayout& lay, char* ws, double* coords,
+                         double* lnprob, int W, int S, const RbvSliceTuning* tuning, unsigned long long seed,
+                         int* flag) {
   P.coords = coords;
   P.lnp = lnprob;
   P.cand = (double*)(ws + lay.cand);
@@ -2836,9 +2838,10 @@ int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers
   P.walker_of = (int*)(ws + lay.walker_of);
   P.flag = flag;
   P.ctr = (SliceCounters*)(ws + lay.ctr);
+  P.nstep = (unsigned int*)(ws + lay.nstep);
   P.seed = seed;
   P.tolerance = tuning->tolerance;
-  P.W = n_walkers;
+  P.W = W;
   P.ndim = ctx->ndim;
   P.maxsteps = tuning->maxsteps;
   P.maxiter = tuning->maxiter;
@@ -2846,36 +2849,42 @@ int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers
   // logical iterations per launch (rbv_slice.cuh, "Speculation"): chains and counters do not depend on it
   P.depth = tuning->depth == 1 ? 1 : 2;
   if (ctx->tune.slice_depth > 0) P.depth = std::min(ctx->tune.slice_depth, 2);
+  P.S = S;
+}
+
+// The run loop shared by rbv_slice_run (S = 1, joint lnprob, optionally over the ranks of a communicator) and
+// rbv_slice_run_sightlines (sl: S ensembles, one sightline-mode lnprob launch per iteration).  `init` is the
+// SliceState the run starts from; on return ctx->h_poll[0] holds the final one.  chain / lnprob_chain /
+// mu_history rows are S W ndim / S W / S wide.
+static int slice_run_impl(RbvContext* ctx, SliceParams& P, const SliceLayout& lay, char* ws, size_t workspace_bytes,
+                          bool sl, const SliceState& init, int n_steps, unsigned long long first_step,
+                          double* chain, double* lnprob_chain, double* mu_history, int use_graph,
+                          cudaStream_t st, const char* who) {
+  const int n_walkers = P.W, S = P.S;
   const int rows_per_walker = 2 * P.depth;
-  {   // loop state: everything zero except mu and its adaptation state (the host slot is reused by the polls below)
-    SliceCounters init;
-    memset(&init, 0, sizeof(init));
-    init.mu = tuning->mu;
-    init.tune = tuning->tune != 0;
-    init.good = tuning->good;
-    ctx->h_poll[0] = init;
-    RBV_CUDA(cudaMemcpyAsync(P.ctr, &ctx->h_poll[0], sizeof(SliceCounters), cudaMemcpyHostToDevice, st));
-    RBV_CUDA(cudaStreamSynchronize(st));
-  }
+  ctx->h_poll[0] = init;         // the host slot is reused by the polls below
+  RBV_CUDA(cudaMemcpyAsync(P.ctr, &ctx->h_poll[0], sizeof(SliceState), cudaMemcpyHostToDevice, st));
+  RBV_CUDA(cudaStreamSynchronize(st));
   const size_t lnprob_ws_bytes = workspace_bytes - lay.lnprob_ws;
   const int h = (n_walkers + 1) / 2;
   const long long launches_before = ctx->launches;
 
-  // one iteration of half `split`: lnprob of the 2 depth n_S candidate rows (masked rows skipped) -> update + the
-  // candidates of the next iteration
+  // one iteration of half `split`: lnprob of the S x 2 depth n_S candidate rows (masked rows skipped) -> update +
+  // the candidates of the next iteration
   auto iteration = [&](int split, int rows, cudaGraphConditionalHandle loop, int use_loop) -> int {
     const int nS = split == 0 ? h : n_walkers - h;
-    const unsigned rows_grid = (unsigned)((nS + 3) / 4);
-    // multi-GPU (rbv_comm_init): this rank evaluates its share of the rows, in-place all-gather of their lnprob
+    const unsigned rows_grid = (unsigned)((S * nS + 3) / 4);
+    // multi-GPU (rbv_comm_init, single ensemble only): this rank evaluates its share of the rows, in-place
+    // all-gather of their lnprob
     int lo = 0, hi = rows, chunk = rows;
-    const bool dist = ctx->comm && ctx->comm_world > 1;
+    const bool dist = !sl && ctx->comm && ctx->comm_world > 1;
     if (dist) rank_rows(rows, ctx->comm_rank, ctx->comm_world, &lo, &hi, &chunk);
     if (hi > lo) {
       // geometry as for the 2 n_S rows of one logical iteration, whatever the depth: about half the rows of a launch
       // are masked, and the two depths then produce the same bits (measured at C2, depth 2: 1.70k steps/s with the
       // 4096-pixel tiles this picks, 1.58k with the 8192-pixel tiles picked for 4 n_S rows)
-      int rc = launch_lnprob(ctx, P.cand + (size_t)lo * ctx->ndim, hi - lo, 0, P.lnp_cand + lo, ws + lay.lnprob_ws,
-                             lnprob_ws_bytes, stream, "rbv_slice_run", nullptr, -1, P.skip + lo, 2 * nS);
+      int rc = launch_lnprob(ctx, P.cand + (size_t)lo * ctx->ndim, hi - lo, sl ? rows / S : 0, P.lnp_cand + lo,
+                             ws + lay.lnprob_ws, lnprob_ws_bytes, st, who, nullptr, -1, P.skip + lo, 2 * nS * S);
       if (rc != RBV_OK) return rc;
     }
     if (dist) {
@@ -2888,23 +2897,25 @@ int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers
   };
   auto begin = [&](unsigned long long step, int split) -> int {
     const int nS = split == 0 ? h : n_walkers - h;
-    slice_begin_kernel<<<(unsigned)((nS + 3) / 4), 128, 0, st>>>(P, step, split);
+    slice_begin_kernel<<<(unsigned)((S * nS + 3) / 4), 128, 0, st>>>(P, step, split);
     RBV_CUDA(cudaGetLastError());
-    slice_candidate_kernel<<<(unsigned)((nS + 3) / 4), 128, 0, st>>>(P, split);     // the first candidates
+    slice_candidate_kernel<<<(unsigned)((S * nS + 3) / 4), 128, 0, st>>>(P, split);     // the first candidates
     RBV_CUDA(cudaGetLastError());
     return RBV_OK;
   };
   auto record = [&](int s) -> int {
-    slice_record_kernel<<<(unsigned)((n_walkers + 3) / 4), 128, 0, st>>>(
-        P, chain ? chain + (size_t)s * n_walkers * ctx->ndim : nullptr,
-        lnprob_chain ? lnprob_chain + (size_t)s * n_walkers : nullptr, mu_history ? mu_history + s : nullptr);
+    const size_t step_rows = (size_t)S * n_walkers;
+    slice_record_kernel<<<(unsigned)((step_rows + 3) / 4), 128, 0, st>>>(
+        P, chain ? chain + (size_t)s * step_rows * ctx->ndim : nullptr,
+        lnprob_chain ? lnprob_chain + (size_t)s * step_rows : nullptr,
+        mu_history ? mu_history + (size_t)s * S : nullptr);
     RBV_CUDA(cudaGetLastError());
     return RBV_OK;
   };
 
   int rc = RBV_OK;
   long long per_iteration = 0;
-  const bool dist_run = ctx->comm && ctx->comm_world > 1;
+  const bool dist_run = !sl && ctx->comm && ctx->comm_world > 1;
   if (dist_run) {
     // multi-GPU: NCCL sets up its buffers on the first collective of a size -- do that outside any capture
     // (lnp_cand is scratch here).  The WHILE-node loop with a collective in its body is opt-in
@@ -2944,7 +2955,7 @@ int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers
                                         cudaStreamCaptureModeThreadLocal);
       if (e != cudaSuccess) break;
       const long long l0 = ctx->launches;
-      rc = iteration(split, rows_per_walker * nS, loop, 1);
+      rc = iteration(split, S * rows_per_walker * nS, loop, 1);
       per_iteration = ctx->launches - l0 + 1;
       cudaGraph_t captured = nullptr;
       e = cudaStreamEndCapture(st, &captured);
@@ -2964,7 +2975,7 @@ int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers
       if (graph[k]) cudaGraphDestroy(graph[k]);
     }
     if (rc != RBV_OK) return rc;
-    if (e != cudaSuccess) return fail(RBV_ECUDA, std::string("rbv_slice_run (graph): ") + cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail(RBV_ECUDA, std::string(who) + " (graph): " + cudaGetErrorString(e));
   } else {
     // Polling mode: iterations are enqueued one ahead of the read-back of the counters -- while the host waits for
     // those of iteration it - 1 the device already runs iteration it; when it - 1 left nothing to do, iteration it
@@ -2978,14 +2989,15 @@ int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers
         bool done = false;
         for (int it = 0; !done; ++it) {
           const long long l0 = ctx->launches;
-          rc = iteration(split, rows_per_walker * nS, 0, 0);
+          rc = iteration(split, S * rows_per_walker * nS, 0, 0);
           if (rc != RBV_OK) return rc;
           per_iteration = ctx->launches - l0 + 1;
-          RBV_CUDA(cudaMemcpyAsync(&ctx->h_poll[it & 1], P.ctr, sizeof(SliceCounters), cudaMemcpyDeviceToHost, st));
+          RBV_CUDA(cudaMemcpyAsync(&ctx->h_poll[it & 1].c, P.ctr, sizeof(SliceCounters), cudaMemcpyDeviceToHost,
+                                   st));
           RBV_CUDA(cudaEventRecord(ctx->poll_ev[it & 1], st));
           if (it >= 1) {
             RBV_CUDA(cudaEventSynchronize(ctx->poll_ev[(it - 1) & 1]));
-            const SliceCounters& c = ctx->h_poll[(it - 1) & 1];
+            const SliceCounters& c = ctx->h_poll[(it - 1) & 1].c;
             if (c.pending == 0u || c.error) done = true;
           }
         }
@@ -2993,19 +3005,101 @@ int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers
       rc = record(s);
       if (rc != RBV_OK) return rc;
     }
-    RBV_CUDA(cudaStreamSynchronize(st));
   }
-  RBV_CUDA(cudaMemcpy(&ctx->h_poll[0], P.ctr, sizeof(SliceCounters), cudaMemcpyDeviceToHost));
-  const SliceCounters& c = ctx->h_poll[0];
-  ctx->launches = launches_before + (long long)c.batches * per_iteration + 5LL * n_steps;   // + begin, candidates (x 2), record
-  tuning->mu = c.mu;
-  tuning->tune = c.tune;
-  tuning->good = c.good;
-  tuning->n_expansions = c.total_exp;
-  tuning->n_contractions = c.total_con;
-  tuning->n_calls = c.ncall;
+  RBV_CUDA(cudaMemcpyAsync(&ctx->h_poll[0], P.ctr, sizeof(SliceState), cudaMemcpyDeviceToHost, st));
+  RBV_CUDA(cudaStreamSynchronize(st));
+  // + begin, candidates (x 2), record
+  ctx->launches = launches_before + (long long)ctx->h_poll[0].c.batches * per_iteration + 5LL * n_steps;
+  return RBV_OK;
+}
+
+int rbv_slice_run(RbvContext* ctx, double* coords, double* lnprob, int n_walkers, int n_steps, RbvSliceTuning* tuning,
+                  unsigned long long seed, unsigned long long first_step, double* chain, double* lnprob_chain,
+                  double* mu_history, int* flag, void* workspace, size_t workspace_bytes, int use_graph,
+                  void* stream) {
+  if (!ctx || !coords || !lnprob || !tuning || !flag) return fail(RBV_EINVAL, "rbv_slice_run: null argument");
+  if (n_walkers < 4) return fail(RBV_EINVAL, "rbv_slice_run: need at least four walkers (two per complement)");
+  if (n_steps < 0 || !(tuning->mu > 0.0) || tuning->maxsteps < 1 || tuning->maxiter < 1)
+    return fail(RBV_EINVAL, "rbv_slice_run: n_steps < 0, mu <= 0, maxsteps < 1 or maxiter < 1");
+  if (ctx->inst.empty() || ctx->ndim == 0) return fail(RBV_ESTATE, "rbv_slice_run: context not set up");
+  if (n_steps == 0) return RBV_OK;
+  const SliceLayout lay = slice_layout(ctx, n_walkers, false);
+  if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, "rbv_slice_run: workspace too small");
+  RBV_ON_DEVICE(ctx);
+  char* ws = (char*)workspace;
+  SliceParams P;
+  slice_params(ctx, P, lay, ws, coords, lnprob, n_walkers, 1, tuning, seed, flag);
+  SliceState* dev = (SliceState*)(ws + lay.ctr);
+  P.mu = &dev->solo.mu;
+  P.adapt = dev->solo.adapt;
+  P.totals = dev->solo.totals;
+  // loop state: everything zero except mu and its adaptation state
+  SliceState init;
+  memset(&init, 0, sizeof(init));
+  init.solo.mu = tuning->mu;
+  init.solo.adapt[0] = tuning->tune != 0;
+  init.solo.adapt[1] = tuning->good;
+  int rc = slice_run_impl(ctx, P, lay, ws, workspace_bytes, false, init, n_steps, first_step, chain, lnprob_chain,
+                          mu_history, use_graph, (cudaStream_t)stream, "rbv_slice_run");
+  if (rc != RBV_OK) return rc;
+  const SliceState& c = ctx->h_poll[0];
+  tuning->mu = c.solo.mu;
+  tuning->tune = c.solo.adapt[0];
+  tuning->good = c.solo.adapt[1];
+  tuning->n_expansions = c.solo.totals[0];
+  tuning->n_contractions = c.solo.totals[1];
+  tuning->n_calls = c.solo.totals[2];
+  tuning->n_batches = c.c.batches;
+  if (c.c.error) return fail(RBV_ESTATE, "rbv_slice_run: number of contractions exceeded the maximum (maxiter)");
+  return RBV_OK;
+}
+
+int rbv_slice_run_sightlines(RbvContext* ctx, double* coords, double* lnprob, int walkers_per_sightline, int n_steps,
+                             RbvSliceTuning* tuning, double* mu, int* tune_good, unsigned long long* totals,
+                             unsigned long long seed, unsigned long long first_step, double* chain,
+                             double* lnprob_chain, double* mu_history, int* flag, void* workspace,
+                             size_t workspace_bytes, int use_graph, void* stream) {
+  const char* who = "rbv_slice_run_sightlines";
+  if (!ctx || !coords || !lnprob || !tuning || !mu || !tune_good || !totals || !flag)
+    return fail(RBV_EINVAL, std::string(who) + ": null argument");
+  const int W = walkers_per_sightline;
+  if (W < 4) return fail(RBV_EINVAL, std::string(who) + ": need at least four walkers per sightline");
+  if (n_steps < 0 || tuning->maxsteps < 1 || tuning->maxiter < 1)
+    return fail(RBV_EINVAL, std::string(who) + ": n_steps < 0, maxsteps < 1 or maxiter < 1");
+  if (ctx->inst.empty() || ctx->ndim == 0) return fail(RBV_ESTATE, std::string(who) + ": context not set up");
+  const long long S = (long long)ctx->inst.size();
+  if (S * W > 0x7fffffffLL || 4LL * ((W + 1) / 2) * S > 0x7fffffffLL)
+    return fail(RBV_EINVAL, std::string(who) + ": too many walkers");
+  const InstDev& A = ctx->inst[0].dev;
+  for (auto& hi : ctx->inst)
+    if (hi.dev.P != A.P || hi.dev.K != A.K || hi.dev.L != A.L || hi.dev.C != A.C)
+      return fail(RBV_EINVAL, std::string(who) + ": sightlines must share n_pixels, n_taps, n_lines, n_components");
+  if (n_steps == 0) return RBV_OK;
+  const SliceLayout lay = slice_layout(ctx, W, true);
+  if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, std::string(who) + ": workspace too small");
+  RBV_ON_DEVICE(ctx);
+  cudaStream_t st = (cudaStream_t)stream;
+  {   // every sightline's mu must be positive (the one read-back before the run)
+    std::vector<double> m((size_t)S);
+    RBV_CUDA(cudaMemcpyAsync(m.data(), mu, (size_t)S * sizeof(double), cudaMemcpyDeviceToHost, st));
+    RBV_CUDA(cudaStreamSynchronize(st));
+    for (double v : m)
+      if (!(v > 0.0)) return fail(RBV_EINVAL, std::string(who) + ": mu <= 0");
+  }
+  char* ws = (char*)workspace;
+  SliceParams P;
+  slice_params(ctx, P, lay, ws, coords, lnprob, W, (int)S, tuning, seed, flag);
+  P.mu = mu;
+  P.adapt = tune_good;
+  P.totals = totals;
+  SliceState init;
+  memset(&init, 0, sizeof(init));
+  int rc = slice_run_impl(ctx, P, lay, ws, workspace_bytes, true, init, n_steps, first_step, chain, lnprob_chain,
+                          mu_history, use_graph, st, who);
+  if (rc != RBV_OK) return rc;
+  const SliceCounters& c = ctx->h_poll[0].c;
   tuning->n_batches = c.batches;
-  if (c.error) return fail(RBV_ESTATE, "rbv_slice_run: number of contractions exceeded the maximum (maxiter)");
+  if (c.error) return fail(RBV_ESTATE, std::string(who) + ": number of contractions exceeded the maximum (maxiter)");
   return RBV_OK;
 }
 

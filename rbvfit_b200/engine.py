@@ -715,6 +715,42 @@ class Engine:
             int(bool(use_graph)), self._stream()), "rbv_slice_run")
         return mus_t.cpu().numpy()[:int(n_steps)]
 
+    def slice_run_sightlines(self, coords_t, lnp_t, n_steps: int, tuning, mu_t, tune_good_t, totals_t, seed: int,
+                             first_step: int, chain_t, lnp_chain_t, mu_history_t, flag_t, use_graph: bool = True):
+        """Survey-mode ensemble slice sampling (rbv_slice_run_sightlines) on the current torch stream: ``coords_t``
+        [S, W, ndim], one ensemble per sightline of this context, all advancing in lockstep.  ``tuning`` is an
+        ``RbvSliceTuning`` carrying the settings every sightline shares (its ``n_batches`` is written); each
+        sightline's state is on the device and updated in place: ``mu_t`` [S] f64, ``tune_good_t`` [S, 2] i32,
+        ``totals_t`` [S, 3] i64 (expansions, contractions, likelihood rows; accumulated).  ``mu_history_t``
+        [n_steps, S] or None.  The call returns when the run is done."""
+        torch = _torch()
+        S, W, ndim = coords_t.shape
+        if ndim != self.ndim or S != len(self.pixels):
+            raise ValueError(f"coords must be [{len(self.pixels)}, walkers_per_sightline, {self.ndim}]")
+        for t, dt in ((coords_t, torch.float64), (lnp_t, torch.float64), (flag_t, torch.int32)):
+            if t.dtype != dt or not t.is_contiguous() or t.device != self.tdev:
+                raise ValueError("sampler state tensors must be contiguous, on the engine's device, f64 / i32")
+        self._dev_tensor(lnp_t, torch.float64, "lnprob", (S, W))
+        self._dev_tensor(mu_t, torch.float64, "mu", (S,))
+        self._dev_tensor(tune_good_t, torch.int32, "tune / good", (S, 2))
+        self._dev_tensor(totals_t, torch.int64, "totals", (S, 3))
+        self._dev_tensor(chain_t, torch.float64, "chain", (int(n_steps), S, W, ndim))
+        self._dev_tensor(lnp_chain_t, torch.float64, "lnprob chain", (int(n_steps), S, W))
+        self._dev_tensor(mu_history_t, torch.float64, "mu history", (int(n_steps), S))
+        nbytes = C.c_size_t(0)
+        check(self.lib.rbv_slice_workspace_bytes_sightlines(self._h, W, C.byref(nbytes)),
+              "rbv_slice_workspace_bytes_sightlines")
+        if self._slice_ws is None or self._slice_ws.numel() < nbytes.value:
+            self._slice_ws = torch.empty(int(nbytes.value), dtype=torch.uint8, device=self.tdev)
+        check(self.lib.rbv_slice_run_sightlines(
+            self._h, coords_t.data_ptr(), lnp_t.data_ptr(), W, int(n_steps), C.byref(tuning), mu_t.data_ptr(),
+            tune_good_t.data_ptr(), totals_t.data_ptr(), int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_step),
+            chain_t.data_ptr() if chain_t is not None else None,
+            lnp_chain_t.data_ptr() if lnp_chain_t is not None else None,
+            mu_history_t.data_ptr() if mu_history_t is not None else None,
+            flag_t.data_ptr(), self._slice_ws.data_ptr(), self._slice_ws.numel(), int(bool(use_graph)),
+            self._stream()), "rbv_slice_run_sightlines")
+
     def model_flux(self, inst: int, theta: np.ndarray, convolve: bool = True) -> np.ndarray:
         """HOST theta [W, ndim] -> HOST model flux [W, P] of instrument ``inst``; ``convolve=False`` skips the LSF
         (``VoigtModel.evaluate(return_unconvolved=True)``)."""

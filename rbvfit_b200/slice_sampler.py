@@ -315,3 +315,245 @@ class DistributedDeviceSliceSampler(DeviceEnsembleSliceSampler):
             from ._lib import RbvError
             raise RbvError("the peer-memory all-gather gave up waiting for a rank (30 s without its rows)")
         return out
+
+
+class _SliceSightlineView:
+    """One sightline of a ``SightlineEnsembleSliceSampler`` behind ``DeviceEnsembleSliceSampler``'s (zeus's) accessor
+    contract -- what a caller hands to the reference's ``UnifiedResults`` for that sightline."""
+
+    def __init__(self, parent, index: int):
+        self._p, self._s = parent, int(index)
+        self.nwalkers, self.ndim = parent.nwalkers, parent.ndim
+
+    @property
+    def iteration(self):
+        return self._p.iteration
+
+    def get_chain(self, flat=False, thin=1, discard=0):
+        return self._p.get_chain(flat=flat, thin=thin, discard=discard, sightline=self._s)
+
+    def get_log_prob(self, flat=False, thin=1, discard=0):
+        return self._p.get_log_prob(flat=flat, thin=thin, discard=discard, sightline=self._s)
+
+    @property
+    def chain(self):
+        return self.get_chain()
+
+    @property
+    def acceptance_fraction(self):
+        return self._p.acceptance_fraction[self._s]
+
+    @property
+    def efficiency(self):
+        return float(self._p.efficiency[self._s])
+
+    @property
+    def mu(self):
+        return float(self._p.mu[self._s])
+
+    @property
+    def tune(self):
+        return bool(self._p.tune[self._s])
+
+    @property
+    def mus(self):
+        return self._p.mus[:, self._s]
+
+    @property
+    def ncall(self):
+        return int(self._p.ncall[self._s])
+
+    @property
+    def nexp(self):
+        return int(self._p.nexp[self._s])
+
+    @property
+    def ncon(self):
+        return int(self._p.ncon[self._s])
+
+    @property
+    def nbatches(self):
+        return self._p.nbatches
+
+    def get_autocorr_time(self, discard=0, thin=1, **kwargs):
+        return thin * integrated_time(self.get_chain(discard=discard, thin=thin), **kwargs)
+
+    def get_last_sample(self):
+        last = self._p.get_last_sample()
+        return None if last is None else (last[0][self._s], last[1][self._s])
+
+
+class SightlineEnsembleSliceSampler(_ChunkedHistory):
+    """Survey mode of ``DeviceEnsembleSliceSampler``: one zeus ensemble PER SIGHTLINE of a ``SightlineBatch``, all S
+    ensembles advancing in lockstep on the device (``rbv_slice_run_sightlines``) -- the reference would run S separate
+    ``vfit(..., sampler='zeus')`` fits one after the other.  Every iteration of a half-step is ONE sightline
+    likelihood launch over the candidate rows of every sightline; a sightline whose walkers have finished masks its
+    rows.  Each sightline keeps its own mu, tuning state and counters, exactly as S separate samplers would: its chain
+    does not depend on the other sightlines, and sightline 0 reproduces ``DeviceEnsembleSliceSampler`` with the same
+    seed on that sightline alone (same random streams, walker counter offset by s W for sightline s).  Sightlines
+    shard across GPUs with no collective: every rank runs this sampler over its own ``SightlineBatch``.
+
+    Accessors follow zeus (``arr[discard::thin]``): ``get_chain`` [steps, S, W, ndim], ``sightline=s`` -> [steps, W,
+    ndim]; ``flat`` merges the steps and walkers of each sightline, never across sightlines.  Per sightline: ``mu``,
+    ``tune``, ``ncall``, ``nexp``, ``ncon``, ``efficiency`` [S], ``mus`` [steps, S] (mu after every step),
+    ``acceptance_fraction`` [S, W]; ``nbatches`` counts likelihood launches.  ``sightline(s)`` returns a one-sightline
+    view with ``DeviceEnsembleSliceSampler``'s accessors."""
+
+    def __init__(self, nwalkers: int, ndim: int, batch, mu: float = 1.0, tune: bool = True,
+                 tolerance: float = 0.05, patience: int = 5, maxsteps: int = 10000, maxiter: int = 10000,
+                 seed: Optional[int] = None, use_graph: bool = True, depth: int = 2):
+        from .likelihood import SightlineBatch
+        if not isinstance(batch, SightlineBatch):
+            raise TypeError("SightlineEnsembleSliceSampler needs a SightlineBatch")
+        if batch.ndim != ndim:
+            raise ValueError(f"the sightline batch has ndim={batch.ndim}, sampler was given ndim={ndim}")
+        if nwalkers < 2 * ndim or nwalkers % 2:
+            raise ValueError("Please provide at least (2 * ndim) walkers, and an even number of them.")
+        if not mu > 0:
+            raise ValueError("mu must be positive")
+        if depth not in (1, 2):
+            raise ValueError("depth must be 1 or 2")
+        self.batch = batch
+        self.n_sightlines = int(batch.n_sightlines)
+        self.nwalkers, self.ndim = int(nwalkers), int(ndim)
+        self.mu0, self.tune0 = float(mu), bool(tune)
+        self.tolerance, self.patience = float(tolerance), int(patience)
+        self.maxsteps, self.maxiter = int(maxsteps), int(maxiter)
+        self.use_graph, self.depth = bool(use_graph), int(depth)
+        self._seed = int(np.random.SeedSequence(seed).generate_state(1, dtype=np.uint64)[0])
+        self._stream = None
+        self.reset()
+
+    def reset(self):
+        import torch
+        S, W, nd = self.n_sightlines, self.nwalkers, self.ndim
+        dev = self.batch.engine.tdev
+        self._chain = np.empty((0, S, W, nd))
+        self._log_prob = np.empty((0, S, W))
+        self._mus = []
+        self.iteration = 0
+        self.nbatches = 0
+        self._init_calls = np.zeros(S, dtype=np.int64)
+        # per-sightline state of rbv_slice_run_sightlines, kept on the device between runs
+        self._mu_t = torch.full((S,), self.mu0, dtype=torch.float64, device=dev)
+        self._tune_good_t = torch.zeros((S, 2), dtype=torch.int32, device=dev)
+        self._tune_good_t[:, 0] = int(self.tune0)
+        self._totals_t = torch.zeros((S, 3), dtype=torch.int64, device=dev)
+        self._pull_state()
+        self._state = None
+        self._last = None
+
+    def _pull_state(self):
+        self.mu = self._mu_t.cpu().numpy()
+        tg = self._tune_good_t.cpu().numpy()
+        self.tune, self.good = tg[:, 0] != 0, tg[:, 1].copy()
+        tot = self._totals_t.cpu().numpy()
+        self.nexp, self.ncon = tot[:, 0].copy(), tot[:, 1].copy()
+        self.ncall = self._init_calls + tot[:, 2]
+
+    def run_mcmc(self, start, nsteps, progress=False, **_ignored):
+        """``start`` [S, W, ndim], or None to continue the last run; returns the last sample (coords [S, W, ndim],
+        lnprob [S, W])."""
+        import torch
+        from ._lib import RbvSliceTuning
+        eng = self.batch.engine
+        dev = eng.tdev
+        S, W, nd = self.n_sightlines, self.nwalkers, self.ndim
+        if self._stream is None:
+            self._stream = torch.cuda.Stream(device=dev)
+        torch.cuda.current_stream(dev).synchronize()
+        with torch.cuda.stream(self._stream):
+            if start is None:
+                if self._state is None:
+                    raise ValueError("Cannot have `start=None` if run_mcmc has never been called.")
+                coords_t, lnp_t = self._state
+            else:
+                X = np.array(start, dtype=np.float64, copy=True)
+                if X.shape != (S, W, nd):
+                    raise ValueError(f"Incompatible input dimensions! Please provide array of shape ({S}, {W}, {nd})")
+                coords_t = torch.as_tensor(X, device=dev)
+                lnp_t = eng.lnprob_sightlines_device(coords_t.view(S * W, nd), W).view(S, W)
+                self._init_calls += W
+                self.nbatches += 1
+                if not bool(torch.isfinite(lnp_t).all()):
+                    raise ValueError("Invalid walker initial positions! Initialise walkers from positions of "
+                                     "finite log probability.")
+            chain_t = torch.empty((nsteps, S, W, nd), dtype=torch.float64, device=dev)
+            lps_t = torch.empty((nsteps, S, W), dtype=torch.float64, device=dev)
+            mus_t = torch.empty((nsteps, S), dtype=torch.float64, device=dev)
+            flag_t = torch.zeros(1, dtype=torch.int32, device=dev)
+            tuning = RbvSliceTuning(tolerance=self.tolerance, patience=self.patience, maxsteps=self.maxsteps,
+                                    maxiter=self.maxiter, depth=self.depth)
+            try:
+                eng.slice_run_sightlines(coords_t, lnp_t, nsteps, tuning, self._mu_t, self._tune_good_t,
+                                         self._totals_t, self._seed, self.iteration, chain_t, lps_t, mus_t, flag_t,
+                                         use_graph=self.use_graph)
+            finally:
+                self._stream.synchronize()
+                self.nbatches += int(tuning.n_batches)
+                self._pull_state()
+            if int(flag_t.item()) & 1:
+                raise ValueError("Probability function returned NaN")
+            self._state = (coords_t, lnp_t)
+            chain, lps = chain_t.cpu().numpy(), lps_t.cpu().numpy()
+            self._mus.append(mus_t.cpu().numpy())
+        self._hist_append(chain, lps)
+        self.iteration += nsteps
+        if nsteps:
+            self._last = (chain[-1].copy(), lps[-1].copy())
+        return self._last
+
+    # ------------------------------------------------------------------ zeus-shaped accessors
+    def _get(self, arr, discard, thin, flat, sightline):
+        v = arr[discard::thin]
+        if sightline is not None:
+            v = v[:, int(sightline)]
+            if flat:
+                return v.reshape((-1,) + v.shape[2:])
+            return v
+        if flat:                                  # [S, steps * W, ...]: flat per sightline, never across sightlines
+            v = np.swapaxes(v, 0, 1)
+            return v.reshape((v.shape[0], -1) + v.shape[3:])
+        return v
+
+    def get_chain(self, flat=False, thin=1, discard=0, sightline=None):
+        """[steps, S, W, ndim]; ``sightline=s`` -> [steps, W, ndim]; ``flat`` merges the steps and walkers of each
+        sightline (never across sightlines)."""
+        return self._get(self._chain, discard, thin, flat, sightline)
+
+    def get_log_prob(self, flat=False, thin=1, discard=0, sightline=None):
+        return self._get(self._log_prob, discard, thin, flat, sightline)
+
+    @property
+    def chain(self):
+        return self._chain
+
+    @property
+    def mus(self):
+        """[steps, S]: every sightline's mu after each step"""
+        if not self._mus:
+            return np.empty((0, self.n_sightlines))
+        if len(self._mus) > 1:
+            self._mus[:] = [np.concatenate(self._mus, axis=0)]
+        return self._mus[0]
+
+    @property
+    def acceptance_fraction(self):
+        """[S, W]: fraction of steps in which the walker moved (slice moves always move, so ~1)"""
+        c = self._chain
+        if len(c) < 2:
+            return np.ones((self.n_sightlines, self.nwalkers))
+        return np.mean(np.any(c[1:] != c[:-1], axis=3), axis=0)
+
+    @property
+    def efficiency(self):
+        """[S]"""
+        return self.iteration * self.nwalkers / np.maximum(self.ncall, 1)
+
+    def sightline(self, index: int) -> _SliceSightlineView:
+        if not 0 <= int(index) < self.n_sightlines:
+            raise IndexError(index)
+        return _SliceSightlineView(self, index)
+
+    def get_last_sample(self):
+        return self._last
