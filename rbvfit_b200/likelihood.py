@@ -281,7 +281,7 @@ class SightlineBatch:
             if mask is not None:     # extension: pixels with False do not enter the likelihood (both terms exactly 0)
                 mask = np.asarray(mask, dtype=bool)
                 if mask.shape != wave.shape:
-                    raise ValueError(f"instrument_data['{name}']: weight_mask must have the shape of wave")
+                    raise ValueError(f"sightline {i}: weight_mask must have the shape of wave")
                 inv_sigma2 = np.where(mask, inv_sigma2, inv_sigma2.dtype.type(0))
                 log_inv_sigma2 = np.where(mask, log_inv_sigma2, log_inv_sigma2.dtype.type(0))
             data = compiled.data
