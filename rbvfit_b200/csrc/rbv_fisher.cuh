@@ -18,6 +18,8 @@
 //   fisher_jac_out_kernel  (256 px, row, walker)   rbv_model_jacobian_batch only: [W, ndim, P] out of JM / JF
 // Every reduction runs in an order fixed by the instrument geometry alone (no atomics): a row's results do not
 // depend on the batch size or on the position of the row in the batch.
+// The launches with the walker in grid y or z go over the batch in slices of at most 65 535 rows (the CUDA limit of
+// gridDim.y / gridDim.z): row gp.w0 + blockIdx.y (.z) of the full-size buffers, as in rbv_grad.cuh.
 // Survey mode (SL = true, SlRows of rbv_grad.cuh): the same kernels with the geometry of one sightline and the
 // row's own instrument, so a row gives bit for bit what a one-instrument context of that sightline gives.
 #pragma once
@@ -75,7 +77,7 @@ template <bool SL>
 __global__ void __launch_bounds__(kGradBlock) fisher_col_kernel(const FisherParams fp, const SlRows sl) {
   __shared__ double s_q[kGradLineChunk][2][kNQNear];
   const GradParams& prm = fp.gp;
-  const int w = blockIdx.y, tid = threadIdx.x;
+  const int w = prm.w0 + blockIdx.y, tid = threadIdx.x;
   if (sl_skip<SL>(sl, w)) return;
   const int k = SL ? 0 : grad_inst_of_blk(prm, blockIdx.x);
   const int ki = sl_inst<SL>(sl, w, k);
@@ -125,7 +127,7 @@ __global__ void __launch_bounds__(kGradBlock) fisher_col_kernel(const FisherPara
 template <bool SL>
 __global__ void __launch_bounds__(kGradBlock) fisher_lsf_kernel(const FisherParams fp, const SlRows sl) {
   const GradParams& prm = fp.gp;
-  const int w = blockIdx.z, col = blockIdx.y;
+  const int w = prm.w0 + blockIdx.z, col = blockIdx.y;
   if (sl_skip<SL>(sl, w)) return;
   const int k = SL ? 0 : grad_inst_of_blk(prm, blockIdx.x);
   const int ki = sl_inst<SL>(sl, w, k);
@@ -146,7 +148,7 @@ template <bool SL>
 __global__ void __launch_bounds__(kGradBlock) fisher_gram_kernel(const FisherParams fp, const SlRows sl) {
   extern __shared__ double s_j[];   // [ncol][kFisherChunk] columns, then weights, then residuals
   const GradParams& prm = fp.gp;
-  const int w = blockIdx.y, tid = threadIdx.x;
+  const int w = prm.w0 + blockIdx.y, tid = threadIdx.x;
   if (sl_skip<SL>(sl, w)) return;
   const int k = SL ? 0 : grad_inst_of_tile(prm, blockIdx.x);
   const int ki = sl_inst<SL>(sl, w, k);
@@ -234,7 +236,7 @@ __global__ void __launch_bounds__(128) fisher_finalize_kernel(const FisherParams
 // rbv_model_jacobian_batch: out[w, i, p] = dM_p/dtheta_i of instrument jac_inst, rows beyond ncol zero
 __global__ void __launch_bounds__(kGradBlock) fisher_jac_out_kernel(const FisherParams fp) {
   const GradParams& prm = fp.gp;
-  const int k = fp.jac_inst, w = blockIdx.z, i = blockIdx.y;
+  const int k = fp.jac_inst, w = prm.w0 + blockIdx.z, i = blockIdx.y;
   const InstDev& I = prm.inst[k];
   const int p = blockIdx.x * kGradBlock + threadIdx.x;
   if (p >= I.P) return;

@@ -19,6 +19,8 @@
 //   grad_finalize_kernel (warp per walker)     fixed-order sums over blocks, tiles, lines and instruments
 // Every reduction runs in an order fixed by the instrument geometry alone: a row's value and gradient do not depend
 // on the batch size or on the position of the row in the batch.
+// The launches with the walker in grid y (flux, resid, adjoint, line) go over the batch in slices of at most 65 535
+// rows, the CUDA limit of gridDim.y / gridDim.z: row GradParams::w0 + blockIdx.y of the full-size buffers.
 #pragma once
 
 namespace rbv {
@@ -58,6 +60,7 @@ struct GradParams {
   double* linegrad;       // [W, n_lines_total, 3]
   long long part_stride;
   int W, ndim, n_inst, n_lines_total, n_blk_total, n_tiles_total;
+  int w0;                 // first row of a launch with the row in grid y / z (a slice of at most 65 535 rows)
 };
 
 // Survey mode of the forward and Fisher kernels (template parameter SL): row w is evaluated against instrument
@@ -284,7 +287,7 @@ __global__ void __launch_bounds__(128) grad_prep_kernel(const GradParams prm, co
 // tau over every line, directly, then F = exp(-tau)
 template <bool SL>
 __global__ void __launch_bounds__(kGradBlock) grad_flux_kernel(const GradParams prm, const SlRows sl) {
-  const int w = blockIdx.y;
+  const int w = prm.w0 + blockIdx.y;
   if (sl_skip<SL>(sl, w)) return;
   if (prm.oob[w]) return;
   const int k = SL ? 0 : grad_inst_of_blk(prm, blockIdx.x);
@@ -312,7 +315,7 @@ __global__ void __launch_bounds__(kGradBlock) grad_flux_kernel(const GradParams 
 template <bool SL>
 __global__ void __launch_bounds__(kGradBlock) grad_resid_kernel(const GradParams prm, const SlRows sl) {
   __shared__ double s_red[kGradBlock / 32];
-  const int w = blockIdx.y;
+  const int w = prm.w0 + blockIdx.y;
   if (sl_skip<SL>(sl, w)) return;
   if (prm.oob[w]) return;
   const int k = SL ? 0 : grad_inst_of_blk(prm, blockIdx.x);
@@ -344,7 +347,7 @@ __global__ void __launch_bounds__(kGradBlock) grad_resid_kernel(const GradParams
 // s_q = sum_p r_p dM_p/dF_q, g_q = -F_q s_q.  Interior q: the taps that land on q exactly; q = 0 and q = P - 1 also
 // collect every tap that the edge replication clamps onto them (prefix / suffix sums of the taps).
 __global__ void __launch_bounds__(kGradBlock) grad_adjoint_kernel(const GradParams prm) {
-  const int w = blockIdx.y;
+  const int w = prm.w0 + blockIdx.y;
   if (prm.oob[w]) return;
   const int k = grad_inst_of_blk(prm, blockIdx.x);
   const InstDev& I = prm.inst[k];
@@ -372,7 +375,7 @@ __global__ void __launch_bounds__(kGradBlock) grad_adjoint_kernel(const GradPara
 __global__ void __launch_bounds__(kGradBlock) grad_line_kernel(const GradParams prm) {
   __shared__ double s_q[kGradLineChunk][2][kNQNear];
   __shared__ double s_part[kGradLineChunk][kGradBlock / 32][3];
-  const int w = blockIdx.y;
+  const int w = prm.w0 + blockIdx.y;
   if (prm.oob[w]) return;
   int k = 0;
   while (k + 1 < prm.n_inst && (int)blockIdx.x >= prm.gi[k + 1].tile_off) ++k;

@@ -3260,6 +3260,26 @@ int rbv_grad_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* bytes
   return RBV_OK;
 }
 
+// Launches with the row in grid y or z (gradient, Fisher, Jacobian): CUDA caps gridDim.y / gridDim.z at 65 535, so
+// such a launch goes over the batch in slices [w0, w0 + n) of at most that many rows, every kernel indexing the
+// full-size buffers with row w0 + blockIdx.y (.z).  Nothing is reduced across rows, so a row's results do not depend
+// on the slicing; a batch of up to 65 535 rows is one launch as before.  launch(n) enqueues the kernel of one slice
+// with the current prm.w0.
+constexpr int kMaxGridRows = 65535;
+extern "C++" {
+template <class Launch>
+static int launch_row_slices(RbvContext* ctx, GradParams& prm, int W, Launch launch) {
+  for (int w0 = 0; w0 < W; w0 += kMaxGridRows) {
+    prm.w0 = w0;
+    launch((unsigned)std::min(kMaxGridRows, W - w0));
+    RBV_CUDA(cudaGetLastError());
+    ctx->launches++;
+  }
+  prm.w0 = 0;
+  return RBV_OK;
+}
+}  // extern "C++"
+
 int rbv_lnprob_grad_batch(RbvContext* ctx, const double* theta, int W, int apply_prior, double* value, double* grad,
                           void* workspace, size_t workspace_bytes, void* stream) {
   const char* who = "rbv_lnprob_grad_batch";
@@ -3322,17 +3342,22 @@ int rbv_lnprob_grad_batch(RbvContext* ctx, const double* theta, int W, int apply
   cudaStream_t st = (cudaStream_t)stream;
   grad_prep_kernel<false><<<dim3(W, (ctx->n_lines_total + 127) / 128), 128, 0, st>>>(prm, SlRows{});
   RBV_CUDA(cudaGetLastError());
-  grad_flux_kernel<false><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm, SlRows{});
-  RBV_CUDA(cudaGetLastError());
-  grad_resid_kernel<false><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm, SlRows{});
-  RBV_CUDA(cudaGetLastError());
-  grad_adjoint_kernel<<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm);
-  RBV_CUDA(cudaGetLastError());
-  grad_line_kernel<<<dim3(lay.n_tiles_total, W), kGradBlock, 0, st>>>(prm);
-  RBV_CUDA(cudaGetLastError());
+  ctx->launches++;
+  RBV_CHECK(launch_row_slices(ctx, prm, W, [&](unsigned n) {
+    grad_flux_kernel<false><<<dim3(lay.n_blk_total, n), kGradBlock, 0, st>>>(prm, SlRows{});
+  }));
+  RBV_CHECK(launch_row_slices(ctx, prm, W, [&](unsigned n) {
+    grad_resid_kernel<false><<<dim3(lay.n_blk_total, n), kGradBlock, 0, st>>>(prm, SlRows{});
+  }));
+  RBV_CHECK(launch_row_slices(ctx, prm, W, [&](unsigned n) {
+    grad_adjoint_kernel<<<dim3(lay.n_blk_total, n), kGradBlock, 0, st>>>(prm);
+  }));
+  RBV_CHECK(launch_row_slices(ctx, prm, W, [&](unsigned n) {
+    grad_line_kernel<<<dim3(lay.n_tiles_total, n), kGradBlock, 0, st>>>(prm);
+  }));
   grad_finalize_kernel<<<(W + 3) / 4, 128, 0, st>>>(prm);
   RBV_CUDA(cudaGetLastError());
-  ctx->launches += 6;
+  ctx->launches++;
   return RBV_OK;
 }
 
@@ -3442,37 +3467,38 @@ static int fisher_setup(RbvContext* ctx, const char* who, const double* theta, i
 // prep -> flux [-> resid] -> columns [-> LSF] [-> Gram -> finalize]
 extern "C++" {
 template <bool SL>
-static int fisher_launch(RbvContext* ctx, const FisherParams& fp, const FisherLayout& lay, bool with_resid,
+static int fisher_launch(RbvContext* ctx, const FisherParams& fp_in, const FisherLayout& lay, bool with_resid,
                          bool any_lsf, bool gram, const SlRows& sl, cudaStream_t st) {
+  FisherParams fp = fp_in;          // fp.gp.w0 walks the row slices (launch_row_slices)
   const GradParams& prm = fp.gp;
   const int W = prm.W;
   grad_prep_kernel<SL><<<dim3(W, (prm.n_lines_total + 127) / 128), 128, 0, st>>>(prm, sl);
   RBV_CUDA(cudaGetLastError());
-  grad_flux_kernel<SL><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm, sl);
-  RBV_CUDA(cudaGetLastError());
-  ctx->launches += 2;
-  if (with_resid) {
-    grad_resid_kernel<SL><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(prm, sl);
-    RBV_CUDA(cudaGetLastError());
-    ctx->launches++;
-  }
-  fisher_col_kernel<SL><<<dim3(lay.n_blk_total, W), kGradBlock, 0, st>>>(fp, sl);
-  RBV_CUDA(cudaGetLastError());
   ctx->launches++;
-  if (any_lsf) {
-    fisher_lsf_kernel<SL><<<dim3(lay.n_blk_total, lay.ncol, W), kGradBlock, 0, st>>>(fp, sl);
-    RBV_CUDA(cudaGetLastError());
-    ctx->launches++;
-  }
+  RBV_CHECK(launch_row_slices(ctx, fp.gp, W, [&](unsigned n) {
+    grad_flux_kernel<SL><<<dim3(lay.n_blk_total, n), kGradBlock, 0, st>>>(prm, sl);
+  }));
+  if (with_resid)
+    RBV_CHECK(launch_row_slices(ctx, fp.gp, W, [&](unsigned n) {
+      grad_resid_kernel<SL><<<dim3(lay.n_blk_total, n), kGradBlock, 0, st>>>(prm, sl);
+    }));
+  RBV_CHECK(launch_row_slices(ctx, fp.gp, W, [&](unsigned n) {
+    fisher_col_kernel<SL><<<dim3(lay.n_blk_total, n), kGradBlock, 0, st>>>(fp, sl);
+  }));
+  if (any_lsf)
+    RBV_CHECK(launch_row_slices(ctx, fp.gp, W, [&](unsigned n) {
+      fisher_lsf_kernel<SL><<<dim3(lay.n_blk_total, lay.ncol, n), kGradBlock, 0, st>>>(fp, sl);
+    }));
   if (!gram) return RBV_OK;
   const size_t smem = (size_t)(lay.ncol + 2) * kFisherChunk * sizeof(double);
   if (smem > 48 * 1024)
     RBV_CUDA(cudaFuncSetAttribute(fisher_gram_kernel<SL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  fisher_gram_kernel<SL><<<dim3(lay.n_tiles_total, W), kGradBlock, smem, st>>>(fp, sl);
-  RBV_CUDA(cudaGetLastError());
+  RBV_CHECK(launch_row_slices(ctx, fp.gp, W, [&](unsigned n) {
+    fisher_gram_kernel<SL><<<dim3(lay.n_tiles_total, n), kGradBlock, smem, st>>>(fp, sl);
+  }));
   fisher_finalize_kernel<SL><<<(W + 3) / 4, 128, 0, st>>>(fp, sl);
   RBV_CUDA(cudaGetLastError());
-  ctx->launches += 2;
+  ctx->launches++;
   return RBV_OK;
 }
 }  // extern "C++"
@@ -3563,10 +3589,9 @@ int rbv_model_jacobian_batch(RbvContext* ctx, int inst, const double* theta, int
   fp.jac = out_jac;
   fp.jac_inst = inst;
   const int P = ctx->inst[inst].dev.P;
-  fisher_jac_out_kernel<<<dim3((P + kGradBlock - 1) / kGradBlock, ctx->ndim, W), kGradBlock, 0, st>>>(fp);
-  RBV_CUDA(cudaGetLastError());
-  ctx->launches++;
-  return RBV_OK;
+  return launch_row_slices(ctx, fp.gp, W, [&](unsigned n) {
+    fisher_jac_out_kernel<<<dim3((P + kGradBlock - 1) / kGradBlock, ctx->ndim, n), kGradBlock, 0, st>>>(fp);
+  });
 }
 
 // ------------------------------------------------------------------------------------------ survey-mode LM
