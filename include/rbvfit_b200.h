@@ -267,6 +267,50 @@ int rbv_stretch_run_sightlines(RbvContext* ctx, double* coords, double* lnprob, 
                                double* lnprob_chain, int* n_accepted, int* flag, void* workspace,
                                size_t workspace_bytes, void* stream);
 
+/* Parallel tempering on the device (ptemcee's algorithm: Vousden, Farr & Mandel 2016): n_temps = T ensembles of
+ * n_walkers = W walkers sample prior x L^beta_t on the ladder betas, 1 = beta_0 > beta_1 > ... >= 0, and exchange
+ * states between adjacent temperatures once per step.  A step = two half-steps of the stretch move over all T
+ * ensembles (partners from the same temperature; ONE joint-mode lnprob launch over the T ceil(W/2) proposal rows;
+ * accept against the tempered target, a -inf proposal always rejected, a walker at -inf always moving) -> the swap
+ * stage, hottest pair first: walker p_i(k) of temperature i and q_i(k) of i - 1 exchange coords and lnprob when
+ * ln u < (beta_{i-1} - beta_i)(lnL_{i,p} - lnL_{i-1,q}) -> the record of the state after the swaps.  Every walker keeps
+ * its UNTEMPERED lnprob (ln L inside the bounds of rbv_set_bounds, -inf outside).  Random streams: those of
+ * rbv_stretch_run with the walker counter offset by t * W (purposes 5 and 6 for the swaps, see rbv_pt.cuh), so T = 1
+ * reproduces rbv_stretch_run's chain with the same seed bit for bit, and a run continued with first_step = steps
+ * already done reproduces one long run.  voigt_method, precision and far-field settings act as in rbv_lnprob_batch.
+ * Rows are never split across ranks: an attached communicator is not used.
+ *   coords        DEVICE [T, W, ndim], updated in place;  lnprob DEVICE [T, W] (untempered), updated in place
+ *   betas         DEVICE [T], in/out: the ladder (betas[0] = 1, strictly decreasing, >= 0); adapted in place when
+ *                 control->adapt is set
+ *   control       HOST, see RbvPtControl
+ *   chain         DEVICE [n_steps, n_record, W, ndim] or NULL: coordinates of the n_record coldest temperatures
+ *   lnprob_chain  DEVICE [n_steps, T, W] or NULL: untempered lnprob of every temperature (thermodynamic integration)
+ *   sink          HOST or NULL: instead of chain / lnprob_chain (which must then be NULL), the chain is handed to the
+ *                 host as in rbv_stretch_run_sink, with a step of n_record * W * ndim chain and T * W lnprob doubles:
+ *                 ring_dev / ring_pinned hold 2 * block_steps * (n_record * W * ndim + T * W) doubles; needs
+ *                 use_graph, a non-default stream and n_steps >= 4
+ *   beta_history  DEVICE [n_steps, T] or NULL: the ladder each step ran with
+ *   n_accepted    DEVICE int[T, W], accumulated accepted stretch moves
+ *   n_swaps_accepted  DEVICE uint64[T - 1], accumulated accepted swaps of pair (i, i + 1) (NULL allowed for T = 1)
+ *   flag          DEVICE int, bit 0 set if a proposal's lnprob was NaN
+ *   workspace     DEVICE, rbv_pt_workspace_bytes();  use_graph as in rbv_stretch_run.  The call copies betas to the
+ *                 host to check them (a synchronisation on `stream`); with use_graph it returns after the run. */
+typedef struct RbvPtControl {
+  double a;                             /* stretch scale (> 1; emcee's default 2)                                 */
+  int adapt;                            /* != 0: adapt the interior of the ladder after every step (burn-in only:
+                                         * it breaks detailed balance)                                            */
+  double adaptation_lag;                /* ptemcee: 10000                                                        */
+  double adaptation_time;               /* ptemcee: 100                                                          */
+  unsigned long long adapt_steps_done;  /* adaptation steps of earlier calls (continues the decay of kappa)       */
+  int n_record;                         /* coldest temperatures whose coordinates are recorded, 1 .. T          */
+} RbvPtControl;
+int rbv_pt_workspace_bytes(const RbvContext* ctx, int n_temps, int n_walkers, size_t* bytes);
+int rbv_pt_run(RbvContext* ctx, double* coords, double* lnprob, double* betas, int n_temps, int n_walkers,
+               int n_steps, const RbvPtControl* control, unsigned long long seed, unsigned long long first_step,
+               double* chain, double* lnprob_chain, const RbvChainSink* sink, double* beta_history, int* n_accepted,
+               unsigned long long* n_swaps_accepted, int* flag, void* workspace, size_t workspace_bytes,
+               int use_graph, void* stream);
+
 /* Device-resident ensemble slice sampler (differential move).  Replaces the sampling loop
  * zeus.EnsembleSampler(nwalkers, ndim, self.lnprob).run_mcmc(guesses, no_of_steps), vfit_mcmc.py:425-440, 536-540
  * (zeus-mcmc >= 2.3.0 is not vendored in the reference; Karamanis & Beutler 2021, Algorithms 2-3 with zeus's defaults,

@@ -42,6 +42,11 @@ class RbvChainSink(C.Structure):
                 ("ring_pinned", C.c_void_p), ("block_steps", C.c_int)]
 
 
+class RbvPtControl(C.Structure):
+    _fields_ = [("a", C.c_double), ("adapt", C.c_int), ("adaptation_lag", C.c_double),
+                ("adaptation_time", C.c_double), ("adapt_steps_done", C.c_ulonglong), ("n_record", C.c_int)]
+
+
 EXPORTS = {
     # name: (restype, argtypes)
     "rbv_create": (C.c_int, [C.c_int, C.POINTER(C.c_void_p)]),
@@ -89,6 +94,11 @@ EXPORTS = {
     "rbv_stretch_run_sightlines": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_double,
                                              C.c_ulonglong, C.c_ulonglong, C.c_void_p, C.c_void_p, C.c_void_p,
                                              C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "rbv_pt_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    "rbv_pt_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                             C.POINTER(RbvPtControl), C.c_ulonglong, C.c_ulonglong, C.c_void_p, C.c_void_p,
+                             C.POINTER(RbvChainSink), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                             C.c_size_t, C.c_int, C.c_void_p]),
     "rbv_slice_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_size_t)]),
     "rbv_slice_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(RbvSliceTuning),
                                 C.c_ulonglong, C.c_ulonglong, C.c_void_p, C.c_void_p, C.c_void_p,

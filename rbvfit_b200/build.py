@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(CSRC, "librbvfit_b200.so")
 SOURCES = ["rbv_kernels.cu"]
-HEADERS = ["rbv_device.cuh", "rbv_sampler.cuh", "rbv_slice.cuh", "rbv_stream.cuh", "rbv_grad.cuh", "rbv_fisher.cuh", "rbv_lm.cuh", "faddeeva_tables.h", os.path.join("..", "..", "include", "rbvfit_b200.h")]
+HEADERS = ["rbv_device.cuh", "rbv_sampler.cuh", "rbv_pt.cuh", "rbv_slice.cuh", "rbv_stream.cuh", "rbv_grad.cuh", "rbv_fisher.cuh", "rbv_lm.cuh", "faddeeva_tables.h", os.path.join("..", "..", "include", "rbvfit_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

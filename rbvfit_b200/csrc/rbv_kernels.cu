@@ -34,6 +34,7 @@
 #include "../../include/rbvfit_b200.h"
 #include "rbv_device.cuh"
 #include "rbv_sampler.cuh"   // StretchParams + Philox streams (embedded in LaunchParams for the fused sampler step)
+#include "rbv_pt.cuh"        // parallel tempering: swap stage and record (rbv_pt_run)
 #include "rbv_slice.cuh"     // device-resident ensemble slice sampler (kernels around the lnprob launch)
 
 namespace rbv {
@@ -2120,8 +2121,10 @@ int rbv_lnprob_batch_host(RbvContext* ctx, const double* theta_host, int W, doub
 
 // ------------------------------------------------------------------------------------------ device-resident sampler
 constexpr int kMaxRanks = 64;   // ranks of one communicator (rows of a half-step are padded to world x chunk)
+constexpr int kPtMaxTemps = 4096;   // temperatures of rbv_pt_run (one shared-memory counter each in the plan kernel)
 struct StretchLayout {
   size_t prop, lnp_prop, factors, walker_of, ctr, lnprob_ws, total;
+  size_t pt_tmp = 0, pt_src = 0;   // rbv_pt_run only: coordinates before the swap stage, slot map
 };
 static StretchLayout stretch_layout(const RbvContext* ctx, int W) {
   auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
@@ -2147,24 +2150,51 @@ int rbv_stretch_workspace_bytes(const RbvContext* ctx, int n_walkers, size_t* by
 static void rank_rows(int n, int rank, int world, int* lo, int* hi, int* chunk);
 static int allgather_rows(RbvContext* ctx, double* buf, int chunk, cudaStream_t st);
 
-// The run loop shared by rbv_stretch_run / rbv_stretch_run_dist / rbv_stretch_run_sink.  One step is captured in a
-// CUDA graph (the step index lives in device memory) and replayed.
+// The run loop shared by rbv_stretch_run / rbv_stretch_run_dist / rbv_stretch_run_sink / rbv_pt_run.  One step is
+// captured in a CUDA graph (the step index lives in device memory) and replayed.
 //   dist   rows of every half-step split over the ranks of the context's communicator, in-place NCCL all-gather of
 //          their lnprob inside the captured step (separate propose / accept kernels); otherwise the fused single-GPU
 //          step (proposal in the prep kernel, accept/reject in the finalisation)
 //   sink   chain hand-off to the host while the run goes on: P.chain / P.lnp_chain are device RINGS of
 //          2 x block_steps steps; after every block the finished half is copied to page-locked staging on a second
 //          stream and from there by this thread into the caller's arrays, while the device runs the next block
+//   pt     parallel tempering (rbv_pt.cuh): P holds T = P.S tempered ensembles; a half-step is the separate propose
+//          kernel, ONE lnprob launch over all T ensembles' rows and the accept kernel, then the swap stage records the
+//          step and advances the counter.  A recorded step is row_c chain and row_l lnprob doubles (the sink's ring)
 static int stretch_run_impl(RbvContext* ctx, StretchParams& P, const StretchLayout& lay, char* ws,
                             size_t workspace_bytes, int n_walkers, int n_steps, bool dist, const RbvChainSink* sink,
-                            int use_graph, cudaStream_t st, const char* who) {
+                            int use_graph, cudaStream_t st, const char* who, const PtParams* pt = nullptr) {
   RBV_CUDA(cudaMemsetAsync(ws + lay.ctr, 0, 256, st));
+  const size_t row_c = pt ? (size_t)pt->n_record * n_walkers * ctx->ndim : (size_t)n_walkers * ctx->ndim;
+  const size_t row_l = pt ? (size_t)pt->T * n_walkers : (size_t)n_walkers;
   const size_t lnprob_ws_bytes = workspace_bytes - lay.lnprob_ws;
   const int h = (n_walkers + 1) / 2;
   const int rank = (dist && ctx->comm) ? ctx->comm_rank : 0, world = (dist && ctx->comm) ? ctx->comm_world : 1;
   void* stream = (void*)st;
 
   auto one_step = [&]() -> int {
+    if (pt) {
+      for (int split = 0; split < 2; ++split) {
+        const int rows = P.S * (split == 0 ? h : n_walkers - h);
+        stretch_propose_kernel<<<(unsigned)((rows + 3) / 4), 128, 0, st>>>(P, split);
+        RBV_CUDA(cudaGetLastError());
+        ctx->launches++;
+        int rc = launch_lnprob(ctx, P.prop, rows, 0, P.lnp_prop, ws + lay.lnprob_ws, lnprob_ws_bytes, stream, who);
+        if (rc != RBV_OK) return rc;
+        stretch_accept_kernel<<<(unsigned)((rows + 3) / 4), 128, 0, st>>>(P, split);
+        RBV_CUDA(cudaGetLastError());
+        ctx->launches++;
+      }
+      const int slots = pt->T * n_walkers;
+      RBV_CUDA(cudaMemcpyAsync(pt->coords_tmp, pt->coords, (size_t)slots * ctx->ndim * sizeof(double),
+                               cudaMemcpyDeviceToDevice, st));
+      pt_swap_plan_kernel<<<1, kPtPlanThreads, (size_t)pt->T * sizeof(unsigned int), st>>>(*pt);
+      RBV_CUDA(cudaGetLastError());
+      pt_gather_record_kernel<<<(unsigned)((slots + 3) / 4), 128, 0, st>>>(*pt);
+      RBV_CUDA(cudaGetLastError());
+      ctx->launches += 2;
+      return RBV_OK;
+    }
     for (int split = 0; split < 2; ++split) {
       const int nS = split == 0 ? h : n_walkers - h;
       if (!dist) {
@@ -2202,8 +2232,8 @@ static int stretch_run_impl(RbvContext* ctx, StretchParams& P, const StretchLayo
   // ---- small ensembles: the whole loop as cooperative launches of voigt_mcmc_kernel (one per block of steps)
   LaunchPlan plan;
   bool persistent = false;
-  if (graph_ok && !dist && ctx->tune.mcmc_persistent != 0 && ctx->tune.stream != 1) {   // (STREAM=1: tests force the
-                                                                                         // stream kernel everywhere)
+  if (graph_ok && !dist && !pt && ctx->tune.mcmc_persistent != 0 && ctx->tune.stream != 1) {   // (STREAM=1: tests
+                                                                                       // force the stream kernel everywhere)
     int rc0 = launch_lnprob(ctx, P.prop, h, 0, P.lnp_prop, ws + lay.lnprob_ws, lnprob_ws_bytes, stream, who, &P, 0,
                             nullptr, 0, true, &plan);
     if (rc0 != RBV_OK) return rc0;
@@ -2282,7 +2312,6 @@ static int stretch_run_impl(RbvContext* ctx, StretchParams& P, const StretchLayo
     // ---- pipelined hand-off: block b runs on the device while block b - 1 travels device ring -> pinned staging
     // (copy stream) -> the caller's host arrays (this thread)
     const int K = sink->block_steps;
-    const size_t row_c = (size_t)n_walkers * ctx->ndim, row_l = (size_t)n_walkers;     // doubles per step
     const int n_blocks = (n_steps + K - 1) / K;
     auto steps_of = [&](int b) { return std::min(K, n_steps - b * K); };
     auto drain = [&](int b) -> cudaError_t {       // pinned half of block b -> host arrays
@@ -2323,6 +2352,18 @@ static int stretch_run_impl(RbvContext* ctx, StretchParams& P, const StretchLayo
   return RBV_OK;
 }
 
+// the copy stream and events of the chain sink (created on first use, owned by the context)
+static int sink_stream_setup(RbvContext* ctx) {
+  if (!ctx->sink_stream) {
+    RBV_CUDA(cudaStreamCreateWithFlags(&ctx->sink_stream, cudaStreamNonBlocking));
+    for (int k = 0; k < 2; ++k) {
+      RBV_CUDA(cudaEventCreateWithFlags(&ctx->sink_done[k], cudaEventDisableTiming));
+      RBV_CUDA(cudaEventCreateWithFlags(&ctx->sink_copied[k], cudaEventDisableTiming));
+    }
+  }
+  return RBV_OK;
+}
+
 static int stretch_run_entry(RbvContext* ctx, double* coords, double* lnprob, int n_walkers, int n_steps, double a,
                              unsigned long long seed, unsigned long long first_step, double* chain,
                              double* lnprob_chain, const RbvChainSink* sink, int* n_accepted, int* flag,
@@ -2354,13 +2395,8 @@ static int stretch_run_entry(RbvContext* ctx, double* coords, double* lnprob, in
     P.ring_steps = 2 * sink->block_steps;
     P.chain = sink->ring_dev;
     P.lnp_chain = sink->ring_dev + (size_t)P.ring_steps * n_walkers * ctx->ndim;
-    if (!ctx->sink_stream) {
-      RBV_CUDA(cudaStreamCreateWithFlags(&ctx->sink_stream, cudaStreamNonBlocking));
-      for (int k = 0; k < 2; ++k) {
-        RBV_CUDA(cudaEventCreateWithFlags(&ctx->sink_done[k], cudaEventDisableTiming));
-        RBV_CUDA(cudaEventCreateWithFlags(&ctx->sink_copied[k], cudaEventDisableTiming));
-      }
-    }
+    int rc = sink_stream_setup(ctx);
+    if (rc != RBV_OK) return rc;
   }
   P.n_accepted = n_accepted;
   P.flag = flag;
@@ -2400,6 +2436,117 @@ int rbv_stretch_run_sink(RbvContext* ctx, double* coords, double* lnprob, int n_
   return stretch_run_entry(ctx, coords, lnprob, n_walkers, n_steps, a, seed, first_step, nullptr, nullptr, sink,
                            n_accepted, flag, workspace, workspace_bytes, distributed != 0, 1, stream,
                            "rbv_stretch_run_sink");
+}
+
+// ---- parallel tempering (rbv_pt.cuh): T tempered stretch-move ensembles and ptemcee's swap stage --------------
+static StretchLayout pt_layout(const RbvContext* ctx, int T, int W) {
+  auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
+  const size_t rows = (size_t)((W + 1) / 2) * T, slots = (size_t)T * W, nd = std::max(ctx->ndim, 1);
+  StretchLayout lay;
+  lay.prop = 0;
+  lay.lnp_prop = up(rows * nd * sizeof(double));
+  lay.factors = lay.lnp_prop + up(rows * sizeof(double));
+  lay.walker_of = lay.factors + up(rows * sizeof(double));
+  lay.ctr = lay.walker_of + up(rows * sizeof(int));
+  lay.pt_tmp = lay.ctr + 256;
+  lay.pt_src = lay.pt_tmp + up(slots * nd * sizeof(double));
+  lay.lnprob_ws = lay.pt_src + up(slots * sizeof(int));
+  lay.total = lay.lnprob_ws + workspace_layout(ctx, (int)rows, false).total;
+  return lay;
+}
+
+static int pt_shape_ok(int T, int W) {
+  return T >= 1 && T <= kPtMaxTemps && W >= 2 && (long long)T * W <= 0x7fffffffLL;
+}
+
+int rbv_pt_workspace_bytes(const RbvContext* ctx, int n_temps, int n_walkers, size_t* bytes) {
+  if (!ctx || !bytes || !pt_shape_ok(n_temps, n_walkers)) return fail(RBV_EINVAL, "rbv_pt_workspace_bytes: bad argument");
+  *bytes = pt_layout(ctx, n_temps, n_walkers).total;
+  return RBV_OK;
+}
+
+int rbv_pt_run(RbvContext* ctx, double* coords, double* lnprob, double* betas, int n_temps, int n_walkers,
+               int n_steps, const RbvPtControl* control, unsigned long long seed, unsigned long long first_step,
+               double* chain, double* lnprob_chain, const RbvChainSink* sink, double* beta_history, int* n_accepted,
+               unsigned long long* n_swaps_accepted, int* flag, void* workspace, size_t workspace_bytes,
+               int use_graph, void* stream) {
+  const char* who = "rbv_pt_run";
+  const int T = n_temps, W = n_walkers;
+  if (!ctx || !coords || !lnprob || !betas || !control || !n_accepted || !flag || (T > 1 && !n_swaps_accepted))
+    return fail(RBV_EINVAL, "rbv_pt_run: null argument");
+  if (!pt_shape_ok(T, W))
+    return fail(RBV_EINVAL, "rbv_pt_run: need 1 <= n_temps <= 4096, n_walkers >= 2 and n_temps * n_walkers in int range");
+  if (n_steps < 0 || !(control->a > 1.0)) return fail(RBV_EINVAL, "rbv_pt_run: n_steps < 0 or stretch scale a <= 1");
+  if (control->n_record < 1 || control->n_record > T) return fail(RBV_EINVAL, "rbv_pt_run: n_record outside 1 .. n_temps");
+  if (control->adapt && !(control->adaptation_lag > 0.0 && control->adaptation_time > 0.0))
+    return fail(RBV_EINVAL, "rbv_pt_run: adaptation_lag and adaptation_time must be > 0");
+  if (sink && (chain || lnprob_chain)) return fail(RBV_EINVAL, "rbv_pt_run: pass device chains or a sink, not both");
+  if (sink && (sink->block_steps < 1 || !sink->ring_dev || !sink->ring_pinned))
+    return fail(RBV_EINVAL, "rbv_pt_run: incomplete chain sink");
+  if (ctx->inst.empty() || ctx->ndim == 0) return fail(RBV_ESTATE, "rbv_pt_run: context not set up");
+  const StretchLayout lay = pt_layout(ctx, T, W);
+  if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, "rbv_pt_run: workspace too small");
+  RBV_ON_DEVICE(ctx);
+  cudaStream_t st = (cudaStream_t)stream;
+  std::vector<double> b((size_t)T);      // the ladder is checked on the host: a 8 T-byte copy before the run
+  RBV_CUDA(cudaMemcpyAsync(b.data(), betas, (size_t)T * sizeof(double), cudaMemcpyDeviceToHost, st));
+  RBV_CUDA(cudaStreamSynchronize(st));
+  if (b[0] != 1.0) return fail(RBV_EINVAL, "rbv_pt_run: betas[0] must be 1");
+  for (int t = 1; t < T; ++t)
+    if (!(b[t] < b[t - 1]) || !(b[t] >= 0.0))
+      return fail(RBV_EINVAL, "rbv_pt_run: betas must be strictly decreasing and >= 0");
+  if (n_steps == 0) return RBV_OK;
+  char* ws = (char*)workspace;
+  StretchParams P;
+  memset(&P, 0, sizeof(P));
+  P.coords = coords;
+  P.lnp = lnprob;
+  P.prop = (double*)(ws + lay.prop);
+  P.lnp_prop = (double*)(ws + lay.lnp_prop);
+  P.factors = (double*)(ws + lay.factors);
+  P.walker_of = (int*)(ws + lay.walker_of);
+  P.n_accepted = n_accepted;
+  P.flag = flag;
+  P.step_ctr = (unsigned long long*)(ws + lay.ctr);
+  P.ticket = nullptr;            // the accept kernels neither record nor advance the step: the swap stage does
+  P.first_step = first_step;
+  P.seed = seed;
+  P.a = control->a;
+  P.W = W;
+  P.ndim = ctx->ndim;
+  P.S = T;
+  P.beta = betas;
+  PtParams Q;
+  memset(&Q, 0, sizeof(Q));
+  Q.coords = coords;
+  Q.lnp = lnprob;
+  Q.betas = betas;
+  Q.coords_tmp = (double*)(ws + lay.pt_tmp);
+  Q.src = (int*)(ws + lay.pt_src);
+  Q.n_swaps = n_swaps_accepted;
+  Q.chain = chain;
+  Q.lnp_chain = lnprob_chain;
+  Q.beta_history = beta_history;
+  Q.step_ctr = P.step_ctr;
+  Q.ticket = (unsigned int*)(ws + lay.ctr + 64);
+  Q.first_step = first_step;
+  Q.seed = seed;
+  Q.adapt_t0 = control->adapt_steps_done;
+  Q.adapt_lag = control->adaptation_lag;
+  Q.adapt_time = control->adaptation_time;
+  Q.adapt = control->adapt != 0;
+  Q.T = T;
+  Q.W = W;
+  Q.ndim = ctx->ndim;
+  Q.n_record = control->n_record;
+  if (sink) {
+    Q.ring_steps = 2 * sink->block_steps;
+    Q.chain = sink->ring_dev;
+    Q.lnp_chain = sink->ring_dev + (size_t)Q.ring_steps * Q.n_record * W * ctx->ndim;
+    int rc = sink_stream_setup(ctx);
+    if (rc != RBV_OK) return rc;
+  }
+  return stretch_run_impl(ctx, P, lay, ws, workspace_bytes, W, n_steps, false, sink, use_graph, st, who, &Q);
 }
 
 // ---- multi-GPU form of the sampler: half-step = propose_eval | caller's all-gather of lnprob | accept ----------

@@ -47,6 +47,8 @@ struct StretchParams {
                          // sightline, rbv_stretch_run_sightlines); 1 everywhere else.  Ensemble e owns walkers
                          // e W .. e W + W - 1 of coords / lnp / n_accepted and rows e n_S .. of the half-step buffers;
                          // its random streams are those of a single ensemble with the walker counter offset by e W
+  const double* beta;    // [S] or NULL: ensemble e accepts against prior x L^beta[e] (parallel tempering, rbv_pt.cuh;
+                         // lnp stays the untempered lnprob).  NULL: the untempered test of every other path
 };
 
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
@@ -79,10 +81,8 @@ __device__ __forceinline__ uint4 stretch_rand(const StretchParams& P, unsigned l
   return sampler_rand(P.seed, step, walker, purpose);
 }
 
-// the step's affine permutation of walker positions: walker(pos) = (a pos + b) mod W
-__device__ __forceinline__ void sampler_perm(unsigned long long seed, int n_walkers, unsigned long long step,
-                                             uint32_t& a, uint32_t& b) {
-  const uint4 r = sampler_rand(seed, step, 0xffffffffu, 0u);
+// an affine permutation of W positions from one random draw r: pos -> (a pos + b) mod W, a advanced until gcd(a, W) = 1
+__device__ __forceinline__ void affine_perm(uint4 r, int n_walkers, uint32_t& a, uint32_t& b) {
   const uint32_t W = (uint32_t)n_walkers;
   a = r.x % W;
   b = r.y % W;
@@ -96,6 +96,12 @@ __device__ __forceinline__ void sampler_perm(unsigned long long seed, int n_walk
     if (x == 1u || W == 1u) break;
     a = (a + 1u) % W;
   }
+}
+
+// the step's affine permutation of walker positions: walker(pos) = (a pos + b) mod W
+__device__ __forceinline__ void sampler_perm(unsigned long long seed, int n_walkers, unsigned long long step,
+                                             uint32_t& a, uint32_t& b) {
+  affine_perm(sampler_rand(seed, step, 0xffffffffu, 0u), n_walkers, a, b);
 }
 
 __device__ __forceinline__ void stretch_perm(const StretchParams& P, unsigned long long step, uint32_t& a, uint32_t& b) {
@@ -113,6 +119,15 @@ __device__ __forceinline__ void split_geometry(int W, int split, int& offS, int&
   else            { offS = h; nS = W - h; offC = 0; nC = h; }
 }
 
+// The tempered accept test of parallel tempering, case by case on the untempered lnprob values: beta (new - old)
+// would be 0 x (-inf) = NaN at beta = 0, and a walker that starts outside the bounds would never move.  Explicitly
+// rounded operations: the numpy replay evaluates the same expression.
+__device__ __forceinline__ bool tempered_accept(double beta, double factor, double new_lp, double old_lp, double lnu) {
+  if (!(new_lp > -INFINITY)) return false;                  // -inf (or NaN) proposal: always rejected
+  if (old_lp == -INFINITY) return true;
+  return lnu < __dsub_rn(__dadd_rn(factor, __dmul_rn(beta, new_lp)), __dmul_rn(beta, old_lp));
+}
+
 // Accept / reject for row k of the active half once its lnprob is known, by the WARP that finalised it (last CTA of
 // the walker in the tile kernel, or finalize_kernel).  Every lane takes the same decision; the lanes copy the
 // parameter columns in parallel (a single thread would pay one L2 round trip per column: proposal -> walker ->
@@ -126,8 +141,13 @@ __device__ __forceinline__ void stretch_accept_record(const StretchParams& P, in
   const int i = e * P.W + P.walker_of[k];              // k: row of the half-step buffers, i: global walker
   const uint4 r = stretch_rand(P, step, (uint32_t)i, 3u + (uint32_t)split);
   const double old_lp = P.lnp[i];
-  const double lnpdiff = P.factors[k] + new_lp - old_lp;
-  const bool accept = log(u01(r.x, r.y)) < lnpdiff;
+  bool accept;
+  if (!P.beta) {
+    const double lnpdiff = P.factors[k] + new_lp - old_lp;
+    accept = log(u01(r.x, r.y)) < lnpdiff;
+  } else {
+    accept = tempered_accept(P.beta[e], P.factors[k], new_lp, old_lp, log(u01(r.x, r.y)));
+  }
   const double* __restrict__ src = accept ? P.prop + (size_t)k * P.ndim : P.coords + (size_t)i * P.ndim;
   double* __restrict__ x = P.coords + (size_t)i * P.ndim;
   const unsigned long long srow = P.ring_steps ? s % (unsigned long long)P.ring_steps : s;   // row of the chain buffers
@@ -145,7 +165,7 @@ __device__ __forceinline__ void stretch_accept_record(const StretchParams& P, in
       P.n_accepted[i] += 1;
     }
     if (P.lnp_chain) P.lnp_chain[srow * P.S * P.W + i] = accept ? new_lp : old_lp;
-    if (!P.step_ctr) return;                                 // host-driven steps: no device counters
+    if (!P.ticket) return;        // host-driven steps, or the step ends later (parallel tempering's swap stage)
     __threadfence();
     if (atomicAdd(P.ticket, 1u) == (unsigned)nS - 1u) {      // last walker of this half-step
       *P.ticket = 0u;

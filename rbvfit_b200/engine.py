@@ -12,7 +12,7 @@ from typing import List, Optional
 import numpy as np
 
 from . import _lib
-from ._lib import RbvChainSink, RbvError, RbvLineTable, RbvSpectrum, check
+from ._lib import RbvChainSink, RbvError, RbvLineTable, RbvPtControl, RbvSpectrum, check
 
 VOIGT_METHODS = {"wofz": 0, "fast": 1}
 
@@ -684,6 +684,79 @@ class Engine:
             lnp_chain_t.data_ptr() if lnp_chain_t is not None else None,
             n_accepted_t.data_ptr(), flag_t.data_ptr(), self._stretch_ws.data_ptr(), self._stretch_ws.numel(),
             self._stream()), "rbv_stretch_run_sightlines")
+
+    def _pt_checks(self, coords_t, lnp_t, betas_t, n_steps, beta_hist_t, n_accepted_t, n_swaps_t, flag_t):
+        torch = _torch()
+        if coords_t.dim() != 3:
+            raise ValueError("coords must be [n_temps, n_walkers, ndim]")
+        T, W, ndim = coords_t.shape
+        if ndim != self.ndim:
+            raise ValueError(f"coords has {ndim} columns, bounds were set for ndim={self.ndim}")
+        self._dev_tensor(coords_t, torch.float64, "coords")
+        self._dev_tensor(lnp_t, torch.float64, "lnprob", (T, W))
+        self._dev_tensor(betas_t, torch.float64, "betas", (T,))
+        self._dev_tensor(beta_hist_t, torch.float64, "beta history", (int(n_steps), T))
+        self._dev_tensor(n_accepted_t, torch.int32, "n_accepted", (T, W))
+        self._dev_tensor(n_swaps_t, torch.int64, "n_swaps_accepted", (max(T - 1, 1),))
+        self._dev_tensor(flag_t, torch.int32, "flag")
+        nbytes = C.c_size_t(0)
+        check(self.lib.rbv_pt_workspace_bytes(self._h, T, W, C.byref(nbytes)), "rbv_pt_workspace_bytes")
+        if self._stretch_ws is None or self._stretch_ws.numel() < nbytes.value:
+            self._stretch_ws = torch.empty(int(nbytes.value), dtype=torch.uint8, device=self.tdev)
+        return T, W, ndim
+
+    def _pt_call(self, coords_t, lnp_t, betas_t, T, W, n_steps, a, seed, first_step, chain_p, lnp_chain_p, sink,
+                 beta_hist_t, n_accepted_t, n_swaps_t, flag_t, use_graph, adapt, adaptation_lag, adaptation_time,
+                 adapt_steps_done, n_record):
+        ctl = RbvPtControl(float(a), int(bool(adapt)), float(adaptation_lag), float(adaptation_time),
+                           int(adapt_steps_done), int(n_record))
+        check(self.lib.rbv_pt_run(
+            self._h, coords_t.data_ptr(), lnp_t.data_ptr(), betas_t.data_ptr(), T, W, int(n_steps), C.byref(ctl),
+            int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_step), chain_p, lnp_chain_p, sink,
+            beta_hist_t.data_ptr() if beta_hist_t is not None else None, n_accepted_t.data_ptr(),
+            n_swaps_t.data_ptr(), flag_t.data_ptr(), self._stretch_ws.data_ptr(), self._stretch_ws.numel(),
+            int(bool(use_graph)), self._stream()), "rbv_pt_run")
+
+    def pt_run(self, coords_t, lnp_t, betas_t, n_steps: int, a: float, seed: int, first_step: int, chain_t,
+               lnp_chain_t, beta_hist_t, n_accepted_t, n_swaps_t, flag_t, use_graph: bool = True, adapt: bool = False,
+               adaptation_lag: float = 10000.0, adaptation_time: float = 100.0, adapt_steps_done: int = 0,
+               n_record: int = 1):
+        """Parallel tempering on the device (rbv_pt_run): ``coords_t`` [T, W, ndim], ``lnp_t`` [T, W] (untempered),
+        ``betas_t`` [T] (in/out); ``chain_t`` [n_steps, n_record, W, ndim], ``lnp_chain_t`` [n_steps, T, W] and
+        ``beta_hist_t`` [n_steps, T] may be None; ``n_swaps_t`` int64 [max(T - 1, 1)] (the library's uint64
+        counters).  Every tensor stays on the device; runs on the current torch stream."""
+        torch = _torch()
+        T, W, ndim = self._pt_checks(coords_t, lnp_t, betas_t, n_steps, beta_hist_t, n_accepted_t, n_swaps_t, flag_t)
+        self._dev_tensor(chain_t, torch.float64, "chain", (int(n_steps), int(n_record), W, ndim))
+        self._dev_tensor(lnp_chain_t, torch.float64, "lnprob chain", (int(n_steps), T, W))
+        self._pt_call(coords_t, lnp_t, betas_t, T, W, n_steps, a, seed, first_step,
+                      chain_t.data_ptr() if chain_t is not None else None,
+                      lnp_chain_t.data_ptr() if lnp_chain_t is not None else None, None, beta_hist_t, n_accepted_t,
+                      n_swaps_t, flag_t, use_graph, adapt, adaptation_lag, adaptation_time, adapt_steps_done,
+                      n_record)
+
+    def pt_run_to_host(self, coords_t, lnp_t, betas_t, n_steps: int, a: float, seed: int, first_step: int,
+                       beta_hist_t, n_accepted_t, n_swaps_t, flag_t, adapt: bool = False,
+                       adaptation_lag: float = 10000.0, adaptation_time: float = 100.0, adapt_steps_done: int = 0,
+                       n_record: int = 1):
+        """``pt_run`` with the chain delivered to the HOST while the run goes on (the chain sink of
+        ``stretch_run_to_host``): returns (chain [n_steps, n_record, W, ndim], lnprob chain [n_steps, T, W])."""
+        torch = _torch()
+        T, W, ndim = self._pt_checks(coords_t, lnp_t, betas_t, n_steps, beta_hist_t, n_accepted_t, n_swaps_t, flag_t)
+        row = int(n_record) * W * ndim + T * W
+        K = int(min(256, max(1, (6 << 20) // (row * 8)), max(1, (int(n_steps) + 1) // 2)))   # ~6 MB blocks
+        need = 2 * K * row
+        if self._sink_ring is None or self._sink_ring[0] != K or self._sink_ring[1].numel() < need:
+            self._sink_ring = (K, torch.empty(need, dtype=torch.float64, device=self.tdev),
+                               torch.empty(need, dtype=torch.float64, pin_memory=True))
+        _k, ring_dev, ring_pin = self._sink_ring
+        chain = np.empty((int(n_steps), int(n_record), W, ndim), dtype=np.float64)
+        lps = np.empty((int(n_steps), T, W), dtype=np.float64)
+        sink = RbvChainSink(chain.ctypes.data, lps.ctypes.data, ring_dev.data_ptr(), ring_pin.data_ptr(), K)
+        self._pt_call(coords_t, lnp_t, betas_t, T, W, n_steps, a, seed, first_step, None, None, C.byref(sink),
+                      beta_hist_t, n_accepted_t, n_swaps_t, flag_t, True, adapt, adaptation_lag, adaptation_time,
+                      adapt_steps_done, n_record)
+        return chain, lps
 
     def slice_run(self, coords_t, lnp_t, n_steps: int, tuning, seed: int, first_step: int, chain_t, lnp_chain_t,
                   flag_t, use_graph: bool = True) -> np.ndarray:

@@ -39,7 +39,7 @@ def gelman_rubin(chains) -> np.ndarray:
 class vfit:
     def __init__(self, instrument_data: Dict, theta, lb, ub, no_of_Chain=50, no_of_steps=1000,
                  perturbation=1e-4, sampler="emcee", skip_initial_state_check=False, device=None, seed=None,
-                 device_sampler=True):
+                 device_sampler=True, betas=None):
         self._validate_unified_instrument_data(instrument_data)
         self._validate_guesses(theta, lb, ub)
         self.theta = np.asarray(theta)
@@ -54,8 +54,12 @@ class vfit:
         self.perturbation = perturbation
         self.skip_initial_state_check = skip_initial_state_check
         self.sampler_name = sampler.lower()
-        if self.sampler_name not in ["emcee", "zeus"]:
-            raise ValueError(f"Unknown sampler '{sampler}'. Use 'emcee' or 'zeus'.")
+        if self.sampler_name not in ["emcee", "zeus", "pt"]:
+            raise ValueError(f"Unknown sampler '{sampler}'. Use 'emcee', 'zeus' or 'pt'.")
+        if self.sampler_name == "pt" and not device_sampler:
+            raise ValueError("sampler='pt' (parallel tempering) runs on the device only")
+        self.betas = betas                 # sampler='pt': the temperature ladder (None: default_betas(ndim))
+        self.pt_sampler = None             # sampler='pt': the DeviceParallelTemperingSampler (fitter.sampler = its cold view)
         self.mcmc_flag = False
         self.sampler = None
         self.best_theta = None
@@ -282,7 +286,12 @@ class vfit:
             if verbose:
                 print("✓ Starting guess optimized")
         guesses = self._initialize_walkers(self.theta)
-        if self.sampler_name == "zeus":
+        if self.sampler_name == "pt":
+            from .pt_sampler import DeviceParallelTemperingSampler
+            sampler = DeviceParallelTemperingSampler(self.nwalkers, self.ndim, self._like, betas=self.betas,
+                                                     seed=self._seed)
+            guesses = np.stack([guesses] + [self._initialize_walkers(self.theta) for _ in range(sampler.ntemps - 1)])
+        elif self.sampler_name == "zeus":
             from .slice_sampler import DeviceEnsembleSliceSampler, EnsembleSliceSampler
             if self.device_sampler:
                 sampler = DeviceEnsembleSliceSampler(self.nwalkers, self.ndim, self._like, seed=self._seed)
@@ -298,13 +307,15 @@ class vfit:
             print(f"   Steps: {self.no_of_steps}")
             print(f"   Instruments: {len(self.instrument_data)}")
         try:
-            if self.sampler_name == "emcee":
+            if self.sampler_name in ("emcee", "pt"):
                 sampler.run_mcmc(guesses, self.no_of_steps, progress=progress,
                                  skip_initial_state_check=self.skip_initial_state_check)
             else:
                 sampler.run_mcmc(guesses, self.no_of_steps, progress=progress)
         except Exception as e:
             raise RuntimeError(f"MCMC sampling failed: {e}")
+        if self.sampler_name == "pt":
+            self.pt_sampler, sampler = sampler, sampler.cold()
         self.sampler = sampler
         self.mcmc_flag = True
         self.samples = None
@@ -346,7 +357,15 @@ class vfit:
                 print("✅ Good acceptance fraction (0.2-0.7)")
         except Exception:
             print("Acceptance fraction not available")
-        if self.sampler_name == "emcee":
+        if self.sampler_name == "pt":
+            try:
+                print("Swap acceptance (coldest pair first): "
+                      + " ".join(f"{x:.2f}" for x in self.pt_sampler.tswap_acceptance_fraction))
+                lnz, dlnz = self.log_evidence()
+                print(f"ln Z (thermodynamic integration, second half of the chain): {lnz:.3f} +- {dlnz:.3f}")
+            except Exception:
+                print("Evidence not available")
+        if self.sampler_name in ("emcee", "pt"):
             try:
                 tau = np.nanmean(self.sampler.get_autocorr_time())
                 print(f"Mean auto-correlation time: {tau:.3f} steps")
@@ -397,6 +416,16 @@ class vfit:
         if instrument_name is None and len(names) > 1:
             results["combined"] = total_chi2 / max(total_n - len(theta), 1)
         return results
+
+    def log_evidence(self, burn_in=0.5):
+        """sampler='pt': (ln Z, d ln Z) by thermodynamic integration over the steps after the first ``burn_in``
+        fraction (``DeviceParallelTemperingSampler.log_evidence_estimate``); Z is normalised to the box prior of the
+        bounds, so two line sets fitted to the same data compare by ln Z."""
+        if not self.mcmc_flag:
+            raise RuntimeError("MCMC has not been run")
+        if self.pt_sampler is None:
+            raise RuntimeError("the evidence needs sampler='pt' (parallel tempering)")
+        return self.pt_sampler.log_evidence_estimate(discard=int(burn_in * self.no_of_steps))
 
     def get_samples(self, flat=True, burn_in=0.5):
         if not self.mcmc_flag:
