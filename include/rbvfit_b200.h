@@ -311,6 +311,36 @@ int rbv_pt_run(RbvContext* ctx, double* coords, double* lnprob, double* betas, i
                unsigned long long* n_swaps_accepted, int* flag, void* workspace, size_t workspace_bytes,
                int use_graph, void* stream);
 
+/* Survey-mode parallel tempering: rbv_pt_run for every sightline of a sightline context (one spectrum per
+ * instrument, as rbv_stretch_run_sightlines), all S sightlines advancing in lockstep in one device loop, and
+ * optionally the moments of ln L that thermodynamic integration needs, accumulated on the device.  Ensemble
+ * e = s T + t (sightline-major).  A half-step is ONE sightline-mode lnprob launch over the S T ceil(W/2) proposal
+ * rows; the swap stage runs one CTA per sightline and stays two kernels and one copy per step whatever S and T are.
+ * Random streams: those of a one-sightline rbv_pt_run with every walker counter offset by s T W, so sightline 0
+ * reproduces rbv_pt_run on that sightline alone and T = 1 reproduces rbv_stretch_run_sightlines, bit for bit.
+ *   coords        DEVICE [S, T, W, ndim], updated in place;  lnprob DEVICE [S, T, W] (untempered), updated in place
+ *   betas         DEVICE [S, T], in/out: one ladder per sightline (each as in rbv_pt_run; a bad ladder is refused
+ *                 with the sightline named); adapted in place, per sightline, when control->adapt is set
+ *   control       HOST, see RbvPtControl
+ *   chain         DEVICE [n_steps, S, n_record, W, ndim] or NULL;  lnprob_chain DEVICE [n_steps, S, T, W] or NULL
+ *   sink          HOST or NULL: as in rbv_pt_run with a step of S * n_record * W * ndim chain doubles and, when
+ *                 sink->lnprob_chain_host is not NULL, S * T * W lnprob doubles; with lnprob_chain_host NULL no lnprob
+ *                 row is recorded or copied and the ring holds chain rows only
+ *   beta_history  DEVICE [n_steps, S, T] or NULL
+ *   ti_moments    DEVICE [S, T, 3] or NULL, in/out, accumulated across calls: (n, mean, M2) of the post-swap lnprob
+ *                 of every temperature of every step (Chan's merge, see rbv_pt.cuh; Var = M2 / n); NULL: nothing is
+ *                 accumulated.  Refused with control->adapt (adaptation breaks detailed balance)
+ *   n_accepted    DEVICE int[S, T, W];  n_swaps_accepted DEVICE uint64[S, T - 1] (NULL allowed for T = 1)
+ *   flag, workspace (rbv_pt_workspace_bytes_sightlines), use_graph, stream  as in rbv_pt_run.
+ * RBV_EINVAL also when S * T * W is outside int range. */
+int rbv_pt_workspace_bytes_sightlines(const RbvContext* ctx, int n_temps, int walkers_per_sightline, size_t* bytes);
+int rbv_pt_run_sightlines(RbvContext* ctx, double* coords, double* lnprob, double* betas, int n_temps,
+                          int walkers_per_sightline, int n_steps, const RbvPtControl* control,
+                          unsigned long long seed, unsigned long long first_step, double* chain,
+                          double* lnprob_chain, const RbvChainSink* sink, double* beta_history,
+                          double* ti_moments, int* n_accepted, unsigned long long* n_swaps_accepted, int* flag,
+                          void* workspace, size_t workspace_bytes, int use_graph, void* stream);
+
 /* Device-resident ensemble slice sampler (differential move).  Replaces the sampling loop
  * zeus.EnsembleSampler(nwalkers, ndim, self.lnprob).run_mcmc(guesses, no_of_steps), vfit_mcmc.py:425-440, 536-540
  * (zeus-mcmc >= 2.3.0 is not vendored in the reference; Karamanis & Beutler 2021, Algorithms 2-3 with zeus's defaults,

@@ -99,6 +99,11 @@ EXPORTS = {
                              C.POINTER(RbvPtControl), C.c_ulonglong, C.c_ulonglong, C.c_void_p, C.c_void_p,
                              C.POINTER(RbvChainSink), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                              C.c_size_t, C.c_int, C.c_void_p]),
+    "rbv_pt_workspace_bytes_sightlines": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_size_t)]),
+    "rbv_pt_run_sightlines": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                        C.POINTER(RbvPtControl), C.c_ulonglong, C.c_ulonglong, C.c_void_p,
+                                        C.c_void_p, C.POINTER(RbvChainSink), C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]),
     "rbv_slice_workspace_bytes": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_size_t)]),
     "rbv_slice_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(RbvSliceTuning),
                                 C.c_ulonglong, C.c_ulonglong, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -2158,15 +2158,17 @@ static int allgather_rows(RbvContext* ctx, double* buf, int chunk, cudaStream_t 
 //   sink   chain hand-off to the host while the run goes on: P.chain / P.lnp_chain are device RINGS of
 //          2 x block_steps steps; after every block the finished half is copied to page-locked staging on a second
 //          stream and from there by this thread into the caller's arrays, while the device runs the next block
-//   pt     parallel tempering (rbv_pt.cuh): P holds T = P.S tempered ensembles; a half-step is the separate propose
-//          kernel, ONE lnprob launch over all T ensembles' rows and the accept kernel, then the swap stage records the
-//          step and advances the counter.  A recorded step is row_c chain and row_l lnprob doubles (the sink's ring)
+//   pt     parallel tempering (rbv_pt.cuh): P holds the S T = P.S tempered ensembles of S sightlines (S = 1: one
+//          joint context); a half-step is the separate propose kernel, ONE lnprob launch over all ensembles' rows (in
+//          sightline mode with T n_S rows per sightline when pt->survey) and the accept kernel, then the swap stage
+//          records the step and advances the counter.  A recorded step is row_c chain and row_l lnprob doubles (the
+//          sink's ring; row_l = 0 when no lnprob chain is recorded)
 static int stretch_run_impl(RbvContext* ctx, StretchParams& P, const StretchLayout& lay, char* ws,
                             size_t workspace_bytes, int n_walkers, int n_steps, bool dist, const RbvChainSink* sink,
                             int use_graph, cudaStream_t st, const char* who, const PtParams* pt = nullptr) {
   RBV_CUDA(cudaMemsetAsync(ws + lay.ctr, 0, 256, st));
-  const size_t row_c = pt ? (size_t)pt->n_record * n_walkers * ctx->ndim : (size_t)n_walkers * ctx->ndim;
-  const size_t row_l = pt ? (size_t)pt->T * n_walkers : (size_t)n_walkers;
+  const size_t row_c = pt ? (size_t)pt->S * pt->n_record * n_walkers * ctx->ndim : (size_t)n_walkers * ctx->ndim;
+  const size_t row_l = pt ? (pt->lnp_chain ? (size_t)pt->S * pt->T * n_walkers : 0) : (size_t)n_walkers;
   const size_t lnprob_ws_bytes = workspace_bytes - lay.lnprob_ws;
   const int h = (n_walkers + 1) / 2;
   const int rank = (dist && ctx->comm) ? ctx->comm_rank : 0, world = (dist && ctx->comm) ? ctx->comm_world : 1;
@@ -2175,20 +2177,21 @@ static int stretch_run_impl(RbvContext* ctx, StretchParams& P, const StretchLayo
   auto one_step = [&]() -> int {
     if (pt) {
       for (int split = 0; split < 2; ++split) {
-        const int rows = P.S * (split == 0 ? h : n_walkers - h);
+        const int nS = split == 0 ? h : n_walkers - h, rows = P.S * nS;
         stretch_propose_kernel<<<(unsigned)((rows + 3) / 4), 128, 0, st>>>(P, split);
         RBV_CUDA(cudaGetLastError());
         ctx->launches++;
-        int rc = launch_lnprob(ctx, P.prop, rows, 0, P.lnp_prop, ws + lay.lnprob_ws, lnprob_ws_bytes, stream, who);
+        int rc = launch_lnprob(ctx, P.prop, rows, pt->survey ? pt->T * nS : 0, P.lnp_prop, ws + lay.lnprob_ws,
+                               lnprob_ws_bytes, stream, who);
         if (rc != RBV_OK) return rc;
         stretch_accept_kernel<<<(unsigned)((rows + 3) / 4), 128, 0, st>>>(P, split);
         RBV_CUDA(cudaGetLastError());
         ctx->launches++;
       }
-      const int slots = pt->T * n_walkers;
+      const int slots = pt->S * pt->T * n_walkers;
       RBV_CUDA(cudaMemcpyAsync(pt->coords_tmp, pt->coords, (size_t)slots * ctx->ndim * sizeof(double),
                                cudaMemcpyDeviceToDevice, st));
-      pt_swap_plan_kernel<<<1, kPtPlanThreads, (size_t)pt->T * sizeof(unsigned int), st>>>(*pt);
+      pt_swap_plan_kernel<<<(unsigned)pt->S, kPtPlanThreads, (size_t)pt->T * sizeof(unsigned int), st>>>(*pt);
       RBV_CUDA(cudaGetLastError());
       pt_gather_record_kernel<<<(unsigned)((slots + 3) / 4), 128, 0, st>>>(*pt);
       RBV_CUDA(cudaGetLastError());
@@ -2439,9 +2442,10 @@ int rbv_stretch_run_sink(RbvContext* ctx, double* coords, double* lnprob, int n_
 }
 
 // ---- parallel tempering (rbv_pt.cuh): T tempered stretch-move ensembles and ptemcee's swap stage --------------
-static StretchLayout pt_layout(const RbvContext* ctx, int T, int W) {
+// S sightlines of T temperatures (survey mode), or S = 1 and one joint context (rbv_pt_run)
+static StretchLayout pt_layout(const RbvContext* ctx, int S, int T, int W, bool survey) {
   auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-  const size_t rows = (size_t)((W + 1) / 2) * T, slots = (size_t)T * W, nd = std::max(ctx->ndim, 1);
+  const size_t rows = (size_t)((W + 1) / 2) * T * S, slots = (size_t)S * T * W, nd = std::max(ctx->ndim, 1);
   StretchLayout lay;
   lay.prop = 0;
   lay.lnp_prop = up(rows * nd * sizeof(double));
@@ -2451,7 +2455,7 @@ static StretchLayout pt_layout(const RbvContext* ctx, int T, int W) {
   lay.pt_tmp = lay.ctr + 256;
   lay.pt_src = lay.pt_tmp + up(slots * nd * sizeof(double));
   lay.lnprob_ws = lay.pt_src + up(slots * sizeof(int));
-  lay.total = lay.lnprob_ws + workspace_layout(ctx, (int)rows, false).total;
+  lay.total = lay.lnprob_ws + workspace_layout(ctx, (int)rows, survey).total;
   return lay;
 }
 
@@ -2459,42 +2463,58 @@ static int pt_shape_ok(int T, int W) {
   return T >= 1 && T <= kPtMaxTemps && W >= 2 && (long long)T * W <= 0x7fffffffLL;
 }
 
+// S T W slots and S T ceil(W / 2) half-step rows in int range
+static int pt_sightlines_shape_ok(long long S, int T, int W) {
+  return S >= 1 && pt_shape_ok(T, W) && S * T * W <= 0x7fffffffLL;
+}
+
 int rbv_pt_workspace_bytes(const RbvContext* ctx, int n_temps, int n_walkers, size_t* bytes) {
   if (!ctx || !bytes || !pt_shape_ok(n_temps, n_walkers)) return fail(RBV_EINVAL, "rbv_pt_workspace_bytes: bad argument");
-  *bytes = pt_layout(ctx, n_temps, n_walkers).total;
+  *bytes = pt_layout(ctx, 1, n_temps, n_walkers, false).total;
   return RBV_OK;
 }
 
-int rbv_pt_run(RbvContext* ctx, double* coords, double* lnprob, double* betas, int n_temps, int n_walkers,
-               int n_steps, const RbvPtControl* control, unsigned long long seed, unsigned long long first_step,
-               double* chain, double* lnprob_chain, const RbvChainSink* sink, double* beta_history, int* n_accepted,
-               unsigned long long* n_swaps_accepted, int* flag, void* workspace, size_t workspace_bytes,
-               int use_graph, void* stream) {
-  const char* who = "rbv_pt_run";
-  const int T = n_temps, W = n_walkers;
-  if (!ctx || !coords || !lnprob || !betas || !control || !n_accepted || !flag || (T > 1 && !n_swaps_accepted))
-    return fail(RBV_EINVAL, "rbv_pt_run: null argument");
-  if (!pt_shape_ok(T, W))
-    return fail(RBV_EINVAL, "rbv_pt_run: need 1 <= n_temps <= 4096, n_walkers >= 2 and n_temps * n_walkers in int range");
-  if (n_steps < 0 || !(control->a > 1.0)) return fail(RBV_EINVAL, "rbv_pt_run: n_steps < 0 or stretch scale a <= 1");
-  if (control->n_record < 1 || control->n_record > T) return fail(RBV_EINVAL, "rbv_pt_run: n_record outside 1 .. n_temps");
+int rbv_pt_workspace_bytes_sightlines(const RbvContext* ctx, int n_temps, int walkers_per_sightline, size_t* bytes) {
+  if (!ctx || !bytes || ctx->inst.empty() ||
+      !pt_sightlines_shape_ok((long long)ctx->inst.size(), n_temps, walkers_per_sightline))
+    return fail(RBV_EINVAL, "rbv_pt_workspace_bytes_sightlines: bad argument");
+  *bytes = pt_layout(ctx, (int)ctx->inst.size(), n_temps, walkers_per_sightline, true).total;
+  return RBV_OK;
+}
+
+// The two entry points: S = 1 and a joint context (rbv_pt_run), or one sightline per instrument of the context
+// (rbv_pt_run_sightlines, survey = true).  Arguments are checked by the callers except the ladder, which is copied to
+// the host and checked here.
+static int pt_run_entry(RbvContext* ctx, int S, bool survey, double* coords, double* lnprob, double* betas, int T,
+                        int W, int n_steps, const RbvPtControl* control, unsigned long long seed,
+                        unsigned long long first_step, double* chain, double* lnprob_chain, const RbvChainSink* sink,
+                        double* beta_history, double* ti_moments, int* n_accepted,
+                        unsigned long long* n_swaps_accepted, int* flag, void* workspace, size_t workspace_bytes,
+                        int use_graph, void* stream, const char* who) {
+  const std::string w(who);
+  if (n_steps < 0 || !(control->a > 1.0)) return fail(RBV_EINVAL, w + ": n_steps < 0 or stretch scale a <= 1");
+  if (control->n_record < 1 || control->n_record > T) return fail(RBV_EINVAL, w + ": n_record outside 1 .. n_temps");
   if (control->adapt && !(control->adaptation_lag > 0.0 && control->adaptation_time > 0.0))
-    return fail(RBV_EINVAL, "rbv_pt_run: adaptation_lag and adaptation_time must be > 0");
-  if (sink && (chain || lnprob_chain)) return fail(RBV_EINVAL, "rbv_pt_run: pass device chains or a sink, not both");
+    return fail(RBV_EINVAL, w + ": adaptation_lag and adaptation_time must be > 0");
+  if (sink && (chain || lnprob_chain)) return fail(RBV_EINVAL, w + ": pass device chains or a sink, not both");
   if (sink && (sink->block_steps < 1 || !sink->ring_dev || !sink->ring_pinned))
-    return fail(RBV_EINVAL, "rbv_pt_run: incomplete chain sink");
-  if (ctx->inst.empty() || ctx->ndim == 0) return fail(RBV_ESTATE, "rbv_pt_run: context not set up");
-  const StretchLayout lay = pt_layout(ctx, T, W);
-  if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, "rbv_pt_run: workspace too small");
+    return fail(RBV_EINVAL, w + ": incomplete chain sink");
+  if (ctx->inst.empty() || ctx->ndim == 0) return fail(RBV_ESTATE, w + ": context not set up");
+  const StretchLayout lay = pt_layout(ctx, S, T, W, survey);
+  if (!workspace || workspace_bytes < lay.total) return fail(RBV_ENOMEM, w + ": workspace too small");
   RBV_ON_DEVICE(ctx);
   cudaStream_t st = (cudaStream_t)stream;
-  std::vector<double> b((size_t)T);      // the ladder is checked on the host: a 8 T-byte copy before the run
-  RBV_CUDA(cudaMemcpyAsync(b.data(), betas, (size_t)T * sizeof(double), cudaMemcpyDeviceToHost, st));
+  std::vector<double> b((size_t)S * T);      // the ladders are checked on the host: a 8 S T-byte copy before the run
+  RBV_CUDA(cudaMemcpyAsync(b.data(), betas, b.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
   RBV_CUDA(cudaStreamSynchronize(st));
-  if (b[0] != 1.0) return fail(RBV_EINVAL, "rbv_pt_run: betas[0] must be 1");
-  for (int t = 1; t < T; ++t)
-    if (!(b[t] < b[t - 1]) || !(b[t] >= 0.0))
-      return fail(RBV_EINVAL, "rbv_pt_run: betas must be strictly decreasing and >= 0");
+  for (int sl = 0; sl < S; ++sl) {
+    const double* bs = b.data() + (size_t)sl * T;
+    const std::string where = survey ? w + ": sightline " + std::to_string(sl) + ": " : w + ": ";
+    if (bs[0] != 1.0) return fail(RBV_EINVAL, where + "betas[0] must be 1");
+    for (int t = 1; t < T; ++t)
+      if (!(bs[t] < bs[t - 1]) || !(bs[t] >= 0.0))
+        return fail(RBV_EINVAL, where + "betas must be strictly decreasing and >= 0");
+  }
   if (n_steps == 0) return RBV_OK;
   char* ws = (char*)workspace;
   StretchParams P;
@@ -2514,7 +2534,7 @@ int rbv_pt_run(RbvContext* ctx, double* coords, double* lnprob, double* betas, i
   P.a = control->a;
   P.W = W;
   P.ndim = ctx->ndim;
-  P.S = T;
+  P.S = S * T;                   // ensemble e = s T + t: its stretch streams are offset by e W = s T W + t W
   P.beta = betas;
   PtParams Q;
   memset(&Q, 0, sizeof(Q));
@@ -2527,6 +2547,7 @@ int rbv_pt_run(RbvContext* ctx, double* coords, double* lnprob, double* betas, i
   Q.chain = chain;
   Q.lnp_chain = lnprob_chain;
   Q.beta_history = beta_history;
+  Q.ti = ti_moments;
   Q.step_ctr = P.step_ctr;
   Q.ticket = (unsigned int*)(ws + lay.ctr + 64);
   Q.first_step = first_step;
@@ -2535,18 +2556,58 @@ int rbv_pt_run(RbvContext* ctx, double* coords, double* lnprob, double* betas, i
   Q.adapt_lag = control->adaptation_lag;
   Q.adapt_time = control->adaptation_time;
   Q.adapt = control->adapt != 0;
+  Q.S = S;
   Q.T = T;
   Q.W = W;
   Q.ndim = ctx->ndim;
   Q.n_record = control->n_record;
+  Q.survey = survey ? 1 : 0;
   if (sink) {
     Q.ring_steps = 2 * sink->block_steps;
     Q.chain = sink->ring_dev;
-    Q.lnp_chain = sink->ring_dev + (size_t)Q.ring_steps * Q.n_record * W * ctx->ndim;
+    // survey mode without a host lnprob array: the ring holds chain rows only
+    Q.lnp_chain = (survey && !sink->lnprob_chain_host)
+                      ? nullptr : sink->ring_dev + (size_t)Q.ring_steps * S * Q.n_record * W * ctx->ndim;
     int rc = sink_stream_setup(ctx);
     if (rc != RBV_OK) return rc;
   }
   return stretch_run_impl(ctx, P, lay, ws, workspace_bytes, W, n_steps, false, sink, use_graph, st, who, &Q);
+}
+
+int rbv_pt_run(RbvContext* ctx, double* coords, double* lnprob, double* betas, int n_temps, int n_walkers,
+               int n_steps, const RbvPtControl* control, unsigned long long seed, unsigned long long first_step,
+               double* chain, double* lnprob_chain, const RbvChainSink* sink, double* beta_history, int* n_accepted,
+               unsigned long long* n_swaps_accepted, int* flag, void* workspace, size_t workspace_bytes,
+               int use_graph, void* stream) {
+  const int T = n_temps, W = n_walkers;
+  if (!ctx || !coords || !lnprob || !betas || !control || !n_accepted || !flag || (T > 1 && !n_swaps_accepted))
+    return fail(RBV_EINVAL, "rbv_pt_run: null argument");
+  if (!pt_shape_ok(T, W))
+    return fail(RBV_EINVAL, "rbv_pt_run: need 1 <= n_temps <= 4096, n_walkers >= 2 and n_temps * n_walkers in int range");
+  return pt_run_entry(ctx, 1, false, coords, lnprob, betas, T, W, n_steps, control, seed, first_step, chain,
+                      lnprob_chain, sink, beta_history, nullptr, n_accepted, n_swaps_accepted, flag, workspace,
+                      workspace_bytes, use_graph, stream, "rbv_pt_run");
+}
+
+int rbv_pt_run_sightlines(RbvContext* ctx, double* coords, double* lnprob, double* betas, int n_temps,
+                          int walkers_per_sightline, int n_steps, const RbvPtControl* control, unsigned long long seed,
+                          unsigned long long first_step, double* chain, double* lnprob_chain,
+                          const RbvChainSink* sink, double* beta_history, double* ti_moments, int* n_accepted,
+                          unsigned long long* n_swaps_accepted, int* flag, void* workspace, size_t workspace_bytes,
+                          int use_graph, void* stream) {
+  const int T = n_temps, W = walkers_per_sightline;
+  if (!ctx || !coords || !lnprob || !betas || !control || !n_accepted || !flag || (T > 1 && !n_swaps_accepted))
+    return fail(RBV_EINVAL, "rbv_pt_run_sightlines: null argument");
+  if (ctx->inst.empty() || ctx->ndim == 0) return fail(RBV_ESTATE, "rbv_pt_run_sightlines: context not set up");
+  if (!pt_sightlines_shape_ok((long long)ctx->inst.size(), T, W))
+    return fail(RBV_EINVAL, "rbv_pt_run_sightlines: need 1 <= n_temps <= 4096, walkers_per_sightline >= 2 and "
+                            "n_sightlines * n_temps * walkers_per_sightline in int range");
+  if (control->adapt && ti_moments)
+    return fail(RBV_EINVAL, "rbv_pt_run_sightlines: ti_moments with adapt: adaptation breaks detailed balance, "
+                            "its steps must not enter the evidence");
+  return pt_run_entry(ctx, (int)ctx->inst.size(), true, coords, lnprob, betas, T, W, n_steps, control, seed,
+                      first_step, chain, lnprob_chain, sink, beta_history, ti_moments, n_accepted, n_swaps_accepted,
+                      flag, workspace, workspace_bytes, use_graph, stream, "rbv_pt_run_sightlines");
 }
 
 // ---- multi-GPU form of the sampler: half-step = propose_eval | caller's all-gather of lnprob | accept ----------

@@ -758,6 +758,89 @@ class Engine:
                       adapt_steps_done, n_record)
         return chain, lps
 
+    def _pt_sl_checks(self, coords_t, lnp_t, betas_t, n_steps, beta_hist_t, ti_t, n_accepted_t, n_swaps_t, flag_t):
+        torch = _torch()
+        if coords_t.dim() != 4 or coords_t.shape[0] != len(self.pixels) or coords_t.shape[3] != self.ndim:
+            raise ValueError(f"coords must be [{len(self.pixels)}, n_temps, walkers_per_sightline, {self.ndim}]")
+        S, T, W, ndim = coords_t.shape
+        self._dev_tensor(coords_t, torch.float64, "coords")
+        self._dev_tensor(lnp_t, torch.float64, "lnprob", (S, T, W))
+        self._dev_tensor(betas_t, torch.float64, "betas", (S, T))
+        self._dev_tensor(beta_hist_t, torch.float64, "beta history", (int(n_steps), S, T))
+        self._dev_tensor(ti_t, torch.float64, "ti_moments", (S, T, 3))
+        self._dev_tensor(n_accepted_t, torch.int32, "n_accepted", (S, T, W))
+        self._dev_tensor(n_swaps_t, torch.int64, "n_swaps_accepted", (S, max(T - 1, 1)))
+        self._dev_tensor(flag_t, torch.int32, "flag")
+        nbytes = C.c_size_t(0)
+        check(self.lib.rbv_pt_workspace_bytes_sightlines(self._h, T, W, C.byref(nbytes)),
+              "rbv_pt_workspace_bytes_sightlines")
+        if self._stretch_ws is None or self._stretch_ws.numel() < nbytes.value:
+            self._stretch_ws = None
+            self._stretch_ws = torch.empty(int(nbytes.value), dtype=torch.uint8, device=self.tdev)
+        return S, T, W, ndim
+
+    def _pt_sl_call(self, coords_t, lnp_t, betas_t, T, W, n_steps, a, seed, first_step, chain_p, lnp_chain_p, sink,
+                    beta_hist_t, ti_t, n_accepted_t, n_swaps_t, flag_t, use_graph, adapt, adaptation_lag,
+                    adaptation_time, adapt_steps_done, n_record):
+        ctl = RbvPtControl(float(a), int(bool(adapt)), float(adaptation_lag), float(adaptation_time),
+                           int(adapt_steps_done), int(n_record))
+        check(self.lib.rbv_pt_run_sightlines(
+            self._h, coords_t.data_ptr(), lnp_t.data_ptr(), betas_t.data_ptr(), T, W, int(n_steps), C.byref(ctl),
+            int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_step), chain_p, lnp_chain_p, sink,
+            beta_hist_t.data_ptr() if beta_hist_t is not None else None,
+            ti_t.data_ptr() if ti_t is not None else None, n_accepted_t.data_ptr(), n_swaps_t.data_ptr(),
+            flag_t.data_ptr(), self._stretch_ws.data_ptr(), self._stretch_ws.numel(), int(bool(use_graph)),
+            self._stream()), "rbv_pt_run_sightlines")
+
+    def pt_run_sightlines(self, coords_t, lnp_t, betas_t, n_steps: int, a: float, seed: int, first_step: int,
+                          chain_t, lnp_chain_t, beta_hist_t, ti_t, n_accepted_t, n_swaps_t, flag_t,
+                          use_graph: bool = True, adapt: bool = False, adaptation_lag: float = 10000.0,
+                          adaptation_time: float = 100.0, adapt_steps_done: int = 0, n_record: int = 1):
+        """Survey-mode parallel tempering (rbv_pt_run_sightlines): ``coords_t`` [S, T, W, ndim], one tempered
+        ladder of ensembles per sightline of this context, all advancing in lockstep; ``lnp_t`` [S, T, W]
+        (untempered), ``betas_t`` [S, T] (in/out); ``chain_t`` [n_steps, S, n_record, W, ndim], ``lnp_chain_t``
+        [n_steps, S, T, W], ``beta_hist_t`` [n_steps, S, T] and ``ti_t`` [S, T, 3] (the accumulated (n, mean, M2)
+        of ln L; refused with ``adapt``) may be None; ``n_accepted_t`` int32 [S, T, W], ``n_swaps_t`` int64
+        [S, max(T - 1, 1)].  Every tensor stays on the device; runs on the current torch stream."""
+        torch = _torch()
+        S, T, W, ndim = self._pt_sl_checks(coords_t, lnp_t, betas_t, n_steps, beta_hist_t, ti_t, n_accepted_t,
+                                           n_swaps_t, flag_t)
+        self._dev_tensor(chain_t, torch.float64, "chain", (int(n_steps), S, int(n_record), W, ndim))
+        self._dev_tensor(lnp_chain_t, torch.float64, "lnprob chain", (int(n_steps), S, T, W))
+        self._pt_sl_call(coords_t, lnp_t, betas_t, T, W, n_steps, a, seed, first_step,
+                         chain_t.data_ptr() if chain_t is not None else None,
+                         lnp_chain_t.data_ptr() if lnp_chain_t is not None else None, None, beta_hist_t, ti_t,
+                         n_accepted_t, n_swaps_t, flag_t, use_graph, adapt, adaptation_lag, adaptation_time,
+                         adapt_steps_done, n_record)
+
+    def pt_run_sightlines_to_host(self, coords_t, lnp_t, betas_t, n_steps: int, a: float, seed: int,
+                                  first_step: int, beta_hist_t, ti_t, n_accepted_t, n_swaps_t, flag_t,
+                                  adapt: bool = False, adaptation_lag: float = 10000.0, adaptation_time: float = 100.0,
+                                  adapt_steps_done: int = 0, n_record: int = 1, record_chain: bool = True,
+                                  record_log_like: bool = True):
+        """``pt_run_sightlines`` with the chain delivered to the HOST while the run goes on (the chain sink of
+        ``pt_run_to_host``): returns (chain [n_steps, S, n_record, W, ndim] or None, lnprob chain [n_steps, S, T, W]
+        or None).  Without ``record_log_like`` no lnprob row is recorded or copied."""
+        torch = _torch()
+        S, T, W, ndim = self._pt_sl_checks(coords_t, lnp_t, betas_t, n_steps, beta_hist_t, ti_t, n_accepted_t,
+                                           n_swaps_t, flag_t)
+        row = S * int(n_record) * W * ndim + (S * T * W if record_log_like else 0)
+        K = int(min(256, max(1, (6 << 20) // (row * 8)), max(1, (int(n_steps) + 1) // 2)))   # ~6 MB blocks
+        need = 2 * K * row
+        if self._sink_ring is None or self._sink_ring[0] != K or self._sink_ring[1].numel() < need:
+            self._sink_ring = None
+            self._sink_ring = (K, torch.empty(need, dtype=torch.float64, device=self.tdev),
+                               torch.empty(need, dtype=torch.float64, pin_memory=True))
+        _k, ring_dev, ring_pin = self._sink_ring
+        chain = np.empty((int(n_steps), S, int(n_record), W, ndim), dtype=np.float64) if record_chain else None
+        lps = np.empty((int(n_steps), S, T, W), dtype=np.float64) if record_log_like else None
+        sink = RbvChainSink(chain.ctypes.data if chain is not None else None,
+                            lps.ctypes.data if lps is not None else None, ring_dev.data_ptr(), ring_pin.data_ptr(), K)
+        self._pt_sl_call(coords_t, lnp_t, betas_t, T, W, n_steps, a, seed, first_step, None, None, C.byref(sink),
+                         beta_hist_t, ti_t, n_accepted_t, n_swaps_t, flag_t, True, adapt, adaptation_lag,
+                         adaptation_time, adapt_steps_done, n_record)
+        return chain, lps
+
     def slice_run(self, coords_t, lnp_t, n_steps: int, tuning, seed: int, first_step: int, chain_t, lnp_chain_t,
                   flag_t, use_graph: bool = True) -> np.ndarray:
         """Device-resident ensemble slice sampling (rbv_slice_run) on the current torch stream; ``tuning`` is an
