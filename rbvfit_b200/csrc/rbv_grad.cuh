@@ -30,6 +30,10 @@ constexpr int kGradBlock = 256;                 // pixels per block of the per-p
 constexpr int kGradPPT = 4;                     // pixels per thread of the line pass
 constexpr int kGradTile = kGradBlock * kGradPPT;
 constexpr int kGradLineChunk = 32;              // lines whose series coefficients sit in shared memory at once
+// terms of the rho-series derivatives beyond kDFar.  E = H + x H_x + a H_a starts at rho^2 (its p = 1 terms cancel),
+// so its truncation after NQ terms is ~rho^(NQ - 1) relative: kNQFar = 3 (enough for H, 2e-13) leaves E off by up to
+// 1.6e-8 at |z|^2 = 4e4, 5 terms by 4e-16
+constexpr int kNQFarGrad = 5;
 
 struct GradInst {
   int blk_off;        // first 256-pixel block of the instrument (pixel buffers are padded to whole blocks)
@@ -244,7 +248,7 @@ __device__ __forceinline__ HGrad voigt_hgrad(double x, double a, double a2, doub
                                              const double* qd, const double* __restrict__ tab) {
   if (a > kABig) return (d < kDCore) ? weideman_grad(x, a) : asym_complex_grad(x, a, d);
   if (d < kDCore) return (a <= kAFast) ? table_grad(x, a, a2, tab) : weideman_grad(x, a);
-  if (d >= kDFar) return series_grad<kNQFar>(x, a, a2, d, q, qd);
+  if (d >= kDFar) return series_grad<kNQFarGrad>(x, a, a2, d, q, qd);
   if (d >= kDNear) return series_grad<kNQMid>(x, a, a2, d, q, qd);
   return series_grad<kNQNear>(x, a, a2, d, q, qd);
 }

@@ -31,13 +31,14 @@ def line_x_a(om, theta, wave):
     return (freq - freq0) / b_f, (np.asarray(om.atomic_gamma, dtype=np.float64)[:, None] / (4 * np.pi * b_f))[:, 0]
 
 
-def probe_pixels(P, K, om=None, theta=None, wave=None, n_random=24, seed=0):
+def probe_pixels(P, K, om=None, theta=None, wave=None, n_random=24, seed=0, targets=(64.0, 576.0, 4e4)):
     """Sorted unique pixel indices where a lnprob kernel can go wrong:
     - every pixel within K + 1 of a multiple of 1024 (any range boundary of any schedule);
     - the first and the last K + 2 pixels (edge replication of the LSF);
     - +-1 around each multiple of 256 (row starts) in the first two super-chunks;
-    - per line (with ``om``, ``theta``, ``wave``): the pixels nearest to |z|^2 = x^2 + a^2 = 64, 576 and 4e4 on either
-      side of the line, and the one nearest to its centre (the Voigt tier switches);
+    - per line (with ``om``, ``theta``, ``wave``): the pixels nearest to |z|^2 = x^2 + a^2 = each of ``targets``
+      (default 64, 576 and 4e4, the kernels' Voigt tier switches) on either side of the line, and the one nearest to
+      its centre;
     - ``n_random`` seeded random pixels."""
     sel = [np.arange(min(P, K + 2)), np.arange(max(0, P - K - 2), P)]
     for m in range(SUPER, P, SUPER):
@@ -49,7 +50,7 @@ def probe_pixels(P, K, om=None, theta=None, wave=None, n_random=24, seed=0):
         for xl, al in zip(x, a):
             z2 = xl * xl + al * al
             sel.append([int(np.argmin(np.abs(xl)))])
-            for target in (64.0, 576.0, 4e4):
+            for target in targets:
                 for side in (xl < 0, xl >= 0):
                     if side.any():
                         d = np.where(side, np.abs(z2 - target), np.inf)
